@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - QMIX learner episodes/sec (+ MAC agent-steps/sec) on SMAC-shaped synthetic episodes: BASELINE.json's metric.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 27m_vs_30m] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 27m_vs_30m] [--impl reference] [--dump-outputs DIR]
 
 One "step" is one QLearner.train call over one batch (both agent unrolls, double-Q targets, both mixers, masked TD loss,
 backward, clip, RMSprop, target-sync bookkeeping).  Default workload = BASELINE config 4: QMIX on 27m_vs_30m shapes,
@@ -325,19 +325,18 @@ def reference_arm(a, cfg):
         return
     shape = SMAC_SHAPES[cfg["shape"]]
     batch = a.cpu_batch or (32 if shape.n_agents > 5 else min(cfg["batch"], 64))
-    steps, warmup = max(1, min(a.steps, 6)), max(1, min(a.warmup, 2))
-    cb = cpu_learner(cfg, batch, steps, warmup)
-    ro = cpu_rollout(a.cpu_envs, max(1, min(a.steps, 10)), 2)
+    cb = cpu_learner(cfg, batch, a.steps, a.warmup)
+    ro = cpu_rollout(a.cpu_envs, a.steps, a.warmup)
     line = {
-        "impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": a.gpus, "steps": steps,
-        "warmup": warmup, "ms_per_step": cb["ms_per_step"], "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
+        "impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": a.gpus, "steps": a.steps,
+        "warmup": a.warmup, "ms_per_step": cb["ms_per_step"], "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
         "dtype": "f32", "data": "synthetic",
         "config": {"workload": _workload_name(cfg), "name": a.config, "shape": cfg["shape"], "T": cfg["T"], "mixer": cfg["mixer"],
                    "batch": batch, "note": "CPU reference on the host cores; each step a bounded sample of the workload"},
         "cpu_baseline": cb,
         "e2e": {"value": cb["value"], "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
-        "select_actions": {"metric": RO_METRIC, "value": ro["value"], "unit": RO_UNIT, "ms_per_step": ro["ms_per_step"],
-                           "cpu_baseline": ro},
+        "select_actions": {"metric": RO_METRIC, "value": ro["value"], "unit": RO_UNIT, "steps": a.steps, "warmup": a.warmup,
+                           "ms_per_step": ro["ms_per_step"], "cpu_baseline": ro},
     }
     print(json.dumps(line), flush=True)
 
@@ -405,10 +404,44 @@ def build_learner(ctx, cfg, precision, **over):
     return learner
 
 
-def time_learner(ctx, learner, batch, steps, warmup, profile):
+def learner_outputs(learner):
+    """What QLearner.train hands its caller after a step: the updated online parameters and the step's statistics."""
+    import numpy as np
+    out = {}
+    for tag, mod in (("agent", learner.mac.agent), ("mixer", learner.mixer)):
+        if mod is not None:
+            for k, v in mod.state_dict().items():
+                out[tag + "." + k] = v.detach().float().cpu().numpy()
+    st = learner.stats()
+    for k in ("loss", "grad_norm", "td_error_abs", "q_taken_mean", "target_mean"):
+        out[k] = np.array([st[k]], dtype=np.float64)
+    return out
+
+
+def rollout_outputs(actions, hidden, n_envs, max_envs=4096):
+    """What BasicMAC.select_actions hands its caller after a step: the chosen actions and the hidden state carried into the
+    next step, for a fixed, seeded sample of at most `max_envs` envs (the hidden state of 16384 envs is 113 MB).  With
+    the default epsilon schedule most actions are random draws; the hidden state carries the network's arithmetic."""
+    import numpy as np
+    import torch as th
+    envs = np.arange(n_envs) if n_envs <= max_envs else np.sort(np.random.default_rng(0).choice(n_envs, max_envs, replace=False))
+    idx = th.from_numpy(envs).to(actions.device)
+    return {"actions": actions[idx].float().cpu().numpy(),
+            "hidden_states": hidden.reshape(n_envs, -1, hidden.shape[-1])[idx].float().cpu().numpy()}
+
+
+def write_outputs(outputs, out_dir):
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+
+
+def time_learner(ctx, learner, batch, steps, warmup, profile, after_timed=None):
     """W untimed + K timed steps (barrier + synchronize on both sides, CUDA events on the launch stream, max over ranks).
     profile=True arms the library's per-phase events for the TIMED steps themselves, so the per-kernel times see the
-    clocks `ms_per_step` sees.  -> (ms per step, phases_ms averaged per step, launches per step, clocks)."""
+    clocks `ms_per_step` sees.  after_timed() runs right after the last timed step, before the untimed steps that keep
+    the GPU busy for the clock sampler.  -> (ms per step, phases_ms averaged per step, launches per step, clocks)."""
     th = ctx.th
     from pymarl_b200 import _lib
     l0 = _lib.lib().pmb_launch_count()
@@ -429,6 +462,8 @@ def time_learner(ctx, learner, batch, steps, warmup, profile):
     ctx.barrier()
     phases = _lib.profile_end(max_phases=1024) if profile else []
     ms = ctx.max_over_ranks(ev0.elapsed_time(ev1) / steps)
+    if after_timed is not None:
+        after_timed()
     clocks = _finish_sampling(th, sampler, lambda i: learner.train(batch, i, 0), ms, collective=ctx.world > 1)
     phase_ms = {}
     for name, pms in phases:
@@ -586,10 +621,10 @@ def dp_self_check(ctx):
 
 
 # ------------------------------------------------------------------------------------------
-def rollout_record(ctx, a, envs, precision, steps, warmup, e2e_steps, with_cpu):
+def rollout_record(ctx, a, envs, precision, steps, warmup, e2e_steps, with_cpu, outputs=None):
     """BASELINE config 5: one BasicMAC.select_actions step (fc1 -> GRUCell -> fc2 -> avail mask -> epsilon-greedy) over
     `envs` synthetic envs x 27 agents per GPU; agent-steps/s.  The obs of 4 timesteps live in HBM and the step index
-    cycles over them (2 GB, larger than L2)."""
+    cycles over them (2 GB, larger than L2).  A dict passed as `outputs` receives rollout_outputs() of the last timed step."""
     th = ctx.th
     from pymarl_b200 import mac_REGISTRY, _lib
     from pymarl_b200.synthetic import make_scheme, torch_episode_fields
@@ -616,11 +651,13 @@ def rollout_record(ctx, a, envs, precision, steps, warmup, e2e_steps, with_cpu):
     ctx.barrier()
     ev0.record()
     for i in range(steps):
-        mac.select_actions(batch, 1 + i % 3, 1000 * i)
+        acts = mac.select_actions(batch, 1 + i % 3, 1000 * i)
     ev1.record()
     ctx.barrier()
     launches = (_lib.lib().pmb_launch_count() - launches0) // max(1, steps)
     ms = ctx.max_over_ranks(ev0.elapsed_time(ev1) / steps)
+    if outputs is not None:
+        outputs.update(rollout_outputs(acts, mac.hidden_states, envs))
     clocks = _finish_sampling(th, sampler, lambda i: mac.select_actions(batch, 1 + i % 3, 0), ms)     # no collective in this step
     value = ctx.world * envs * N / (ms * 1e-3)
     rows = envs * N
@@ -811,13 +848,21 @@ def main():
                     help="select_actions: where the epsilon-greedy draws come from")
     ap.add_argument("--precision", default="bf16", choices=["fp32", "bf16"],
                     help="bf16 = tcgen05 tensor-core tier (fp32 accumulate, parity 1e-2); fp32 = CUDA-core tier (parity 1e-5)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy, to compare two builds: the updated "
+                    "agent / mixer parameters (float32) and the loss statistics (float64) of a learner step; the chosen "
+                    "actions and the carried hidden state (float32) of a select_actions step")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs compares builds of this project; the reference arm has nothing to dump")
     if a.config == "select_actions":
         if a.impl == "reference":
             if int(os.environ.get("RANK", "0")) == 0:
-                ro = cpu_rollout(a.cpu_envs, max(1, min(a.steps, 20)), 2)
+                ro = cpu_rollout(a.cpu_envs, a.steps, a.warmup)
                 print(json.dumps({"impl": "reference", "metric": RO_METRIC, "value": ro["value"], "unit": RO_UNIT,
-                                  "n_gpus": a.gpus, "steps": a.steps, "warmup": 2, "ms_per_step": ro["ms_per_step"],
+                                  "n_gpus": a.gpus, "steps": a.steps, "warmup": a.warmup, "ms_per_step": ro["ms_per_step"],
                                   "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
                                   "data": "synthetic", "config": {"workload": "BasicMAC.select_actions step, 27m_vs_30m shapes",
                                                                    "envs": a.cpu_envs},
@@ -825,10 +870,13 @@ def main():
                                                               "d2h_bytes_per_step": 0}}), flush=True)
             return
         ctx = Ctx()
+        outputs = {} if a.dump_outputs else None
         rec = rollout_record(ctx, a, a.batch or 16384, a.precision, a.steps, a.warmup, 0 if a.no_e2e else a.e2e_steps,
-                             with_cpu=(ctx.rank == 0 and ctx.world == 1 and not a.no_cpu_baseline))
+                             with_cpu=(ctx.rank == 0 and ctx.world == 1 and not a.no_cpu_baseline), outputs=outputs)
         rec["vs_baseline"] = None
         if ctx.rank == 0:
+            if outputs is not None:
+                write_outputs(outputs, a.dump_outputs)
             print(json.dumps(rec), flush=True)
         if ctx.world > 1:
             ctx.dist.destroy_process_group()
@@ -868,8 +916,8 @@ def main():
     weak = None
     if want_weak:
         wb = _DictBatch(fields_all, B_gen, T)
-        wms, _, _, _ = time_learner(ctx, learner, wb, max(3, a.steps // 2), 3, profile=False)
-        weak = {"value": ctx.world * B_gen / (wms * 1e-3), "unit": UNIT, "ms_per_step": wms, "batch_per_gpu": B_gen,
+        wms, _, _, _ = time_learner(ctx, learner, wb, a.steps, a.warmup, profile=False)
+        weak = {"value": ctx.world * B_gen / (wms * 1e-3), "unit": UNIT, "ms_per_step": wms, "steps": a.steps, "batch_per_gpu": B_gen,
                 "global_batch": ctx.world * B_gen, "scaling": "weak"}
         del wb
     fields = {k: v[:B_local] for k, v in fields_all.items()} if B_gen != B_local else fields_all
@@ -884,7 +932,12 @@ def main():
     exchange_desc = "single GPU" if ctx.world == 1 else (
         "exchange + clip + RMSprop fused in one kernel over NVLink peer memory" if getattr(learner, "_px", None) is not None
         else "one NCCL all-reduce of [grads | loss sums] per step")
-    ms, phase_ms, launches, clocks = time_learner(ctx, learner, batch, a.steps, a.warmup, profile=not a.cuda_graph)
+    outputs = {}
+    ms, phase_ms, launches, clocks = time_learner(
+        ctx, learner, batch, a.steps, a.warmup, profile=not a.cuda_graph,
+        after_timed=(lambda: outputs.update(learner_outputs(learner))) if a.dump_outputs else None)
+    if a.dump_outputs and ctx.rank == 0:
+        write_outputs(outputs, a.dump_outputs)
     if a.cuda_graph:
         phase_ms = profile_pass(learner, batch, 3)
     rec = learner_record(ctx, cfg, B_local, ms, phase_ms, launches, clocks, a.precision)
