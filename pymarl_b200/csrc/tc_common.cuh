@@ -124,6 +124,22 @@ __device__ __forceinline__ void tmem_ld_32x32(uint32_t taddr, uint32_t (&v)[32])
         : "memory");
 }
 
+// 32 lanes x 32 consecutive 32-bit columns from registers: thread i of the warp writes lane (base_lane + i)
+__device__ __forceinline__ void tmem_st_32x32(uint32_t taddr, const uint32_t (&v)[32]) {
+    asm volatile(
+        "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
+        "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, "
+        "%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};"
+        :
+        : "r"(taddr), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]), "r"(v[8]),
+          "r"(v[9]), "r"(v[10]), "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15]), "r"(v[16]), "r"(v[17]),
+          "r"(v[18]), "r"(v[19]), "r"(v[20]), "r"(v[21]), "r"(v[22]), "r"(v[23]), "r"(v[24]), "r"(v[25]), "r"(v[26]),
+          "r"(v[27]), "r"(v[28]), "r"(v[29]), "r"(v[30]), "r"(v[31])
+        : "memory");
+}
+// this thread's tcgen05.st have completed (before a fence / barrier hands the columns to the tensor core)
+__device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
+
 // ---- UMMA descriptors ------------------------------------------------------------------------
 // Shared-memory matrix descriptor, 128-byte swizzle (cute::UMMA::SmemDescriptor): start address
 // [0,14) >>4, leading byte offset [16,30) >>4, stride byte offset [32,46) >>4, version [46,48) = 1,
@@ -150,6 +166,18 @@ __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t a_desc, uint
         "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
         :
         : "r"(tmem_d), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
+        : "memory");
+}
+// D[tmem] (+)= A[tmem] . B[smem]: A (M x K, K-major) is read from tensor memory - lane = row of A, two bf16 per 32-bit
+// column (lower k in the low half), so one K = 16 step is 8 columns
+__device__ __forceinline__ void umma_bf16_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t b_desc, uint32_t idesc,
+                                             uint32_t accumulate) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
+        :
+        : "r"(tmem_d), "r"(tmem_a), "l"(b_desc), "r"(idesc), "r"(accumulate)
         : "memory");
 }
 // arrive on an mbarrier when all previously issued tcgen05.mma of this thread have completed

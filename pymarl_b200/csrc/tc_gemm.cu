@@ -551,6 +551,7 @@ struct Fc1StreamParams {
     int l2_prefetch;               // n > 0: prefetch the runs of the CTA's n-th next tile into L2 (off by default)
     int n_nets;                    // 2: online + target (learner step), 1: online only (rollout step)
     int t0;                        // batch timestep of item t = 0 (rollout: the step index; obs is addressed at t0 + t)
+    int n_act;                     // A: rows of tab_act16
 };
 
 __device__ __forceinline__ float lds_f32(uint32_t addr) {
@@ -568,22 +569,238 @@ __device__ __forceinline__ void sts_b32(uint32_t addr, uint32_t v) {
 // Per-role wait accounting (build with PMB_EXTRA_NVCC_FLAGS=-DPMB_FC1_PROFILE, read with tools/fc1_role_profile.py): cycles
 // each role spends blocked on each barrier / in each converter phase, summed over CTAs.  This is what located the
 // obs-image bulk store as the reason the converters idled between tiles.
+// Slots: 0-7 and 10-15 role cycles (names in the tool), 8 kernel cycles, 9 CTAs, 15 producer warps (= staging slots).
 #ifdef PMB_FC1_PROFILE
 __device__ unsigned long long g_fc1_prof[16];
 #define TWAIT(idx, bar, par) do { long long _t0 = clock64(); mbar_wait(bar, par); if (lane == 0) prof_acc[idx] += clock64() - _t0; } while (0)
 #define TMARK(var) const long long var = clock64()
 #define TADD(idx, expr) do { if (lane == 0) prof_acc[idx] += (expr); } while (0)
+#define FC1_PROF_BEGIN long long prof_acc[16] = {}; const long long prof_t0 = clock64()
+#define FC1_PROF_END(ns)                                                                                                  \
+    do {                                                                                                                  \
+        if (lane == 0)                                                                                                    \
+            for (int i = 0; i < 15; ++i)                                                                                  \
+                if (i != 8 && i != 9 && prof_acc[i]) atomicAdd(&g_fc1_prof[i], (unsigned long long)prof_acc[i]);          \
+        if (threadIdx.x == 0) {                                                                                           \
+            atomicAdd(&g_fc1_prof[8], (unsigned long long)(clock64() - prof_t0)); atomicAdd(&g_fc1_prof[9], 1ull);        \
+            atomicAdd(&g_fc1_prof[15], (unsigned long long)(ns));                                                         \
+        }                                                                                                                 \
+    } while (0)
 #else
 #define TWAIT(idx, bar, par) mbar_wait(bar, par)
 #define TMARK(var)
 #define TADD(idx, expr)
+#define FC1_PROF_BEGIN long long prof_acc[16]
+#define FC1_PROF_END(ns) do { } while (0)
 #endif
+// The two roles the learner and the rollout kernels below share: the producer warps that stream the obs runs of a
+// 16-row group into the fp32 staging ring, and the converter warps that turn a staged group into bf16 rows of the
+// K-major / 128B-swizzle obs tile (and of the obs image).
+struct Fc1Ring {
+    uint8_t* stage;         // [NS][slot_bytes]
+    int* rowoff;            // [NS][16] byte offset of a row in its slot
+    int* rown;              // [NS][16] agent index of the row
+    uint64_t* st_full;      // [NS]
+    uint64_t* st_empty;     // [NS]
+};
+
+template <int NC, int NS>
+__device__ __forceinline__ void fc1_produce(const Fc1StreamParams& P, const Fc1Ring& ring, int pw, int lane,
+                                            long long (&prof_acc)[16]) {
+    using namespace fs;
+    constexpr int N_SLOTS = NS;
+    uint8_t* stage = ring.stage;
+    int* rowoff = ring.rowoff;
+    int* rown = ring.rown;
+    uint64_t* st_full = ring.st_full;
+    uint64_t* st_empty = ring.st_empty;
+    const int64_t n_items = (int64_t)P.T * P.n_tiles;
+
+    // Lane i owns the i-th contiguous run of a group (one episode each) and computes its descriptor - global
+    // address, staging offset, head / interior / tail split - in closed form, in parallel with the other lanes
+    // and BEFORE the slot is free; once it is, every lane just issues its copies.  (The first version walked the
+    // runs serially after the wait: ~1.5 us of dependent integer code per group during which the slot sat empty,
+    // which bounded the stream at three slots per (walk + load + convert).)
+    uint32_t git = 0;
+    for (int64_t item = blockIdx.x; item < n_items; item += gridDim.x) {
+        const int64_t t = item / P.n_tiles, tile = item - t * P.n_tiles;
+        for (int g = 0; g < GROUPS; ++g, ++git) {
+            const int slot = git % N_SLOTS;
+            if (slot != pw) continue;
+            TMARK(pp0);
+            uint8_t* sl = stage + slot * P.slot_bytes;
+            int* ro = rowoff + slot * GROUP_ROWS;
+            int* rn = rown + slot * GROUP_ROWS;
+            const int64_t p0 = tile * BM + g * GROUP_ROWS;
+            int rows_here = P.R - p0 < GROUP_ROWS ? (int)(P.R - p0) : GROUP_ROWS;     // rows of this group below R
+            if (rows_here < 0) rows_here = 0;
+            const uint32_t b0 = (uint32_t)p0 / (uint32_t)P.N;               // B*N < 2^31 (validated on the host)
+            const int n00 = (int)((uint32_t)p0 - b0 * (uint32_t)P.N);
+            int first_cnt = P.N - n00;
+            if (first_cnt > rows_here) first_cnt = rows_here;
+            // run `lane`: rows [lr, lr + cnt) of the group, agent index n0 .. of episode b0 + lane
+            const int lr = lane == 0 ? 0 : first_cnt + (lane - 1) * P.N;
+            int cnt = lane == 0 ? first_cnt : (rows_here - lr < P.N ? rows_here - lr : P.N);
+            if (cnt < 0) cnt = 0;
+            const int n0 = lane == 0 ? n00 : 0;
+            const char* ga = nullptr;
+            uint32_t cur = 0, phase = 0, cp_bytes = 0;
+            if (cnt > 0) {
+                ga = reinterpret_cast<const char*>(P.obs + ep_row(P.ep_index, (int64_t)b0 + lane) * P.obs_sb +
+                                                   ((t + P.t0) * P.N + n0) * (int64_t)P.O);
+                phase = (uint32_t)(reinterpret_cast<uintptr_t>(ga) & 15);
+                // staging offset: same 128-BYTE phase as the source (the copy engine then moves whole lines: with only the
+                // 16-byte phase matched every line is split and shifted); 320 bytes of slack per run keep the runs - and
+                // the up to 15 bytes copied before / after each of them - disjoint
+                cur = (((uint32_t)lr * P.O * 4u + 127u) & ~127u) + 320u * lane + (uint32_t)(reinterpret_cast<uintptr_t>(ga) & 127);
+                // ONE bulk copy per run, widened to 16-byte boundaries on both sides (the extra bytes stay inside the
+                // 16-byte granules the run touches anyway - never another page - and land in the slack).  The first
+                // version copied the aligned interior and fetched head / tail with 4-byte cp.async: with the 32
+                // no-increment barrier arrivals that needs, publishing a slot took ~1600 cycles.
+                cp_bytes = (phase + (uint32_t)cnt * P.O * 4u + 15u) & ~15u;
+            }
+            const uint32_t tx = __reduce_add_sync(0xffffffffu, cp_bytes);
+            // L2 prefetch of the same group of this CTA's NEXT tile: the staging ring is all the shared memory that is
+            // left (3 x 18 KB in flight per SM), so the copies should see L2 latency, not loaded-HBM latency
+            if (P.l2_prefetch && cnt > 0 && item + (int64_t)P.l2_prefetch * gridDim.x < n_items) {
+                const int64_t item2 = item + (int64_t)P.l2_prefetch * gridDim.x;
+                const int64_t t2 = item2 / P.n_tiles, tile2 = item2 - t2 * P.n_tiles;
+                const int64_t q0 = tile2 * BM + g * GROUP_ROWS;
+                int rows2 = P.R - q0 < GROUP_ROWS ? (int)(P.R - q0) : GROUP_ROWS;
+                if (rows2 < 0) rows2 = 0;
+                const uint32_t c0 = (uint32_t)q0 / (uint32_t)P.N;
+                const int m00 = (int)((uint32_t)q0 - c0 * (uint32_t)P.N);
+                int fc = P.N - m00;
+                if (fc > rows2) fc = rows2;
+                const int lr2 = lane == 0 ? 0 : fc + (lane - 1) * P.N;
+                int cnt2 = lane == 0 ? fc : (rows2 - lr2 < P.N ? rows2 - lr2 : P.N);
+                if (cnt2 > 0) {
+                    const char* gb = reinterpret_cast<const char*>(P.obs + ep_row(P.ep_index, (int64_t)c0 + lane) * P.obs_sb +
+                                                                   ((t2 + P.t0) * P.N + (lane == 0 ? m00 : 0)) * (int64_t)P.O);
+                    const uintptr_t a0 = (reinterpret_cast<uintptr_t>(gb) + 15) & ~(uintptr_t)15;
+                    const uintptr_t a1 = (reinterpret_cast<uintptr_t>(gb) + (uint64_t)cnt2 * P.O * 4) & ~(uintptr_t)15;
+                    if (a1 > a0)
+                        asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(a0), "r"((uint32_t)(a1 - a0)) : "memory");
+                }
+            }
+            // row tables, one row per lane: row j belongs to run rj (run 0 holds first_cnt rows, the others N each)
+            const int rj = lane < first_cnt ? 0 : 1 + (lane - first_cnt) / P.N;
+            const int lrj = rj == 0 ? 0 : first_cnt + (rj - 1) * P.N;
+            const uint32_t cur_j = __shfl_sync(0xffffffffu, cur, rj & 31);
+            TADD(10, clock64() - pp0);                         // producer: descriptors of the group (before the slot wait)
+            TWAIT(0, &st_empty[slot], ((git / N_SLOTS) & 1) ^ 1);
+            TMARK(pp1);
+            if (lane < GROUP_ROWS) {
+                ro[lane] = lane < rows_here ? (int)(cur_j + (uint32_t)(lane - lrj) * P.O * 4u) : -1;   // rows beyond R: zeros
+                rn[lane] = (rj == 0 ? n00 : 0) + (lane - lrj);
+            }
+            if (cnt > 0) bulk_copy_g2s(sl + cur - phase, ga - phase, cp_bytes, &st_full[slot]);
+            __syncwarp();
+            if (lane == 0) {
+                if (tx) mbar_arrive_expect_tx(&st_full[slot], tx); else mbar_arrive(&st_full[slot]);
+            }
+            TADD(11, clock64() - pp1);                         // producer: tables, copies, arrival
+        }
+    }
+}
+
+// converter warp cw owns rows RPW cw .. RPW cw + RPW - 1 of every group; arrives on a_full once per finished tile
+template <int NC, int NS>
+__device__ __forceinline__ void fc1_convert(const Fc1StreamParams& P, const Fc1Ring& ring, uint8_t* a_s, uint64_t* a_free,
+                                            uint64_t* a_full, int cw, int lane, long long (&prof_acc)[16]) {
+    using namespace fs;
+    constexpr int N_SLOTS = NS;
+    constexpr int tile_bytes = NC * A_STAGE_BYTES;
+    uint8_t* stage = ring.stage;
+    int* rowoff = ring.rowoff;
+    int* rown = ring.rown;
+    uint64_t* st_full = ring.st_full;
+    uint64_t* st_empty = ring.st_empty;
+    const int64_t n_items = (int64_t)P.T * P.n_tiles;
+    constexpr int c_last = NC - 1;
+    // every column of the chunks before the last exists (O > 64 (NC-1)); the last chunk: per lane
+    const bool okl0 = c_last * BK + 2 * lane < P.O, okl1 = c_last * BK + 2 * lane + 1 < P.O;
+    const int j_pad = c_last * BK + 2 * lane - P.O;       // index of this lane's first column in the K padding
+    const uint32_t a_s_u32 = smem_u32(a_s);
+    const uint32_t a_base = a_s_u32 + ((uint32_t)(lane >> 2) << 4) + (lane & 3) * 4;   // + row*128, ^ swizzle
+    uint32_t git = 0, ti = 0;
+    for (int64_t item = blockIdx.x; item < n_items; item += gridDim.x, ++ti) {
+        for (int g = 0; g < GROUPS; ++g, ++git) {
+            const int slot = git % N_SLOTS;
+            TWAIT(1, &st_full[slot], (git / N_SLOTS) & 1);
+            TMARK(pt1);
+            const uint32_t sl = smem_u32(stage + slot * P.slot_bytes) + 8u * lane;
+            int offs[RPW], nns[RPW];
+#pragma unroll
+            for (int rr = 0; rr < RPW; ++rr) {
+                offs[rr] = rowoff[slot * GROUP_ROWS + RPW * cw + rr];
+                nns[rr] = rown[slot * GROUP_ROWS + RPW * cw + rr];
+            }
+            float v0[RPW][NC], v1[RPW][NC];
+            {
+#pragma unroll
+                for (int rr = 0; rr < RPW; ++rr) {           // all loads first
+                    const int off = offs[rr];
+                    const bool real = off >= 0;
+                    const uint32_t src = sl + (uint32_t)(real ? off : 0);
+#pragma unroll
+                    for (int c = 0; c < NC; ++c) {
+                        v0[rr][c] = 0.f; v1[rr][c] = 0.f;
+                        if (real && (c < c_last || okl0)) v0[rr][c] = lds_f32(src + c * 256);
+                        if (real && (c < c_last || okl1)) v1[rr][c] = lds_f32(src + c * 256 + 4);
+                    }
+                }
+                // pack first (consumes every loaded value), release the staging slot, then write the A tile
+                uint32_t pk[RPW][NC];
+#pragma unroll
+                for (int rr = 0; rr < RPW; ++rr) {
+                    const int off = offs[rr];
+                    const int nn = nns[rr];
+                    // one-hot(agent) and the bias column live in the K padding of the last chunk
+                    const bool fold = P.fold_id && off >= 0;
+                    const bool hit0 = fold && j_pad >= 0 && (j_pad == nn || j_pad == P.N);
+                    const bool hit1 = fold && j_pad + 1 >= 0 && (j_pad + 1 == nn || j_pad + 1 == P.N);
+#pragma unroll
+                    for (int c = 0; c < NC; ++c) {
+                        float a = v0[rr][c], b = v1[rr][c];
+                        if (c == c_last) { a = hit0 ? 1.0f : a; b = hit1 ? 1.0f : b; }
+                        pk[rr][c] = pack_bf16x2(a, b);
+                    }
+                }
+                __syncwarp();
+                if (lane == 0) mbar_arrive(&st_empty[slot]);
+                TMARK(pt2);
+                TADD(6, pt2 - pt1);                            // load + pack phase
+                // the first group of a tile waits here (values already in registers, slot already released) until
+                // the MMAs and the image store of the previous tile are done with the A tile
+                if (g == 0) TWAIT(2, a_free, (ti & 1) ^ 1);
+#pragma unroll
+                for (int rr = 0; rr < RPW; ++rr) {
+                    const uint32_t rt = (uint32_t)(g * GROUP_ROWS + RPW * cw + rr);
+                    const uint32_t dst = (a_base + rt * 128u) ^ ((rt & 7u) << 4);
+#pragma unroll
+                    for (int c = 0; c < NC; ++c) sts_b32(dst + c * A_STAGE_BYTES, pk[rr][c]);
+                    // the obs image leaves from here too: the warp's 32 words are one full 128-byte line of the image
+                    // (a bulk store of the finished A tile kept the tile busy for ~2500 cycles after the MMAs were
+                    // done with it: the converters of the next tile waited 22 % of the kernel time for it)
+                    if (P.obs_img) {
+                        uint8_t* img = P.obs_img + item * tile_bytes + (dst - a_s_u32);
+#pragma unroll
+                        for (int c = 0; c < NC; ++c) __stcs(reinterpret_cast<uint32_t*>(img + c * A_STAGE_BYTES), pk[rr][c]);
+                    }
+                }
+                TADD(7, clock64() - pt2);                      // store phase (includes the a_free wait of group 0)
+            }
+        }
+        fence_proxy_async_smem();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(a_full);
+    }
+}
+
 template <int NC, int NS>
 __global__ void __launch_bounds__(fs::threads_for(NS), 1) fc1_stream_kernel(Fc1StreamParams P) {
-#ifdef PMB_FC1_PROFILE
-    long long prof_acc[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
-    const long long prof_t0 = clock64();
-#endif
+    FC1_PROF_BEGIN;
     using namespace fs;
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
@@ -620,6 +837,7 @@ __global__ void __launch_bounds__(fs::threads_for(NS), 1) fc1_stream_kernel(Fc1S
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
     const int64_t n_items = (int64_t)P.T * P.n_tiles;
+    const Fc1Ring ring{stage, rowoff, rown, st_full, st_empty};
     // programmatic dependent launch (rollout step only; see gru_rollout_kernel): the next kernel may be scheduled as the
     // CTAs of this grid leave; this kernel reads nothing its predecessor writes and only its epilogue warps write something
     // the predecessor (the GRU step of the previous rollout step) may still be reading - the x images
@@ -635,176 +853,12 @@ __global__ void __launch_bounds__(fs::threads_for(NS), 1) fc1_stream_kernel(Fc1S
             for (int c = 0; c < NC; ++c)
                 bulk_copy_g2s(w_s + c * w_chunk, reinterpret_cast<const uint8_t*>(P.Wp) + c * A_STAGE_BYTES, (uint32_t)w_chunk, w_full);
         }
-        // Lane i owns the i-th contiguous run of a group (one episode each) and computes its descriptor - global
-        // address, staging offset, head / interior / tail split - in closed form, in parallel with the other lanes
-        // and BEFORE the slot is free; once it is, every lane just issues its copies.  (The first version walked the
-        // runs serially after the wait: ~1.5 us of dependent integer code per group during which the slot sat empty,
-        // which bounded the stream at three slots per (walk + load + convert).)
-        uint32_t git = 0;
-        for (int64_t item = blockIdx.x; item < n_items; item += gridDim.x) {
-            const int64_t t = item / P.n_tiles, tile = item - t * P.n_tiles;
-            for (int g = 0; g < GROUPS; ++g, ++git) {
-                const int slot = git % N_SLOTS;
-                if (slot != pw) continue;
-                TMARK(pp0);
-                uint8_t* sl = stage + slot * P.slot_bytes;
-                int* ro = rowoff + slot * GROUP_ROWS;
-                int* rn = rown + slot * GROUP_ROWS;
-                const int64_t p0 = tile * BM + g * GROUP_ROWS;
-                int rows_here = P.R - p0 < GROUP_ROWS ? (int)(P.R - p0) : GROUP_ROWS;     // rows of this group below R
-                if (rows_here < 0) rows_here = 0;
-                const uint32_t b0 = (uint32_t)p0 / (uint32_t)P.N;               // B*N < 2^31 (validated on the host)
-                const int n00 = (int)((uint32_t)p0 - b0 * (uint32_t)P.N);
-                int first_cnt = P.N - n00;
-                if (first_cnt > rows_here) first_cnt = rows_here;
-                // run `lane`: rows [lr, lr + cnt) of the group, agent index n0 .. of episode b0 + lane
-                const int lr = lane == 0 ? 0 : first_cnt + (lane - 1) * P.N;
-                int cnt = lane == 0 ? first_cnt : (rows_here - lr < P.N ? rows_here - lr : P.N);
-                if (cnt < 0) cnt = 0;
-                const int n0 = lane == 0 ? n00 : 0;
-                const char* ga = nullptr;
-                uint32_t cur = 0, phase = 0, cp_bytes = 0;
-                if (cnt > 0) {
-                    ga = reinterpret_cast<const char*>(P.obs + ep_row(P.ep_index, (int64_t)b0 + lane) * P.obs_sb +
-                                                       ((t + P.t0) * P.N + n0) * (int64_t)P.O);
-                    phase = (uint32_t)(reinterpret_cast<uintptr_t>(ga) & 15);
-                    // staging offset: same 128-BYTE phase as the source (the copy engine then moves whole lines: with only the
-                    // 16-byte phase matched every line is split and shifted); 320 bytes of slack per run keep the runs - and
-                    // the up to 15 bytes copied before / after each of them - disjoint
-                    cur = (((uint32_t)lr * P.O * 4u + 127u) & ~127u) + 320u * lane + (uint32_t)(reinterpret_cast<uintptr_t>(ga) & 127);
-                    // ONE bulk copy per run, widened to 16-byte boundaries on both sides (the extra bytes stay inside the
-                    // 16-byte granules the run touches anyway - never another page - and land in the slack).  The first
-                    // version copied the aligned interior and fetched head / tail with 4-byte cp.async: with the 32
-                    // no-increment barrier arrivals that needs, publishing a slot took ~1600 cycles.
-                    cp_bytes = (phase + (uint32_t)cnt * P.O * 4u + 15u) & ~15u;
-                }
-                const uint32_t tx = __reduce_add_sync(0xffffffffu, cp_bytes);
-                // L2 prefetch of the same group of this CTA's NEXT tile: the staging ring is all the shared memory that is
-                // left (3 x 18 KB in flight per SM), so the copies should see L2 latency, not loaded-HBM latency
-                if (P.l2_prefetch && cnt > 0 && item + (int64_t)P.l2_prefetch * gridDim.x < n_items) {
-                    const int64_t item2 = item + (int64_t)P.l2_prefetch * gridDim.x;
-                    const int64_t t2 = item2 / P.n_tiles, tile2 = item2 - t2 * P.n_tiles;
-                    const int64_t q0 = tile2 * BM + g * GROUP_ROWS;
-                    int rows2 = P.R - q0 < GROUP_ROWS ? (int)(P.R - q0) : GROUP_ROWS;
-                    if (rows2 < 0) rows2 = 0;
-                    const uint32_t c0 = (uint32_t)q0 / (uint32_t)P.N;
-                    const int m00 = (int)((uint32_t)q0 - c0 * (uint32_t)P.N);
-                    int fc = P.N - m00;
-                    if (fc > rows2) fc = rows2;
-                    const int lr2 = lane == 0 ? 0 : fc + (lane - 1) * P.N;
-                    int cnt2 = lane == 0 ? fc : (rows2 - lr2 < P.N ? rows2 - lr2 : P.N);
-                    if (cnt2 > 0) {
-                        const char* gb = reinterpret_cast<const char*>(P.obs + ep_row(P.ep_index, (int64_t)c0 + lane) * P.obs_sb +
-                                                                       ((t2 + P.t0) * P.N + (lane == 0 ? m00 : 0)) * (int64_t)P.O);
-                        const uintptr_t a0 = (reinterpret_cast<uintptr_t>(gb) + 15) & ~(uintptr_t)15;
-                        const uintptr_t a1 = (reinterpret_cast<uintptr_t>(gb) + (uint64_t)cnt2 * P.O * 4) & ~(uintptr_t)15;
-                        if (a1 > a0)
-                            asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(a0), "r"((uint32_t)(a1 - a0)) : "memory");
-                    }
-                }
-                // row tables, one row per lane: row j belongs to run rj (run 0 holds first_cnt rows, the others N each)
-                const int rj = lane < first_cnt ? 0 : 1 + (lane - first_cnt) / P.N;
-                const int lrj = rj == 0 ? 0 : first_cnt + (rj - 1) * P.N;
-                const uint32_t cur_j = __shfl_sync(0xffffffffu, cur, rj & 31);
-                TADD(10, clock64() - pp0);                         // producer: descriptors of the group (before the slot wait)
-                TWAIT(0, &st_empty[slot], ((git / N_SLOTS) & 1) ^ 1);
-                TMARK(pp1);
-                if (lane < GROUP_ROWS) {
-                    ro[lane] = lane < rows_here ? (int)(cur_j + (uint32_t)(lane - lrj) * P.O * 4u) : -1;   // rows beyond R: zeros
-                    rn[lane] = (rj == 0 ? n00 : 0) + (lane - lrj);
-                }
-                if (cnt > 0) bulk_copy_g2s(sl + cur - phase, ga - phase, cp_bytes, &st_full[slot]);
-                __syncwarp();
-                if (lane == 0) {
-                    if (tx) mbar_arrive_expect_tx(&st_full[slot], tx); else mbar_arrive(&st_full[slot]);
-                }
-                TADD(11, clock64() - pp1);                         // producer: tables, copies, arrival
-            }
-        }
+        fc1_produce<NC, NS>(P, ring, pw, lane, prof_acc);
     } else if (warp >= FIRST_CONV_W) {
         // ===== converters: warp cw owns rows 2cw, 2cw+1 of every group.  Everything that does not depend on the row
         // (which of a lane's two columns per chunk exist, where the one-hot padding columns are) is hoisted: the
         // first version spent ~2400 cycles per group in a serial chain of predicate / address arithmetic. =====
-        const int cw = warp - FIRST_CONV_W;
-        constexpr int c_last = NC - 1;
-        // every column of the chunks before the last exists (O > 64 (NC-1)); the last chunk: per lane
-        const bool okl0 = c_last * BK + 2 * lane < P.O, okl1 = c_last * BK + 2 * lane + 1 < P.O;
-        const int j_pad = c_last * BK + 2 * lane - P.O;       // index of this lane's first column in the K padding
-        const uint32_t a_s_u32 = smem_u32(a_s);
-        const uint32_t a_base = a_s_u32 + ((uint32_t)(lane >> 2) << 4) + (lane & 3) * 4;   // + row*128, ^ swizzle
-        uint32_t git = 0, ti = 0;
-        for (int64_t item = blockIdx.x; item < n_items; item += gridDim.x, ++ti) {
-            for (int g = 0; g < GROUPS; ++g, ++git) {
-                const int slot = git % N_SLOTS;
-                TWAIT(1, &st_full[slot], (git / N_SLOTS) & 1);
-                TMARK(pt1);
-                const uint32_t sl = smem_u32(stage + slot * P.slot_bytes) + 8u * lane;
-                int offs[RPW], nns[RPW];
-#pragma unroll
-                for (int rr = 0; rr < RPW; ++rr) {
-                    offs[rr] = rowoff[slot * GROUP_ROWS + RPW * cw + rr];
-                    nns[rr] = rown[slot * GROUP_ROWS + RPW * cw + rr];
-                }
-                float v0[RPW][NC], v1[RPW][NC];
-                {
-#pragma unroll
-                    for (int rr = 0; rr < RPW; ++rr) {           // all loads first
-                        const int off = offs[rr];
-                        const bool real = off >= 0;
-                        const uint32_t src = sl + (uint32_t)(real ? off : 0);
-#pragma unroll
-                        for (int c = 0; c < NC; ++c) {
-                            v0[rr][c] = 0.f; v1[rr][c] = 0.f;
-                            if (real && (c < c_last || okl0)) v0[rr][c] = lds_f32(src + c * 256);
-                            if (real && (c < c_last || okl1)) v1[rr][c] = lds_f32(src + c * 256 + 4);
-                        }
-                    }
-                    // pack first (consumes every loaded value), release the staging slot, then write the A tile
-                    uint32_t pk[RPW][NC];
-#pragma unroll
-                    for (int rr = 0; rr < RPW; ++rr) {
-                        const int off = offs[rr];
-                        const int nn = nns[rr];
-                        // one-hot(agent) and the bias column live in the K padding of the last chunk
-                        const bool fold = P.fold_id && off >= 0;
-                        const bool hit0 = fold && j_pad >= 0 && (j_pad == nn || j_pad == P.N);
-                        const bool hit1 = fold && j_pad + 1 >= 0 && (j_pad + 1 == nn || j_pad + 1 == P.N);
-#pragma unroll
-                        for (int c = 0; c < NC; ++c) {
-                            float a = v0[rr][c], b = v1[rr][c];
-                            if (c == c_last) { a = hit0 ? 1.0f : a; b = hit1 ? 1.0f : b; }
-                            pk[rr][c] = pack_bf16x2(a, b);
-                        }
-                    }
-                    __syncwarp();
-                    if (lane == 0) mbar_arrive(&st_empty[slot]);
-                    TMARK(pt2);
-                    TADD(6, pt2 - pt1);                            // load + pack phase
-                    // the first group of a tile waits here (values already in registers, slot already released) until
-                    // the MMAs and the image store of the previous tile are done with the A tile
-                    if (g == 0) TWAIT(2, a_free, (ti & 1) ^ 1);
-#pragma unroll
-                    for (int rr = 0; rr < RPW; ++rr) {
-                        const uint32_t rt = (uint32_t)(g * GROUP_ROWS + RPW * cw + rr);
-                        const uint32_t dst = (a_base + rt * 128u) ^ ((rt & 7u) << 4);
-#pragma unroll
-                        for (int c = 0; c < NC; ++c) sts_b32(dst + c * A_STAGE_BYTES, pk[rr][c]);
-                        // the obs image leaves from here too: the warp's 32 words are one full 128-byte line of the image
-                        // (a bulk store of the finished A tile kept the tile busy for ~2500 cycles after the MMAs were
-                        // done with it: the converters of the next tile waited 22 % of the kernel time for it)
-                        if (P.obs_img) {
-                            uint8_t* img = P.obs_img + item * tile_bytes + (dst - a_s_u32);
-#pragma unroll
-                            for (int c = 0; c < NC; ++c) __stcs(reinterpret_cast<uint32_t*>(img + c * A_STAGE_BYTES), pk[rr][c]);
-                        }
-                    }
-                    TADD(7, clock64() - pt2);                      // store phase (includes the a_free wait of group 0)
-                }
-            }
-            fence_proxy_async_smem();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(a_full);
-        }
+        fc1_convert<NC, NS>(P, ring, a_s, a_free, a_full, warp - FIRST_CONV_W, lane, prof_acc);
     } else if (warp == MMA_W) {
         if (lane == 0) {
             const uint32_t idesc = umma_idesc_bf16(BM, 64 * P.n_nets, 0, 0);
@@ -907,18 +961,235 @@ __global__ void __launch_bounds__(fs::threads_for(NS), 1) fc1_stream_kernel(Fc1S
             a_prev = a_next; n_cur = n_nxt;
         }
     }
-#ifdef PMB_FC1_PROFILE
-    if (lane == 0) {
-        for (int i = 0; i < 8; ++i) if (prof_acc[i]) atomicAdd(&g_fc1_prof[i], (unsigned long long)prof_acc[i]);
-        for (int i = 10; i < 12; ++i) if (prof_acc[i]) atomicAdd(&g_fc1_prof[i], (unsigned long long)prof_acc[i]);
-        if (threadIdx.x == 0) { atomicAdd(&g_fc1_prof[8], (unsigned long long)(clock64() - prof_t0)); atomicAdd(&g_fc1_prof[9], 1ull); }
-    }
-#endif
+    FC1_PROF_END(NS);
     tc_fence_before();
     __syncthreads();
     if (warp == MMA_W) {
         tc_fence_after();
         tmem_dealloc(tmem_base, 256);
+    }
+}
+
+
+// ------------------------------------------------------------------------------------------
+// Learner fc1 of both nets with the weights in TENSOR memory.  The MMA runs transposed,
+//   D[hidden, row] = W_tmem[hidden, k] . obs[row, k]^T     (M = 128 hidden units of both nets, N = 128 rows)
+// so W (80 KB at K = 320) leaves shared memory; the obs tile is the B operand with the bytes and descriptor the
+// A operand has in fc1_stream_kernel.  TMEM: [0, 256) two accumulators, [256, 256 + 32 NC) W.  The freed shared
+// memory holds a five-slot staging ring (fc1_stream_kernel: three), the last-action table and a 2 x 16 KB stage
+// from which each net's x tile leaves as ONE bulk store.  Producers and converters are those of fc1_stream_kernel.
+// Epilogue: thread = (net, hidden unit) = accumulator lane, its 32 registers of a column block = 32 rows.
+// fold_id only (the agent id / bias come in through the K padding), two nets only.
+// ------------------------------------------------------------------------------------------
+namespace fs {
+constexpr int N_SLOTS_TS = 5;
+constexpr int TS_TMEM_W = 256;            // first TMEM column of W
+}  // namespace fs
+
+__device__ __forceinline__ void epi_bar_sync() { asm volatile("bar.sync 1, 128;" ::: "memory"); }   // the 4 epilogue warps
+
+template <int NC>
+__global__ void __launch_bounds__(fs::threads_for(fs::N_SLOTS_TS), 1) fc1_stream_ts_kernel(Fc1StreamParams P) {
+    FC1_PROF_BEGIN;
+    using namespace fs;
+    constexpr int NS = N_SLOTS_TS, FIRST_CONV_W = PROD_W + NS;
+    extern __shared__ uint8_t smem_raw[];
+    uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
+    uint8_t* a_s = smem;                                    // [NC][16 KB] obs tile (B operand)
+    uint8_t* xs = a_s + NC * A_STAGE_BYTES;                 // [net 2][16 KB] x tile images
+    uint8_t* stage = xs + 2 * A_STAGE_BYTES;                // [NS][slot_bytes]
+    float* tab_s = reinterpret_cast<float*>(stage + NS * P.slot_bytes);     // [A][128]: fc1.weight[h][O + a] of both nets
+    int* prev_s = reinterpret_cast<int*>(tab_s + P.n_act * 128);            // [2][128] previous action of the tile's rows
+    int* rowoff = prev_s + 2 * BM;
+    int* rown = rowoff + NS * GROUP_ROWS;
+    uint64_t* bars = reinterpret_cast<uint64_t*>(rown + NS * GROUP_ROWS);
+    uint64_t* w_full = bars;                 // W is in TMEM (arrivals of the 4 epilogue warps)
+    uint64_t* st_full = bars + 1;            // [NS]
+    uint64_t* st_empty = st_full + NS;       // [NS]
+    uint64_t* a_full = st_empty + NS;
+    uint64_t* a_free = a_full + 1;
+    uint64_t* tfull = a_free + 1;            // [2]
+    uint64_t* tempty = tfull + 2;            // [2]
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty + 2);
+
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    if (threadIdx.x == 0) {
+        mbar_init(w_full, N_EPI);
+        for (int i = 0; i < NS; ++i) { mbar_init(&st_full[i], 1); mbar_init(&st_empty[i], N_CONV); }
+        mbar_init(a_full, N_CONV); mbar_init(a_free, 1);
+        for (int i = 0; i < 2; ++i) { mbar_init(&tfull[i], 1); mbar_init(&tempty[i], N_EPI); }
+        fence_barrier_init();
+    }
+    if (warp == MMA_W) tmem_alloc(tmem_slot, 512);
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    // (TMEM base and item count are read inside the roles: held across the role branch they spill at 112 registers)
+    const Fc1Ring ring{stage, rowoff, rown, st_full, st_empty};
+
+    if (warp >= PROD_W && warp < PROD_W + NS) {
+        fc1_produce<NC, NS>(P, ring, warp - PROD_W, lane, prof_acc);
+    } else if (warp >= FIRST_CONV_W) {
+        fc1_convert<NC, NS>(P, ring, a_s, a_free, a_full, warp - FIRST_CONV_W, lane, prof_acc);
+    } else if (warp == MMA_W) {
+        if (lane == 0) {
+            const uint32_t tmem_base = *tmem_slot;
+            const int64_t n_items = (int64_t)P.T * P.n_tiles;
+            const uint32_t idesc = umma_idesc_bf16(BM, BM, 0, 0);
+            mbar_wait(w_full, 0);
+            tc_fence_after();
+            uint32_t ti = 0;
+            for (int64_t item = blockIdx.x; item < n_items; item += gridDim.x, ++ti) {
+                const int b = ti & 1;
+                TWAIT(3, a_full, ti & 1);
+                TWAIT(4, &tempty[b], ((ti >> 1) & 1) ^ 1);
+                tc_fence_after();
+                const uint32_t tm = tmem_base + 128u * b;
+#pragma unroll
+                for (int c = 0; c < NC; ++c) {
+                    const uint32_t a_addr = smem_u32(a_s + c * A_STAGE_BYTES);
+#pragma unroll
+                    for (int kk = 0; kk < BK / 16; ++kk)
+                        umma_bf16_ts(tm, tmem_base + TS_TMEM_W + (uint32_t)(c * (BK / 16) + kk) * 8u,
+                                     umma_desc_sw128(a_addr + kk * 32, 16, 1024), idesc, (c | kk) != 0);
+                }
+                umma_commit(a_free);
+                umma_commit(&tfull[b]);
+            }
+        }
+    } else {
+        // ===== epilogue: warp w reads accumulator lanes 32w .. 32w + 31 (its TMEM lane quarter) =====
+        const int hl = warp * 32 + lane;                      // accumulator lane: online hidden 0-63 | target 64-127
+        const int net = warp >> 1;
+        const uint32_t tmem_base = *tmem_slot;
+        const int64_t n_items = (int64_t)P.T * P.n_tiles;
+        TMARK(pe0);
+        // W rows of this thread's hidden unit into TMEM: the packed image's 128-byte row, un-swizzled, is 32 columns
+        {
+            const uint8_t* wrow = reinterpret_cast<const uint8_t*>(P.Wp) + hl * 128;
+#pragma unroll
+            for (int c = 0; c < NC; ++c) {
+                uint32_t v[32];
+#pragma unroll
+                for (int j = 0; j < 8; ++j) {
+                    const uint4 u = __ldg(reinterpret_cast<const uint4*>(wrow + c * A_STAGE_BYTES + ((j ^ (hl & 7)) << 4)));
+                    v[4 * j] = u.x; v[4 * j + 1] = u.y; v[4 * j + 2] = u.z; v[4 * j + 3] = u.w;
+                }
+                tmem_st_32x32(tmem_base + TS_TMEM_W + 32u * c + ((uint32_t)(warp * 32) << 16), v);
+            }
+            tmem_wait_st();
+            tc_fence_before();
+            __syncwarp();
+            if (lane == 0) mbar_arrive(w_full);
+        }
+        {
+            const uint16_t* ta = reinterpret_cast<const uint16_t*>(P.tab_act16);
+            for (int i = hl; i < P.n_act * 128; i += 128) tab_s[i] = __uint_as_float((uint32_t)__ldg(ta + i) << 16);
+        }
+        TADD(14, clock64() - pe0);                             // epilogue: W into TMEM, table into shared memory
+        // the previous action of row hl of an item (-1: none / step not filled, -2: padding row)
+        auto fetch_prev = [&](int64_t item) {
+            if (item >= n_items) return -2;
+            const int64_t t = item / P.n_tiles, tile = item - t * P.n_tiles;
+            const int64_t p = tile * BM + hl;
+            if (p >= P.R) return -2;
+            const int64_t b = p / P.N;
+            const int n = (int)(p - b * P.N);
+            const int64_t tb = t + P.t0;
+            if (!P.use_act || tb == 0) return -1;
+            const int64_t be = ep_row(P.ep_index, b);
+            const int64_t f = __ldg(P.filled + be * P.filled_sb + (tb - 1));
+            const int a = (int)__ldg(P.actions + be * P.actions_sb + (tb - 1) * P.N + n);
+            return f != 0 ? a : -1;
+        };
+        int a_prev = fetch_prev(blockIdx.x);
+        const uint32_t xs_u32 = smem_u32(xs + net * A_STAGE_BYTES);
+        const uint32_t h2 = (uint32_t)(hl & 62);                // even hidden unit of the pair this lane stores
+        const uint32_t xs_lane = xs_u32 + (h2 & 7) * 2;
+        const uint32_t tab_u32 = smem_u32(tab_s + hl);
+        uint32_t ti = 0;
+        for (int64_t item = blockIdx.x; item < n_items; item += gridDim.x, ++ti) {
+            const int b = ti & 1;
+            const int a_next = fetch_prev(item + gridDim.x);
+            const uint32_t pv_u32 = smem_u32(prev_s + b * BM);
+            prev_s[b * BM + hl] = a_prev;
+            TMARK(pe1);
+            if (threadIdx.x == 0) bulk_wait_group_read<0>();    // the x stage of the previous item has been read
+            epi_bar_sync();
+            TADD(12, clock64() - pe1);                         // epilogue: stage free + prev table barrier
+            TWAIT(5, &tfull[b], (ti >> 1) & 1);
+            tc_fence_after();
+            TMARK(pe2);
+            const int64_t tile = item % P.n_tiles;
+            const int rows_valid = P.R - tile * BM < BM ? (int)(P.R - tile * BM) : BM;
+            const uint32_t taddr = tmem_base + 128u * b + ((uint32_t)(warp * 32) << 16);
+#pragma unroll 1
+            for (int g = 0; g < 4; ++g) {                      // 32 accumulator columns = rows 32g .. 32g + 31
+                uint32_t v[32];
+                tmem_ld_32x32(taddr + 32 * g, v);
+                tmem_wait_ld();
+                if (g == 3) {                                  // the accumulator buffer is free for the tile after next
+                    tc_fence_before();
+                    __syncwarp();
+                    if (lane == 0) mbar_arrive(&tempty[b]);
+                }
+                // (explicit shared-space loads, no branches: generic loads and a branch per row made this loop a serial
+                // chain of ~100 cycles per row)
+                int pa[32];
+#pragma unroll
+                for (int q = 0; q < 8; ++q) {
+                    int4 p4;
+                    asm volatile("ld.shared.v4.s32 {%0, %1, %2, %3}, [%4];"
+                                 : "=r"(p4.x), "=r"(p4.y), "=r"(p4.z), "=r"(p4.w) : "r"(pv_u32 + (uint32_t)(32 * g + 4 * q) * 4u));
+                    pa[4 * q] = p4.x; pa[4 * q + 1] = p4.y; pa[4 * q + 2] = p4.z; pa[4 * q + 3] = p4.w;
+                }
+                float o[32];
+                uint32_t mword = 0;
+#pragma unroll
+                for (int e = 0; e < 32; ++e) {
+                    const int a = pa[e];
+                    const float t = lds_f32(tab_u32 + (uint32_t)(a > 0 ? a : 0) * 512u);
+                    float x = __uint_as_float(v[e]);
+                    x = a >= 0 ? x + t : x;
+                    x = fmaxf(x, 0.f);
+                    o[e] = x;
+                    // the online net's ReLU word of (row, half) is the warp's vote: bit j = hidden unit 32 half + j
+                    const uint32_t bal = __ballot_sync(0xffffffffu, x > 0.f);
+                    mword = lane == e ? bal : mword;
+                }
+                if (net == 0 && P.relu_mask && 32 * g + lane < rows_valid)
+                    P.relu_mask[(item * 2 + warp) * 128 + 32 * g + lane] = mword;
+                // bf16 pairs of adjacent hidden units: the even lane stores row e, the odd lane row e + 4 (the two rows
+                // fall on disjoint 16-byte chunks of the swizzle, so the 32 stores of a step hit 32 banks)
+#pragma unroll
+                for (int e = 0; e < 32; ++e) {
+                    if (e & 4) continue;
+                    const bool odd = lane & 1;
+                    const float send = odd ? o[e] : o[e + 4];
+                    const float recv = __shfl_xor_sync(0xffffffffu, send, 1);
+                    const uint32_t w = odd ? pack_bf16x2(recv, o[e + 4]) : pack_bf16x2(o[e], recv);
+                    const uint32_t row = (uint32_t)(32 * g + e + (odd ? 4 : 0));
+                    sts_b32(xs_lane + sw128_offset(row, h2 >> 3), w);
+                }
+            }
+            fence_proxy_async_smem();
+            epi_bar_sync();
+            if (threadIdx.x == 0) {
+                bulk_copy_s2g(P.x_on + item * A_STAGE_BYTES, xs, (uint32_t)rows_valid * 128u);
+                bulk_copy_s2g(P.x_tg + item * A_STAGE_BYTES, xs + A_STAGE_BYTES, (uint32_t)rows_valid * 128u);
+                bulk_commit_group();
+            }
+            TADD(13, clock64() - pe2);                         // epilogue: TMEM loads, tables, ReLU, mask, x stage
+            a_prev = a_next;
+        }
+        if (threadIdx.x == 0) bulk_wait_group<0>();
+    }
+    FC1_PROF_END(NS);
+    tc_fence_before();
+    __syncthreads();
+    if (warp == MMA_W) {
+        tc_fence_after();
+        tmem_dealloc(*tmem_slot, 512);
     }
 }
 
@@ -1105,7 +1376,7 @@ int tc_fc1_fwd_both(const pmb_dims* d, const pmb_batch* b, int t0, int nt, const
             Q.actions = b->actions; Q.actions_sb = b->actions_sb; Q.filled = b->filled; Q.filled_sb = b->filled_sb;
             Q.x_on = reinterpret_cast<uint8_t*>(x_on); Q.x_tg = reinterpret_cast<uint8_t*>(x_tg);
             Q.relu_mask = relu_mask; Q.use_act = d->obs_last_action;
-            Q.n_nets = x_tg ? 2 : 1; Q.t0 = t0;
+            Q.n_nets = x_tg ? 2 : 1; Q.t0 = t0; Q.n_act = d->A;
             // L2 prefetch of the CTA's next tile(s): measured (round 2, same box, alternating) as a LOSS - rollout step 0.196 ms
             // with one tile ahead, 0.217 ms with two, 0.190 ms without; learner fc1 8.1-8.4 / 8.8 / 8.0 ms - the copies of the
             // ring already keep the memory system busy and the prefetch instructions cost the producers issue time.
@@ -1119,9 +1390,19 @@ int tc_fc1_fwd_both(const pmb_dims* d, const pmb_batch* b, int t0, int nt, const
             const int64_t smem_1net = 1024 + (int64_t)n_chunks * (tc::A_STAGE_BYTES / 2) + (int64_t)n_chunks * tc::A_STAGE_BYTES +
                                       tc::fs::N_SLOTS_1NET * (int64_t)slot_bytes + 2 * tc::fs::N_SLOTS_1NET * tc::fs::GROUP_ROWS * 4 + 256;
             const bool wide_ring = Q.n_nets == 1 && smem_1net <= 232448;
+            // learner step: W of both nets in tensor memory (fc1_stream_ts_kernel) when the agent id is folded into the K
+            // padding and its ring, x stage and last-action table fit; PMB_FC1_TS=0 selects fc1_stream_kernel (A/B switch,
+            // read on every call so that one process can run both)
+            const int64_t smem_ts = 1024 + (int64_t)(n_chunks + 2) * tc::A_STAGE_BYTES + tc::fs::N_SLOTS_TS * (int64_t)slot_bytes +
+                                    (int64_t)d->A * 128 * 4 + 2 * tc::BM * 4 + 2 * tc::fs::N_SLOTS_TS * tc::fs::GROUP_ROWS * 4 + 256;
+            const char* e_ts = getenv("PMB_FC1_TS");
+            const bool use_ts = Q.n_nets == 2 && fold_id && smem_ts <= 232448 && !(e_ts && e_ts[0] == '0');
 #define PMB_FC1_STREAM_LAUNCH(NC)                                                                                            \
     case NC:                                                                                                                 \
-        if (wide_ring) {                                                                                                     \
+        if (use_ts) {                                                                                                        \
+            PMB_SMEM_ATTR((tc::fc1_stream_ts_kernel<NC>), (int)smem_ts);                                                     \
+            tc::fc1_stream_ts_kernel<NC><<<grid, tc::fs::threads_for(tc::fs::N_SLOTS_TS), (size_t)smem_ts, s>>>(Q);          \
+        } else if (wide_ring) {                                                                                              \
             PMB_SMEM_ATTR((tc::fc1_stream_kernel<NC, tc::fs::N_SLOTS_1NET>), (int)smem_1net);                               \
             PMB_CUDA(launch_pdl(tc::fc1_stream_kernel<NC, tc::fs::N_SLOTS_1NET>, dim3(grid),                                 \
                                 dim3(tc::fs::threads_for(tc::fs::N_SLOTS_1NET)), (size_t)smem_1net, s, rollout_pdl_enabled(), Q)); \

@@ -1,4 +1,5 @@
-"""Per-role wait profile of fc1_stream_kernel.  Needs a library built with
+"""Per-role wait profile of the learner's streaming fc1 kernel (fc1_stream_ts_kernel, or fc1_stream_kernel with
+PMB_FC1_TS=0).  Needs a library built with
 PMB_EXTRA_NVCC_FLAGS=-DPMB_FC1_PROFILE python -c 'from pymarl_b200.build import build; build(force=True)'."""
 import sys, os, ctypes as C
 _ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -30,9 +31,14 @@ lib.pmb_debug_fc1_prof(out, 1)
 v = list(out)
 n_cta = v[9]
 tot = v[8] / n_cta
-names = ["producer: st_empty (x3 warps)", "converter: st_full (x8 warps)", "converter: a_free (x8)", "MMA: a_full", "MMA: tempty",
-         "epilogue: tfull (x4)", "converter: load + pack phase (x8)", "converter: store phase incl. a_free (x8)"]
-mult = [3, 8, 8, 1, 1, 4, 8, 8]
-print("CTAs", n_cta, "cycles per CTA", round(tot))
-for i, (nm, m) in enumerate(zip(names, mult)):
-    print(f"{nm:34s} {v[i] / n_cta / m / tot * 100:6.1f} % of the kernel time per warp")
+n_prod = round(v[15] / n_cta)                  # producer warps = staging slots
+# (slot, name, warps of the role); per warp: cycles over the kernel's cycles
+rows = [(0, "producer: st_empty", n_prod), (10, "producer: descriptors", n_prod), (11, "producer: tables + copies", n_prod),
+        (1, "converter: st_full", 8), (6, "converter: load + pack", 8), (7, "converter: store incl. a_free", 8),
+        (2, "converter: a_free", 8), (3, "MMA: a_full", 1), (4, "MMA: tempty", 1), (5, "epilogue: tfull", 4),
+        (12, "epilogue: x stage free + barrier", 4), (13, "epilogue: work incl. x bulk stores", 4),
+        (14, "epilogue: W into TMEM (once)", 4)]
+print("CTAs", n_cta, "cycles per CTA", round(tot), "staging slots", n_prod)
+for i, nm, m in rows:
+    if v[i]:
+        print(f"{nm:38s} {v[i] / n_cta / m / tot * 100:6.1f} % of the kernel time per warp")
