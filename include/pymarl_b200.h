@@ -63,7 +63,17 @@ typedef struct pmb_dims {
     int32_t precision;         /* enum pmb_precision                                      */
     int32_t reserved;          /* flags.  bit 0 (pmb_select_actions_step, tensor-core tier only): the packed weight
                                 * images a previous call left in `scratch` are still current - same parameters, same
-                                * scratch - so the step skips its two weight-pack launches.  0 is always safe.      */
+                                * scratch - so the step skips its two weight-pack launches.
+                                * bit 1 (pmb_qlearner_train_step): skip the padded timesteps of a ragged batch.  The step
+                                * sorts the episodes on the device by the forward steps they need (F_b = min(T, l_b + 2),
+                                * l_b = last t with filled = 1; 0 for an empty episode), longest first and stable, and the
+                                * agent kernels (fc1, both recurrences, fc2 + target selection, BPTT, fc1/fc2 weight
+                                * gradients) run only the (t, 128-row tile) items some row of the tile still needs.  Loss
+                                * sums and gradients are those of the unsorted step up to fp32 summation order.  Honoured
+                                * where batch.ep_index is (bf16 tier, H = 64, A <= 64, QMIX with E = 32 or VDN / IQL,
+                                * O <= 320, agent id folding into the K padding of obs); elsewhere ignored, and the step is
+                                * bit-identical to the step without it.  pmb_learner_workspace_bytes counts the schedule
+                                * area only where the bit is honoured.  0 is always safe.                             */
 } pmb_dims;
 
 /* The EpisodeBatch fields the path reads.  *_sb = batch stride in ELEMENTS. */
@@ -105,7 +115,9 @@ typedef struct pmb_hparams {
     int32_t skip_update;             /* 1: stop after the gradients (multi-GPU: all-reduce, then pmb_clip_rmsprop_update) */
     int32_t keep_q;                  /* debug bits (tests): 1 = bf16 tier also writes the Q tensors (mac_out) into the
                                       * workspace; 2 = stop after the forward pass and the loss sums (q_learner.py:39-97),
-                                      * leaving every forward intermediate in the workspace */
+                                      * leaving every forward intermediate in the workspace.  With padded-step skipping
+                                      * (pmb_dims.reserved bit 1) the Q tensors are unspecified on the skipped (t, tile)
+                                      * items, and chosen / tmax are 0 there */
 } pmb_hparams;
 
 /* stats buffer: 16 doubles on the device, written by the step */
@@ -356,6 +368,9 @@ typedef struct pmb_ws_views {
     float* state_img;          /* bf16 tier: state tile images shared by both mixers and the hypernet weight gradients */
     float* h_tg;               /* bf16 tier: h tile images of the target net */
     float* relu_mask;          /* bf16 tier: bit mask (x > 0) of the online fc1 output */
+    /* padded-step skipping (pmb_dims.reserved bit 1), NULL where the bit is not honoured: written by the step */
+    int64_t* ep_order;         /* [B] buffer episode of sorted batch row b (the incoming ep_index composed with the sort) */
+    int32_t* tile_steps;       /* [ceil(B N / 128)] forward steps run for each 128-row tile of the sorted rows */
 } pmb_ws_views;
 int pmb_learner_workspace_views(const pmb_dims* d, void* workspace, int64_t workspace_bytes, pmb_ws_views* out);
 

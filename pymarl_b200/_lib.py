@@ -72,7 +72,9 @@ class WsViews(C.Structure):
               "q_tot", "t_tot", "g", "d_chosen", "scratch")
     _fields_ = [(k, C.c_void_p) for k in _names] + [("scratch_bytes", C.c_int64), ("obs_img", C.c_void_p),
                                                         ("state_img", C.c_void_p), ("h_tg", C.c_void_p),
-                                                        ("relu_mask", C.c_void_p)]
+                                                        ("relu_mask", C.c_void_p),
+                                                        # padded-step skipping (NULL where pmb_dims.reserved bit 1 is not honoured)
+                                                        ("ep_order", C.c_void_p), ("tile_steps", C.c_void_p)]
 
 
 class PmbError(RuntimeError):
@@ -195,11 +197,14 @@ def require_cuda(t, name):
 
 
 def make_dims(B, T, N, O, S, A, H, E, obs_last_action=True, obs_agent_id=True, mixer="qmix", double_q=True,
-              precision="fp32"):
+              precision="fp32", skip_padding=False):
+    """skip_padding sets pmb_dims.reserved bit 1: the learner step skips the padded timesteps of a ragged batch where
+    the fused tensor-core path runs (see include/pymarl_b200.h); elsewhere the bit is ignored."""
     if mixer not in MIXER_IDS:
         raise ValueError("Mixer {} not recognised.".format(mixer))       # learners/q_learner.py:26
     return Dims(int(B), int(T), int(N), int(O), int(S), int(A), int(H), int(E), int(bool(obs_last_action)),
-                int(bool(obs_agent_id)), MIXER_IDS[mixer], int(bool(double_q)), PREC_IDS[precision], 0)
+                int(bool(obs_agent_id)), MIXER_IDS[mixer], int(bool(double_q)), PREC_IDS[precision],
+                2 if skip_padding else 0)
 
 
 def flat_layout(dims):

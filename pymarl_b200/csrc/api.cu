@@ -65,7 +65,7 @@ int tc_gemm_plain(const float* A, RowMap amap, int64_t M, int K, const __nv_bflo
                   const float* bias, float* C, int64_t ldc, cudaStream_t s);
 int tc_fc1_fwd_both(const pmb_dims* d, const pmb_batch* b, int t0, int nt, const AgentParams& on, const AgentParams& tg,
                     float* x_on, float* x_tg, int tile_images, uint8_t* obs_img_out, uint32_t* relu_mask, void* scratch,
-                    int64_t scratch_bytes, cudaStream_t s, int weights_packed = 0);
+                    int64_t scratch_bytes, cudaStream_t s, int weights_packed = 0, const int32_t* live_items = nullptr);
 // tc_atb.cu (tile-image D operand)
 int tc_gemm_atb_ti(const uint8_t* d_ti, int T, int N, int64_t R, int n_tiles, const float* A, RowMap amap, int K,
                    float* out, int64_t ldo, float* bias_out, void* scratch, int64_t scratch_bytes, cudaStream_t s);
@@ -205,8 +205,21 @@ struct WsPlan {
     int64_t off[18];
     int64_t scratch_bytes;
     int64_t mixdw_bytes;
+    int64_t sched_bytes;           // the padded-step skipping schedule (0 when pmb_dims.reserved bit 1 is not honoured)
     int64_t total;
 };
+
+// The fused tensor-core path: tcgen05 agent kernels, the image-fed QMIX mixer (VDN and IQL need none), the streaming fc1
+// kernel (obs dim <= 320) with one-hot(agent) + ones folded into the K padding.  Zero-copy replay sampling (ep_index)
+// and padded-step skipping need it.
+bool fused_tc_path(const pmb_dims* d) {
+    const bool tc_agent = d->precision == PMB_PREC_BF16 && d->H == 64 && d->A <= 64;
+    const bool tc_mixer = d->precision == PMB_PREC_BF16 && d->mixer == PMB_MIXER_QMIX && d->E == 32;
+    return tc_agent && (d->mixer != PMB_MIXER_QMIX || tc_mixer) && d->O <= 320 && ((d->O + 63) / 64) * 64 - d->O >= d->N + 1;
+}
+
+// pmb_dims.reserved bit 1 (pmb_qlearner_train_step): skip the padded steps of a ragged batch.  Ignored off the fused path.
+bool skip_padding(const pmb_dims* d) { return (d->reserved & 2) && fused_tc_path(d); }
 
 int64_t agent_bwd_scratch(const pmb_dims* d) {
     const int64_t rows = (int64_t)d->T * d->B * d->N;
@@ -279,7 +292,8 @@ WsPlan plan_workspace(const pmb_dims* d) {
     // behind the scratch area: the slice partials of the hypernet weight-gradient GEMM when it runs on the side stream next
     // to the agent's BPTT (which owns the scratch area then)
     p.mixdw_bytes = (tc_mix && d->H == 64) ? tc_mixer_dw_scratch_bytes(d) : 0;
-    p.total = off + p.scratch_bytes + p.mixdw_bytes;
+    p.sched_bytes = skip_padding(d) ? skip_schedule_bytes(d->B, d->T, (int)n_tiles) : 0;
+    p.total = off + p.scratch_bytes + p.mixdw_bytes + p.sched_bytes;
     return p;
 }
 
@@ -299,6 +313,13 @@ void fill_views(const pmb_dims* d, void* ws, const WsPlan& p, pmb_ws_views* v) {
     v->h_tg = f(15);
     v->scratch_bytes = p.scratch_bytes;
     v->obs_img = f(9);
+    v->ep_order = nullptr;
+    v->tile_steps = nullptr;
+    if (p.sched_bytes) {
+        SkipSchedule S = skip_schedule_views(base + p.total - p.sched_bytes, d->B, d->T, (int)ceil_div((int64_t)d->B * d->N, 128));
+        v->ep_order = S.ep_order;
+        v->tile_steps = S.tile_steps;
+    }
 }
 
 int fc1_fwd(const pmb_dims* d, const pmb_batch* b, int t0, int nt, const AgentParams& ap, float* x_out,
@@ -688,10 +709,19 @@ int pmb_qlearner_train_step(const pmb_dims* d, const pmb_batch* b, const pmb_hpa
     // q_learner.py:47-52 / 58-62: both nets over all T steps
     const bool tc_agent = d->precision == PMB_PREC_BF16 && d->H == 64 && d->A <= 64;
     const bool tc_mixer = d->precision == PMB_PREC_BF16 && d->mixer == PMB_MIXER_QMIX && d->E == 32;
-    PMB_REQUIRE(b->ep_index == nullptr || (tc_agent && (d->mixer != PMB_MIXER_QMIX || tc_mixer) && d->O <= 320 &&
-                                           ((d->O + 63) / 64) * 64 - d->O >= d->N + 1),
+    PMB_REQUIRE(b->ep_index == nullptr || fused_tc_path(d),
                 "train_step: batch.ep_index (zero-copy replay sampling) needs the tensor-core tier with the fused kernels");
     const int n_tiles = (int)ceil_div(R, 128);
+    // Padded-step skipping: sort the episodes by the steps they need (longest first) on the device; from here on the step
+    // reads the batch in that order (ep_order composes the incoming ep_index), and the agent kernels walk the live
+    // (t, tile) items only.  Launch sizes stay those of the full rectangle.
+    pmb_batch sorted_batch;
+    SkipSchedule sched{};
+    const bool skip = skip_padding(d);
+    if (skip) sched = skip_schedule_views(static_cast<char*>(workspace) + plan.total - plan.sched_bytes, d->B, d->T, n_tiles);
+    const int32_t* live_items = skip ? sched.items : nullptr;
+    const int32_t* n_live = skip ? sched.n_items : nullptr;
+    const int32_t* tile_steps = skip ? sched.tile_steps : nullptr;
     uint8_t *x_on_ti = reinterpret_cast<uint8_t*>(v.x_on), *x_tg_ti = reinterpret_cast<uint8_t*>(v.x_tg);
     uint8_t *h_ti = reinterpret_cast<uint8_t*>(v.h_stash), *g_ti = reinterpret_cast<uint8_t*>(v.gates);
     uint8_t* hg_ti = reinterpret_cast<uint8_t*>(v.h_tg);
@@ -705,9 +735,17 @@ int pmb_qlearner_train_step(const pmb_dims* d, const pmb_batch* b, const pmb_hpa
     if (tc_agent) {
         if ((rc = tc_ti_zero_pad(x_on_ti, d->T, n_tiles, R, s))) return rc;
         if ((rc = tc_ti_zero_pad(x_tg_ti, d->T, n_tiles, R, s))) return rc;
+        if (skip) {                                      // (skip implies the tensor-core agent)
+            PHASE(s, "skip_schedule");
+            if ((rc = tc_skip_schedule(d, b, sched, n_tiles, s))) return rc;
+            sorted_batch = *b;
+            sorted_batch.ep_index = sched.ep_order;
+            b = &sorted_batch;
+        }
         PHASE(s, "fc1_fwd_both_tc");
         if ((rc = tc_fc1_fwd_both(d, b, 0, d->T, on, tg, v.x_on, v.x_tg, 1, fused_dw ? obs_ti : nullptr,
-                                  reinterpret_cast<uint32_t*>(v.relu_mask), v.scratch, v.scratch_bytes, s))) return rc;
+                                  reinterpret_cast<uint32_t*>(v.relu_mask), v.scratch, v.scratch_bytes, s, 0, live_items)))
+            return rc;
         // The two recurrences are independent.  Each runs ceil(n_tiles / 2) CTAs (one per SM): when both fit on the device
         // at once (small configs, or a batch sharded over many GPUs) the target net's pass is forked onto a side stream and
         // the two chains of T dependent steps run side by side instead of back to back.
@@ -726,21 +764,23 @@ int pmb_qlearner_train_step(const pmb_dims* d, const pmb_batch* b, const pmb_hpa
             PMB_CUDA(cudaEventRecord(side->fork, s));
             PMB_CUDA(cudaStreamWaitEvent(side->stream, side->fork, 0));
             if ((rc = tc_gru_fwd2(img(57344), img(57344 + 24576), tg.b_ih, tg.b_hh, x_tg_ti, hg_ti, nullptr, R, d->T, n_tiles,
-                                  side->stream, tpc))) return rc;
+                                  side->stream, tpc, tile_steps))) return rc;
             PMB_CUDA(cudaEventRecord(side->join, side->stream));
         }
-        if ((rc = tc_gru_fwd2(img(0), img(24576), on.b_ih, on.b_hh, x_on_ti, h_ti, g_ti, R, d->T, n_tiles, s, tpc))) return rc;
+        if ((rc = tc_gru_fwd2(img(0), img(24576), on.b_ih, on.b_hh, x_on_ti, h_ti, g_ti, R, d->T, n_tiles, s, tpc, tile_steps)))
+            return rc;
         if (fork_tg) {
             PMB_CUDA(cudaStreamWaitEvent(s, side->join, 0));
         } else {
             PHASE(s, "gru_unroll_fwd_target_tc");
             if ((rc = tc_gru_fwd2(img(57344), img(57344 + 24576), tg.b_ih, tg.b_hh, x_tg_ti, hg_ti, nullptr, R, d->T, n_tiles,
-                                  s))) return rc;
+                                  s, 2, tile_steps))) return rc;
         }
         // :55-78 fused with fc2 of both nets
         PHASE(s, "q_select_tc");
         if ((rc = tc_q_select(d, b, img(49152), img(57344 + 49152), on.fc2_b, tg.fc2_b, h_ti, hg_ti, n_tiles, v.chosen,
-                              v.tmax, (hp->keep_q & 1) ? v.q_on : nullptr, (hp->keep_q & 1) ? v.q_tg : nullptr, s))) return rc;
+                              v.tmax, (hp->keep_q & 1) ? v.q_on : nullptr, (hp->keep_q & 1) ? v.q_tg : nullptr, s, live_items,
+                              n_live, tile_steps))) return rc;
     } else {
         PHASE(s, "fc1_fwd_online");
         if ((rc = fc1_fwd(d, b, 0, d->T, on, v.x_on, s))) return rc;
@@ -824,13 +864,13 @@ int pmb_qlearner_train_step(const pmb_dims* d, const pmb_batch* b, const pmb_hpa
         auto img = [&](int64_t off) { return reinterpret_cast<const __nv_bfloat16*>(gru_img + off); };
         if ((rc = tc_gru_bwd2(img(0), img(24576), img(49152), x_on_ti, h_ti, g_ti, x_tg_ti,
                               reinterpret_cast<const uint32_t*>(v.relu_mask), v.d_chosen, b->actions, b->actions_sb, b->ep_index,
-                              R, d->T, d->N, d->A, n_tiles, rnn_part, s))) return rc;
+                              R, d->T, d->N, d->A, n_tiles, rnn_part, s, tile_steps))) return rc;
         PHASE(s, "dW_rnn_tc");
         if ((rc = tc_gru_bwd2_reduce(rnn_part, n_tiles, gr.w_ih, gr.w_hh, gr.b_ih, gr.b_hh, s))) return rc;
         if (fused_dw) {
             PHASE(s, "dW_fc1_fc2_tc");
             if ((rc = tc_agent_dw(d, b, x_tg_ti, h_ti, obs_ti, v.d_chosen, n_tiles, gr.fc1_w, gr.fc1_b, gr.fc2_w, gr.fc2_b,
-                                  v.scratch, v.scratch_bytes, s))) return rc;
+                                  v.scratch, v.scratch_bytes, s, live_items, n_live))) return rc;
         } else {
             PHASE(s, "dW_fc1_tc");
             RowMap omap{b->obs_sb, (int64_t)d->N * d->O, (int64_t)d->O, d->T, d->N};

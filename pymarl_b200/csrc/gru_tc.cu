@@ -669,6 +669,11 @@ struct AgentDwParams {
     float* partial;
     int64_t R, n_items, items_per_cta;
     int T, N, A, n_tiles, n_chunks, use_act, use_id;
+    // optional (padded-step skipping): the (t, tile) items are live[0 .. *n_live) (t * n_tiles + tile), each two half
+    // items; the split over the grid is then computed here from the device count.  The list must hold every live item
+    // and nothing else: the dpre1 images of the other items are stale x values of the target net.
+    const int32_t* live;
+    const int32_t* n_live;
 };
 
 __global__ void __launch_bounds__(ad::THREADS, 1) agent_dw_tc_kernel(AgentDwParams P) {
@@ -695,8 +700,10 @@ __global__ void __launch_bounds__(ad::THREADS, 1) agent_dw_tc_kernel(AgentDwPara
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
-    const int64_t beg = (int64_t)blockIdx.x * P.items_per_cta;
-    const int64_t end = beg + P.items_per_cta < P.n_items ? beg + P.items_per_cta : P.n_items;
+    const int64_t n_items = P.live ? 2 * (int64_t)__ldg(P.n_live) : P.n_items;
+    const int64_t items_per_cta = P.live ? (n_items + gridDim.x - 1) / gridDim.x : P.items_per_cta;
+    const int64_t beg = (int64_t)blockIdx.x * items_per_cta;
+    const int64_t end = beg + items_per_cta < n_items ? beg + items_per_cta : n_items;
     const int64_t n_my = end > beg ? end - beg : 0;
     const int n_obs_cols = P.n_chunks * 64;
 
@@ -705,7 +712,7 @@ __global__ void __launch_bounds__(ad::THREADS, 1) agent_dw_tc_kernel(AgentDwPara
             for (int64_t i = 0; i < n_my; ++i) {
                 const int s = (int)(i % STAGES);
                 const int64_t item = beg + i;
-                const int64_t tt = item >> 1;                  // t * n_tiles + tile
+                const int64_t tt = P.live ? (int64_t)__ldg(P.live + (item >> 1)) : item >> 1;   // t * n_tiles + tile
                 const int half = (int)(item & 1);
                 const int64_t t = tt / P.n_tiles, tile = tt - t * P.n_tiles;
                 mbar_wait(&empty[s], (uint32_t)(((i / STAGES) & 1) ^ 1));
@@ -757,7 +764,7 @@ __global__ void __launch_bounds__(ad::THREADS, 1) agent_dw_tc_kernel(AgentDwPara
                 Idx x{-1, -1, 0, 0.f};
                 if (i >= n_my) return x;
                 const int64_t item = beg + i;
-                const int64_t tt = item >> 1;
+                const int64_t tt = P.live ? (int64_t)__ldg(P.live + (item >> 1)) : item >> 1;
                 const int half = (int)(item & 1);
                 const int64_t t = tt / P.n_tiles, tile = tt - t * P.n_tiles;
                 const int64_t p = tile * TILE_ROWS + half * 64 + rr;
@@ -965,7 +972,7 @@ int64_t tc_agent_dw_scratch_bytes() { return align_up((int64_t)sm_count() * 2 * 
 
 int tc_agent_dw(const pmb_dims* d, const pmb_batch* b, const uint8_t* dpre1_ti, const uint8_t* h_ti, const uint8_t* obs_ti,
                 const float* d_chosen, int n_tiles, float* fc1_w, float* fc1_b, float* fc2_w, float* fc2_b, void* scratch,
-                int64_t scratch_bytes, cudaStream_t s) {
+                int64_t scratch_bytes, cudaStream_t s, const int32_t* live_items, const int32_t* n_live) {
     tc::AgentDwParams P;
     P.dpre1_ti = dpre1_ti; P.h_ti = h_ti; P.obs_ti = obs_ti; P.d_chosen = d_chosen;
     P.actions = b->actions; P.actions_sb = b->actions_sb; P.filled = b->filled; P.filled_sb = b->filled_sb;
@@ -973,6 +980,7 @@ int tc_agent_dw(const pmb_dims* d, const pmb_batch* b, const uint8_t* dpre1_ti, 
     P.R = (int64_t)d->B * d->N; P.T = d->T; P.N = d->N; P.A = d->A; P.n_tiles = n_tiles;
     P.n_chunks = (d->O + 63) / 64; P.use_act = d->obs_last_action; P.use_id = d->obs_agent_id;
     P.n_items = (int64_t)d->T * n_tiles * 2;
+    P.live = live_items; P.n_live = n_live;
     int grid = (int)(P.n_items < sm_count() ? P.n_items : sm_count());
     if ((int64_t)grid * tc::ad::PARTIAL_FLOATS * 4 > scratch_bytes) { set_error("tc_agent_dw: scratch too small"); return PMB_ERR_WORKSPACE; }
     P.items_per_cta = ceil_div(P.n_items, grid);

@@ -83,7 +83,17 @@ struct GruFwd2Params {
     uint8_t* g_ti;                   // [nt][n_tiles][4][16 KB] (r, z, n, hn) or null
     int64_t R;
     int nt, n_tiles, tiles_per_cta;
+    // optional (padded-step skipping): a CTA runs tile_steps[its first tile] steps.  Tiles are sorted by their step count,
+    // descending, so a CTA's second tile never needs more; the steps it runs beyond its own count are never read.
+    const int32_t* tile_steps;
 };
+
+// the steps a CTA runs sit in shared memory and are re-read at every step (held in a register, the count spills)
+__device__ __forceinline__ int lds_s32(const int* p) {
+    int v;
+    asm volatile("ld.shared.b32 %0, [%1];" : "=r"(v) : "r"(smem_u32(p)));
+    return v;
+}
 
 __global__ void __launch_bounds__(g2::THREADS, 1) gru_fwd2_kernel(GruFwd2Params P) {
     using namespace g2;
@@ -100,6 +110,7 @@ __global__ void __launch_bounds__(g2::THREADS, 1) gru_fwd2_kernel(GruFwd2Params 
     uint64_t* st_ready = bars + 15;          // gate staging written
     uint64_t* st_free = bars + 16;           // the bulk store of the gate staging has finished reading it
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 17);
+    int* nt_s = reinterpret_cast<int*>(bars + 18);   // steps this CTA runs (0: nothing but the h_0 image)
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     // tiles_per_cta = 2: ping-pong (the tensor core works on one tile while the epilogue warps do the other's gate math);
@@ -113,6 +124,7 @@ __global__ void __launch_bounds__(g2::THREADS, 1) gru_fwd2_kernel(GruFwd2Params 
         for (int i = 0; i < 4; ++i) { mbar_init(&x_full[i], 1); mbar_init(&x_empty[i], 1); }
         for (int i = 0; i < 2; ++i) { mbar_init(&gates_full[i], 1); mbar_init(&h_ready[i], N_EPI_WARPS); mbar_init(&ht_free[i], 1); }
         mbar_init(st_ready, N_EPI_WARPS); mbar_init(st_free, 1);
+        *nt_s = P.tile_steps ? min(P.nt, __ldg(P.tile_steps + tile0)) : P.nt;
         fence_barrier_init();
     }
     if (warp == MMA_WARP) tmem_alloc(tmem_slot, 512);
@@ -143,7 +155,7 @@ __global__ void __launch_bounds__(g2::THREADS, 1) gru_fwd2_kernel(GruFwd2Params 
                 bulk_copy_g2s(smem + XB + (2 * i + b) * TILE_BYTES2,
                               P.x_ti + ((int64_t)t * P.n_tiles + tile0 + i) * TILE_BYTES2, TILE_BYTES2, &x_full[2 * i + b]);
             };
-            for (int t = 0; t < 2 && t < P.nt; ++t)
+            for (int t = 0; t < 2 && t < lds_s32(nt_s); ++t)
                 for (int i = 0; i < n_my; ++i) load_x(i, t);
             // h_0 image (zeros) from the operand tiles
             for (int i = 0; i < n_my; ++i)
@@ -152,13 +164,13 @@ __global__ void __launch_bounds__(g2::THREADS, 1) gru_fwd2_kernel(GruFwd2Params 
             bulk_wait_group_read<0>();
             for (int i = 0; i < n_my; ++i) mbar_arrive(&ht_free[i]);    // arrival #0: the h_0 stores no longer read HT
             uint32_t use = 0;
-            for (int t = 0; t < P.nt; ++t)
+            for (int t = 0; t < lds_s32(nt_s); ++t)
                 for (int i = 0; i < n_my; ++i, ++use) {
                     mbar_wait(&h_ready[i], (uint32_t)(t & 1));
                     const int64_t tt = (int64_t)t * P.n_tiles + tile0 + i;
                     bulk_copy_s2g(P.h_ti + (tt + P.n_tiles) * TILE_BYTES2, smem + HT + i * TILE_BYTES2, TILE_BYTES2);
                     bulk_commit_group();
-                    if (t + 2 < P.nt) load_x(i, t + 2);
+                    if (t + 2 < lds_s32(nt_s)) load_x(i, t + 2);
                     if (stash) {
                         mbar_wait(st_ready, use & 1);
                         bulk_copy_s2g(P.g_ti + tt * 4 * TILE_BYTES2, smem + ST, 4 * TILE_BYTES2);
@@ -180,7 +192,7 @@ __global__ void __launch_bounds__(g2::THREADS, 1) gru_fwd2_kernel(GruFwd2Params 
             const uint32_t wih = smem_u32(smem + WIH), whh = smem_u32(smem + WHH);
             const uint32_t id128 = umma_idesc_bf16(128, 128, 0, 0), id64 = umma_idesc_bf16(128, 64, 0, 0);
             mbar_wait(w_full, 0);
-            for (int t = 0; t < P.nt; ++t)
+            for (int t = 0; t < lds_s32(nt_s); ++t)
                 for (int i = 0; i < n_my; ++i) {
                     const int b = t & 1;
                     const uint32_t xt = smem_u32(smem + XB + (2 * i + b) * TILE_BYTES2);
@@ -225,7 +237,7 @@ __global__ void __launch_bounds__(g2::THREADS, 1) gru_fwd2_kernel(GruFwd2Params 
         for (int i = 0; i < 2; ++i) valid[i] = (int64_t)(tile0 + i) * TILE_ROWS2 + r < P.R;
         const uint32_t bias_s = smem_u32(bias) + 64 * c16;     // this thread's 16 columns of brz | bin | bhn
         uint32_t use = 0;                                      // staging-buffer use counter (all tiles, all steps)
-        for (int t = 0; t < P.nt; ++t) {
+        for (int t = 0; t < lds_s32(nt_s); ++t) {
 #pragma unroll
             for (int i = 0; i < 2; ++i) {
                 if (i < n_my) {
@@ -341,6 +353,11 @@ struct QSelectParams {
     float* q_tg_out;
     int64_t R;
     int T, N, A, n_tiles, double_q;
+    // optional (padded-step skipping): walk items[0 .. *n_live) instead of every t * n_tiles + tile, and write 0 to the
+    // chosen / tmax entries of the (t, tile) items left out (t >= tile_steps[tile])
+    const int32_t* items;
+    const int32_t* n_live;
+    const int32_t* tile_steps;
 };
 
 __global__ void __launch_bounds__(qs::THREADS, 2) q_select_kernel(QSelectParams P) {
@@ -373,7 +390,7 @@ __global__ void __launch_bounds__(qs::THREADS, 2) q_select_kernel(QSelectParams 
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
-    const int64_t n_items = (int64_t)P.T * P.n_tiles;
+    const int64_t n_items = P.items ? (int64_t)__ldg(P.n_live) : (int64_t)P.T * P.n_tiles;
 
     if (warp == 5) {
         if (lane == 0) {
@@ -381,7 +398,8 @@ __global__ void __launch_bounds__(qs::THREADS, 2) q_select_kernel(QSelectParams 
             bulk_copy_g2s(smem + W2ON, P.w2_on_img, 8192, w_full);
             bulk_copy_g2s(smem + W2TG, P.w2_tg_img, 8192, w_full);
             uint32_t it = 0;
-            for (int64_t item = blockIdx.x; item < n_items; item += gridDim.x, ++it) {
+            for (int64_t k = blockIdx.x; k < n_items; k += gridDim.x, ++it) {
+                const int64_t item = P.items ? (int64_t)__ldg(P.items + k) : k;
                 const int s = it % STAGES;
                 mbar_wait(&empty[s], ((it / STAGES) & 1) ^ 1);
                 mbar_arrive_expect_tx(&full[s], STAGE_BYTES);
@@ -424,7 +442,8 @@ __global__ void __launch_bounds__(qs::THREADS, 2) q_select_kernel(QSelectParams 
         const uint32_t bias_s = smem_u32(bias);
         const int n_q4 = (P.A + 3) >> 2;
         uint32_t it = 0;
-        for (int64_t item = blockIdx.x; item < n_items; item += gridDim.x, ++it) {
+        for (int64_t k = blockIdx.x; k < n_items; k += gridDim.x, ++it) {
+            const int64_t item = P.items ? (int64_t)__ldg(P.items + k) : k;
             const int b2 = it & 1;
             const int t = (int)((uint32_t)item / (uint32_t)P.n_tiles);           // T * n_tiles < 2^31
             const int tile = (int)item - t * P.n_tiles;
@@ -505,6 +524,22 @@ __global__ void __launch_bounds__(qs::THREADS, 2) q_select_kernel(QSelectParams 
                 P.tmax[(b * (P.T - 1) + (t - 1)) * P.N + n] = P.double_q ? tsel : best;
             }
         }
+        if (P.tile_steps) {
+            // the items the schedule left out: chosen of step t and tmax of step t - 1 are 0 there.  The mixers and the loss
+            // read every (b, t) and the loss multiplies by a zero mask, so these entries must be finite; 0 is the cheapest.
+            for (int tile = blockIdx.x; tile < P.n_tiles; tile += gridDim.x) {
+                const int64_t p = (int64_t)tile * TILE_ROWS2 + r;
+                if (p >= P.R) continue;
+                const int64_t b = (int64_t)((uint32_t)p / (uint32_t)P.N);
+                const int n = (int)(p - b * P.N);
+                float* ch = P.chosen + b * (P.T - 1) * P.N + n;
+                float* tm = P.tmax + b * (P.T - 1) * P.N + n;
+                for (int t = __ldg(P.tile_steps + tile); t < P.T; ++t) {
+                    if (t < P.T - 1) ch[(int64_t)t * P.N] = 0.f;
+                    if (t >= 1) tm[(int64_t)(t - 1) * P.N] = 0.f;
+                }
+            }
+        }
     }
     tc_fence_before();
     __syncthreads();
@@ -564,6 +599,9 @@ struct GruBwd2Params {
     float* partial;                  // [n_tiles][b2::PARTIAL_FLOATS]
     int64_t R;
     int T, N, A, n_tiles;
+    // optional (padded-step skipping): tile `tile` runs steps t = tile_steps[tile] - 1 .. 0 only.  dh = 0 at the start is
+    // exact: d_chosen is 0 for every row of the tile at every later step.  A tile with no steps writes zero partials.
+    const int32_t* tile_steps;
 };
 
 // BPTT through the GRU over one 128-row tile, fused with ALL recurrent weight gradients: per step the gate gradients
@@ -588,6 +626,7 @@ __global__ void __launch_bounds__(b2::THREADS, 1) gru_bwd2_kernel(GruBwd2Params 
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int tile = blockIdx.x;
+    const int steps = P.tile_steps ? __ldg(P.tile_steps + tile) : P.T;
     if (threadIdx.x == 0) {
         mbar_init(w_full, 1);
         mbar_init(&in_full[0], 1); mbar_init(&in_full[1], 1); mbar_init(x_full, 1);
@@ -609,13 +648,16 @@ __global__ void __launch_bounds__(b2::THREADS, 1) gru_bwd2_kernel(GruBwd2Params 
     const uint32_t r = (uint32_t)(q4 * 32 + lane);
     const uint32_t tlane = tmem_base + ((uint32_t)(q4 * 32) << 16) + 32 * ch;
 
-    if (warp == IO_WARP) {
+    if (steps == 0) {
+        // no live step: zero partials for gru_bwd2_reduce_kernel
+        for (int i = threadIdx.x; i < PARTIAL_FLOATS; i += THREADS) P.partial[(int64_t)tile * PARTIAL_FLOATS + i] = 0.f;
+    } else if (warp == IO_WARP) {
         if (lane == 0) {
             mbar_arrive_expect_tx(w_full, 2 * 24576);
             bulk_copy_g2s(smem + WIH, P.w_ih_img, 24576, w_full);
             bulk_copy_g2s(smem + WHH, P.w_hh_img, 24576, w_full);
             auto load = [&](int i) {                            // step index i <-> t = T-1-i, buffer i & 1
-                const int t = P.T - 1 - i;
+                const int t = steps - 1 - i;
                 const int64_t tt = (int64_t)t * P.n_tiles + tile;
                 uint8_t* buf = smem + BUF + (i & 1) * BUF_BYTES;
                 mbar_arrive_expect_tx(&in_full[i & 1], BUF_BYTES);
@@ -623,15 +665,15 @@ __global__ void __launch_bounds__(b2::THREADS, 1) gru_bwd2_kernel(GruBwd2Params 
                 bulk_copy_g2s(buf + 4 * TILE_BYTES2, P.h_ti + tt * TILE_BYTES2, TILE_BYTES2, &in_full[i & 1]);
             };
             auto load_x = [&](int i) {
-                const int64_t tt = (int64_t)(P.T - 1 - i) * P.n_tiles + tile;
+                const int64_t tt = (int64_t)(steps - 1 - i) * P.n_tiles + tile;
                 mbar_arrive_expect_tx(x_full, TILE_BYTES2);
                 bulk_copy_g2s(smem + XS, P.x_ti + tt * TILE_BYTES2, TILE_BYTES2, x_full);
-                if (i + 1 < P.T)                                // the next one comes out of L2
+                if (i + 1 < steps)                                // the next one comes out of L2
                     asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(P.x_ti + (tt - P.n_tiles) * TILE_BYTES2),
                                  "r"((uint32_t)TILE_BYTES2) : "memory");
             };
             auto prefetch = [&](int i) {                        // stage i into L2: its buffer frees late, the copy must be short
-                const int64_t tt = (int64_t)(P.T - 1 - i) * P.n_tiles + tile;
+                const int64_t tt = (int64_t)(steps - 1 - i) * P.n_tiles + tile;
                 asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(P.g_ti + tt * 4 * TILE_BYTES2),
                              "r"((uint32_t)(4 * TILE_BYTES2)) : "memory");
                 asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(P.h_ti + tt * TILE_BYTES2),
@@ -639,19 +681,19 @@ __global__ void __launch_bounds__(b2::THREADS, 1) gru_bwd2_kernel(GruBwd2Params 
             };
             load(0);
             load_x(0);
-            if (P.T > 1) load(1);
-            if (P.T > 2) prefetch(2);
-            for (int i = 0; i < P.T; ++i) {
-                if (i + 3 < P.T) prefetch(i + 3);
-                const int64_t tt = (int64_t)(P.T - 1 - i) * P.n_tiles + tile;
+            if (steps > 1) load(1);
+            if (steps > 2) prefetch(2);
+            for (int i = 0; i < steps; ++i) {
+                if (i + 3 < steps) prefetch(i + 3);
+                const int64_t tt = (int64_t)(steps - 1 - i) * P.n_tiles + tile;
                 uint8_t* buf = smem + BUF + (i & 1) * BUF_BYTES;
                 mbar_wait(dw_done, (uint32_t)(i & 1));          // the x slot is free: refill it first
-                if (i + 1 < P.T) load_x(i + 1);
+                if (i + 1 < steps) load_x(i + 1);
                 mbar_wait(dp_ready, (uint32_t)(i & 1));
                 bulk_copy_s2g(P.dpre1_ti + tt * TILE_BYTES2, buf + 4 * TILE_BYTES2, TILE_BYTES2);
                 bulk_commit_group();
                 bulk_wait_group_read<0>();                     // buffer i & 1 is free again
-                if (i + 2 < P.T) load(i + 2);
+                if (i + 2 < steps) load(i + 2);
             }
             bulk_wait_group<0>();
         }
@@ -665,7 +707,7 @@ __global__ void __launch_bounds__(b2::THREADS, 1) gru_bwd2_kernel(GruBwd2Params 
             const uint32_t idesc_b = umma_idesc_bf16(128, 16, 1, 1);
             const uint64_t b_one = umma_desc_sw128(ones, TILE_BYTES2, 1024);
             mbar_wait(w_full, 0);
-            for (int i = 0; i < P.T; ++i) {
+            for (int i = 0; i < steps; ++i) {
                 const uint32_t dg = smem_u32(smem + BUF + (i & 1) * BUF_BYTES);
                 const uint32_t xh_lbo = dg + 4 * TILE_BYTES2 - xs;          // [x | h_prev]: two 64-column blocks this far apart
                 mbar_wait(dg_ready, (uint32_t)(i & 1));
@@ -728,14 +770,14 @@ __global__ void __launch_bounds__(b2::THREADS, 1) gru_bwd2_kernel(GruBwd2Params 
             for (int c = 0; c < 4; ++c)
                 w[c] = __ldg(reinterpret_cast<const uint4*>(wr + (((uint32_t)(4 * ch + c) ^ ((uint32_t)a & 7u)) << 4)));
         };
-        float dq = fetch_dq(P.T - 1);
-        uint32_t xm = fetch_m(P.T - 1);
+        float dq = fetch_dq(steps - 1);
+        uint32_t xm = fetch_m(steps - 1);
         uint4 w2[4];
         uint32_t dpk[16];                                       // dpre1 of the previous step (bf16 pairs), staged late
-        fetch_w2(fetch_a(P.T - 1), w2);
-        int act_n = fetch_a(P.T - 2);
-        for (int i = 0; i < P.T; ++i) {
-            const int t = P.T - 1 - i;
+        fetch_w2(fetch_a(steps - 1), w2);
+        int act_n = fetch_a(steps - 2);
+        for (int i = 0; i < steps; ++i) {
+            const int t = steps - 1 - i;
             uint8_t* buf = smem + BUF + (i & 1) * BUF_BYTES;
             const float dq_n = fetch_dq(t - 1);
             const uint32_t xm_n = fetch_m(t - 1);
@@ -831,7 +873,7 @@ __global__ void __launch_bounds__(b2::THREADS, 1) gru_bwd2_kernel(GruBwd2Params 
                     dh[j + 1] = fmaf(dh[j + 1], zk[j + 1], __uint_as_float(ah[j + 1]));
                 }
             }
-            if (i == P.T - 1) stage_dp(i);
+            if (i == steps - 1) stage_dp(i);
             dq = dq_n; xm = xm_n;
         }
     }
@@ -839,7 +881,7 @@ __global__ void __launch_bounds__(b2::THREADS, 1) gru_bwd2_kernel(GruBwd2Params 
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
-    if (warp < N_EPI_WARPS) {
+    if (warp < N_EPI_WARPS && steps > 0) {
         // accumulator row = gate column (r < 64: first gate of the pair, else the second), accumulator columns 0..63 =
         // x columns (weight_ih), 64..127 = h_{t-1} columns (weight_hh): warp half ch takes the x resp. the h block
         float* part = P.partial + (int64_t)tile * PARTIAL_FLOATS;
@@ -925,11 +967,12 @@ __global__ void __launch_bounds__(256) gru_bwd2_reduce_kernel(const float* __res
 
 int tc_gru_fwd2(const __nv_bfloat16* w_ih_img, const __nv_bfloat16* w_hh_img, const float* b_ih, const float* b_hh,
                 const uint8_t* x_ti, uint8_t* h_ti, uint8_t* g_ti, int64_t R, int nt, int n_tiles, cudaStream_t s,
-                int tiles_per_cta) {
+                int tiles_per_cta, const int32_t* tile_steps) {
     tc::GruFwd2Params P;
     P.w_ih_img = w_ih_img; P.w_hh_img = w_hh_img; P.b_ih = b_ih; P.b_hh = b_hh;
     P.x_ti = x_ti; P.h_ti = h_ti; P.g_ti = g_ti; P.R = R; P.nt = nt; P.n_tiles = n_tiles;
     P.tiles_per_cta = tiles_per_cta == 1 ? 1 : 2;
+    P.tile_steps = tile_steps;
     PMB_SMEM_ATTR(tc::gru_fwd2_kernel, tc::g2::SMEM_BYTES);
     tc::gru_fwd2_kernel<<<(n_tiles + P.tiles_per_cta - 1) / P.tiles_per_cta, tc::g2::THREADS, tc::g2::SMEM_BYTES, s>>>(P);
     PMB_LAUNCH_CHECK("gru_fwd2_kernel");
@@ -938,7 +981,8 @@ int tc_gru_fwd2(const __nv_bfloat16* w_ih_img, const __nv_bfloat16* w_hh_img, co
 
 int tc_q_select(const pmb_dims* d, const pmb_batch* b, const __nv_bfloat16* w2_on_img, const __nv_bfloat16* w2_tg_img,
                 const float* b2_on, const float* b2_tg, const uint8_t* h_on_ti, const uint8_t* h_tg_ti, int n_tiles,
-                float* chosen, float* tmax, float* q_on_out, float* q_tg_out, cudaStream_t s) {
+                float* chosen, float* tmax, float* q_on_out, float* q_tg_out, cudaStream_t s, const int32_t* live_items,
+                const int32_t* n_live, const int32_t* tile_steps) {
     tc::QSelectParams P;
     P.w2_on_img = w2_on_img; P.w2_tg_img = w2_tg_img; P.b2_on = b2_on; P.b2_tg = b2_tg;
     P.h_on_ti = h_on_ti; P.h_tg_ti = h_tg_ti;
@@ -946,6 +990,7 @@ int tc_q_select(const pmb_dims* d, const pmb_batch* b, const __nv_bfloat16* w2_o
     P.ep_index = b->ep_index;
     P.chosen = chosen; P.tmax = tmax; P.q_on_out = q_on_out; P.q_tg_out = q_tg_out;
     P.R = (int64_t)d->B * d->N; P.T = d->T; P.N = d->N; P.A = d->A; P.n_tiles = n_tiles; P.double_q = d->double_q;
+    P.items = live_items; P.n_live = n_live; P.tile_steps = tile_steps;
     const int64_t n_items = (int64_t)d->T * n_tiles;
     int grid = 2 * sm_count();
     if (grid > n_items) grid = (int)n_items;
@@ -962,13 +1007,13 @@ int64_t tc_gru_bwd2_partial_bytes(int n_tiles) {
 int tc_gru_bwd2(const __nv_bfloat16* w_ih_img, const __nv_bfloat16* w_hh_img, const __nv_bfloat16* w2_img,
                 const uint8_t* x_ti, const uint8_t* h_ti, const uint8_t* g_ti, uint8_t* dpre1_ti, const uint32_t* relu_mask,
                 const float* d_chosen, const int64_t* actions, int64_t actions_sb, const int64_t* ep_index, int64_t R, int T,
-                int N, int A, int n_tiles, float* partial, cudaStream_t s) {
+                int N, int A, int n_tiles, float* partial, cudaStream_t s, const int32_t* tile_steps) {
     tc::GruBwd2Params P;
     P.w_ih_img = w_ih_img; P.w_hh_img = w_hh_img; P.w2_img = reinterpret_cast<const uint8_t*>(w2_img);
     P.x_ti = x_ti; P.h_ti = h_ti; P.g_ti = g_ti; P.dpre1_ti = dpre1_ti;
     P.relu_mask = relu_mask; P.d_chosen = d_chosen; P.actions = actions; P.actions_sb = actions_sb;
     P.partial = partial; P.ep_index = ep_index;
-    P.R = R; P.T = T; P.N = N; P.A = A; P.n_tiles = n_tiles;
+    P.R = R; P.T = T; P.N = N; P.A = A; P.n_tiles = n_tiles; P.tile_steps = tile_steps;
     PMB_SMEM_ATTR(tc::gru_bwd2_kernel, tc::b2::SMEM_BYTES);
     tc::gru_bwd2_kernel<<<n_tiles, tc::b2::THREADS, tc::b2::SMEM_BYTES, s>>>(P);
     PMB_LAUNCH_CHECK("gru_bwd2_kernel");

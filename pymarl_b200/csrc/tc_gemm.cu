@@ -552,7 +552,15 @@ struct Fc1StreamParams {
     int n_nets;                    // 2: online + target (learner step), 1: online only (rollout step)
     int t0;                        // batch timestep of item t = 0 (rollout: the step index; obs is addressed at t0 + t)
     int n_act;                     // A: rows of tab_act16
+    // optional live-item schedule (learner step, pmb_dims.reserved bit 1): the grid walks items[k] instead of every item
+    // k = t * n_tiles + tile, up to the first negative entry (the list is padded with -1 to T * n_tiles entries: a count
+    // loaded in every role is hoisted above the role branch and spills in fc1_stream_ts_kernel).  Items not listed are
+    // neither read nor written.
+    const int32_t* items;
 };
+
+// the k-th item of the grid's walk, < 0 past the end of a live-item list (T * n_tiles < 2^31, validated on the host)
+__device__ __forceinline__ int fc1_item(const Fc1StreamParams& P, int k) { return P.items ? __ldg(P.items + k) : k; }
 
 __device__ __forceinline__ float lds_f32(uint32_t addr) {
     float v;
@@ -614,7 +622,7 @@ __device__ __forceinline__ void fc1_produce(const Fc1StreamParams& P, const Fc1R
     int* rown = ring.rown;
     uint64_t* st_full = ring.st_full;
     uint64_t* st_empty = ring.st_empty;
-    const int64_t n_items = (int64_t)P.T * P.n_tiles;
+    const int n_items = P.T * P.n_tiles;
 
     // Lane i owns the i-th contiguous run of a group (one episode each) and computes its descriptor - global
     // address, staging offset, head / interior / tail split - in closed form, in parallel with the other lanes
@@ -622,7 +630,9 @@ __device__ __forceinline__ void fc1_produce(const Fc1StreamParams& P, const Fc1R
     // runs serially after the wait: ~1.5 us of dependent integer code per group during which the slot sat empty,
     // which bounded the stream at three slots per (walk + load + convert).)
     uint32_t git = 0;
-    for (int64_t item = blockIdx.x; item < n_items; item += gridDim.x) {
+    for (int k = blockIdx.x; k < n_items; k += gridDim.x) {
+        const int64_t item = fc1_item(P, k);
+        if (item < 0) break;
         const int64_t t = item / P.n_tiles, tile = item - t * P.n_tiles;
         for (int g = 0; g < GROUPS; ++g, ++git) {
             const int slot = git % N_SLOTS;
@@ -662,8 +672,8 @@ __device__ __forceinline__ void fc1_produce(const Fc1StreamParams& P, const Fc1R
             const uint32_t tx = __reduce_add_sync(0xffffffffu, cp_bytes);
             // L2 prefetch of the same group of this CTA's NEXT tile: the staging ring is all the shared memory that is
             // left (3 x 18 KB in flight per SM), so the copies should see L2 latency, not loaded-HBM latency
-            if (P.l2_prefetch && cnt > 0 && item + (int64_t)P.l2_prefetch * gridDim.x < n_items) {
-                const int64_t item2 = item + (int64_t)P.l2_prefetch * gridDim.x;
+            if (P.l2_prefetch && cnt > 0 && k + P.l2_prefetch * (int)gridDim.x < n_items) {
+                const int64_t item2 = max(fc1_item(P, k + P.l2_prefetch * (int)gridDim.x), 0);
                 const int64_t t2 = item2 / P.n_tiles, tile2 = item2 - t2 * P.n_tiles;
                 const int64_t q0 = tile2 * BM + g * GROUP_ROWS;
                 int rows2 = P.R - q0 < GROUP_ROWS ? (int)(P.R - q0) : GROUP_ROWS;
@@ -716,7 +726,7 @@ __device__ __forceinline__ void fc1_convert(const Fc1StreamParams& P, const Fc1R
     int* rown = ring.rown;
     uint64_t* st_full = ring.st_full;
     uint64_t* st_empty = ring.st_empty;
-    const int64_t n_items = (int64_t)P.T * P.n_tiles;
+    const int n_items = P.T * P.n_tiles;
     constexpr int c_last = NC - 1;
     // every column of the chunks before the last exists (O > 64 (NC-1)); the last chunk: per lane
     const bool okl0 = c_last * BK + 2 * lane < P.O, okl1 = c_last * BK + 2 * lane + 1 < P.O;
@@ -724,7 +734,9 @@ __device__ __forceinline__ void fc1_convert(const Fc1StreamParams& P, const Fc1R
     const uint32_t a_s_u32 = smem_u32(a_s);
     const uint32_t a_base = a_s_u32 + ((uint32_t)(lane >> 2) << 4) + (lane & 3) * 4;   // + row*128, ^ swizzle
     uint32_t git = 0, ti = 0;
-    for (int64_t item = blockIdx.x; item < n_items; item += gridDim.x, ++ti) {
+    for (int k = blockIdx.x; k < n_items; k += gridDim.x, ++ti) {
+        const int item = fc1_item(P, k);
+        if (item < 0) break;
         for (int g = 0; g < GROUPS; ++g, ++git) {
             const int slot = git % N_SLOTS;
             TWAIT(1, &st_full[slot], (git / N_SLOTS) & 1);
@@ -784,7 +796,7 @@ __device__ __forceinline__ void fc1_convert(const Fc1StreamParams& P, const Fc1R
                     // (a bulk store of the finished A tile kept the tile busy for ~2500 cycles after the MMAs were
                     // done with it: the converters of the next tile waited 22 % of the kernel time for it)
                     if (P.obs_img) {
-                        uint8_t* img = P.obs_img + item * tile_bytes + (dst - a_s_u32);
+                        uint8_t* img = P.obs_img + (int64_t)item * tile_bytes + (dst - a_s_u32);
 #pragma unroll
                         for (int c = 0; c < NC; ++c) __stcs(reinterpret_cast<uint32_t*>(img + c * A_STAGE_BYTES), pk[rr][c]);
                     }
@@ -836,7 +848,7 @@ __global__ void __launch_bounds__(fs::threads_for(NS), 1) fc1_stream_kernel(Fc1S
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
-    const int64_t n_items = (int64_t)P.T * P.n_tiles;
+    const int n_items = P.T * P.n_tiles;
     const Fc1Ring ring{stage, rowoff, rown, st_full, st_empty};
     // programmatic dependent launch (rollout step only; see gru_rollout_kernel): the next kernel may be scheduled as the
     // CTAs of this grid leave; this kernel reads nothing its predecessor writes and only its epilogue warps write something
@@ -864,7 +876,8 @@ __global__ void __launch_bounds__(fs::threads_for(NS), 1) fc1_stream_kernel(Fc1S
             const uint32_t idesc = umma_idesc_bf16(BM, 64 * P.n_nets, 0, 0);
             mbar_wait(w_full, 0);
             uint32_t ti = 0;
-            for (int64_t item = blockIdx.x; item < n_items; item += gridDim.x, ++ti) {
+            for (int k = blockIdx.x; k < n_items; k += gridDim.x, ++ti) {
+                if (fc1_item(P, k) < 0) break;
                 const int b = ti & 1;
                 TWAIT(3, a_full, ti & 1);
                 TWAIT(4, &tempty[b], ((ti >> 1) & 1) ^ 1);
@@ -888,10 +901,12 @@ __global__ void __launch_bounds__(fs::threads_for(NS), 1) fc1_stream_kernel(Fc1S
         // ===== epilogue: one row per thread; x = relu(acc [+ id/bias table] + act table) -> bf16 tile images + mask.
         // (Eight epilogue warps, one per row and net, measured slower: 7.21 -> 7.53 ms.) =====
         const uint32_t r = (uint32_t)(warp * 32 + lane);
-        // the previous action of a row, fetched one item ahead (-1: none / step not filled, -2: padding row)
-        auto fetch_prev = [&](int64_t item, int& n_out) {
+        // the previous action of a row of the k-th item, fetched one item ahead (-1: none / step not filled, -2: padding row)
+        auto fetch_prev = [&](int k, int& n_out) {
             n_out = 0;
-            if (item >= n_items) return -2;
+            if (k >= n_items) return -2;
+            const int64_t item = fc1_item(P, k);
+            if (item < 0) return -2;
             const int64_t t = item / P.n_tiles, tile = item - t * P.n_tiles;
             const int64_t p = tile * BM + r;
             if (p >= P.R) return -2;
@@ -908,9 +923,11 @@ __global__ void __launch_bounds__(fs::threads_for(NS), 1) fc1_stream_kernel(Fc1S
         int a_prev = fetch_prev(blockIdx.x, n_cur);
         uint32_t ti = 0;
         pdl_wait();                                            // before the first store to the x images
-        for (int64_t item = blockIdx.x; item < n_items; item += gridDim.x, ++ti) {
+        for (int k = blockIdx.x; k < n_items; k += gridDim.x, ++ti) {
+            const int64_t item = fc1_item(P, k);
+            if (item < 0) break;
             const int b = ti & 1;
-            const int a_next = fetch_prev(item + gridDim.x, n_nxt);
+            const int a_next = fetch_prev(k + gridDim.x, n_nxt);
             TWAIT(5, &tfull[b], (ti >> 1) & 1);
             tc_fence_after();
             const uint32_t taddr = tmem_base + 128u * b + ((uint32_t)(warp * 32) << 16);
@@ -1034,12 +1051,13 @@ __global__ void __launch_bounds__(fs::threads_for(fs::N_SLOTS_TS), 1) fc1_stream
     } else if (warp == MMA_W) {
         if (lane == 0) {
             const uint32_t tmem_base = *tmem_slot;
-            const int64_t n_items = (int64_t)P.T * P.n_tiles;
+            const int n_items = P.T * P.n_tiles;
             const uint32_t idesc = umma_idesc_bf16(BM, BM, 0, 0);
             mbar_wait(w_full, 0);
             tc_fence_after();
             uint32_t ti = 0;
-            for (int64_t item = blockIdx.x; item < n_items; item += gridDim.x, ++ti) {
+            for (int k = blockIdx.x; k < n_items; k += gridDim.x, ++ti) {
+                if (fc1_item(P, k) < 0) break;
                 const int b = ti & 1;
                 TWAIT(3, a_full, ti & 1);
                 TWAIT(4, &tempty[b], ((ti >> 1) & 1) ^ 1);
@@ -1062,7 +1080,7 @@ __global__ void __launch_bounds__(fs::threads_for(fs::N_SLOTS_TS), 1) fc1_stream
         const int hl = warp * 32 + lane;                      // accumulator lane: online hidden 0-63 | target 64-127
         const int net = warp >> 1;
         const uint32_t tmem_base = *tmem_slot;
-        const int64_t n_items = (int64_t)P.T * P.n_tiles;
+        const int n_items = P.T * P.n_tiles;
         TMARK(pe0);
         // W rows of this thread's hidden unit into TMEM: the packed image's 128-byte row, un-swizzled, is 32 columns
         {
@@ -1087,9 +1105,11 @@ __global__ void __launch_bounds__(fs::threads_for(fs::N_SLOTS_TS), 1) fc1_stream
             for (int i = hl; i < P.n_act * 128; i += 128) tab_s[i] = __uint_as_float((uint32_t)__ldg(ta + i) << 16);
         }
         TADD(14, clock64() - pe0);                             // epilogue: W into TMEM, table into shared memory
-        // the previous action of row hl of an item (-1: none / step not filled, -2: padding row)
-        auto fetch_prev = [&](int64_t item) {
-            if (item >= n_items) return -2;
+        // the previous action of row hl of the k-th item (-1: none / step not filled, -2: padding row)
+        auto fetch_prev = [&](int k) {
+            if (k >= n_items) return -2;
+            const int64_t item = fc1_item(P, k);
+            if (item < 0) return -2;
             const int64_t t = item / P.n_tiles, tile = item - t * P.n_tiles;
             const int64_t p = tile * BM + hl;
             if (p >= P.R) return -2;
@@ -1108,9 +1128,11 @@ __global__ void __launch_bounds__(fs::threads_for(fs::N_SLOTS_TS), 1) fc1_stream
         const uint32_t xs_lane = xs_u32 + (h2 & 7) * 2;
         const uint32_t tab_u32 = smem_u32(tab_s + hl);
         uint32_t ti = 0;
-        for (int64_t item = blockIdx.x; item < n_items; item += gridDim.x, ++ti) {
+        for (int k = blockIdx.x; k < n_items; k += gridDim.x, ++ti) {
+            const int item = fc1_item(P, k);
+            if (item < 0) break;
             const int b = ti & 1;
-            const int a_next = fetch_prev(item + gridDim.x);
+            const int a_next = fetch_prev(k + gridDim.x);
             const uint32_t pv_u32 = smem_u32(prev_s + b * BM);
             prev_s[b * BM + hl] = a_prev;
             TMARK(pe1);
@@ -1120,7 +1142,7 @@ __global__ void __launch_bounds__(fs::threads_for(fs::N_SLOTS_TS), 1) fc1_stream
             TWAIT(5, &tfull[b], (ti >> 1) & 1);
             tc_fence_after();
             TMARK(pe2);
-            const int64_t tile = item % P.n_tiles;
+            const int tile = item % P.n_tiles;
             const int rows_valid = P.R - tile * BM < BM ? (int)(P.R - tile * BM) : BM;
             const uint32_t taddr = tmem_base + 128u * b + ((uint32_t)(warp * 32) << 16);
 #pragma unroll 1
@@ -1158,7 +1180,7 @@ __global__ void __launch_bounds__(fs::threads_for(fs::N_SLOTS_TS), 1) fc1_stream
                     mword = lane == e ? bal : mword;
                 }
                 if (net == 0 && P.relu_mask && 32 * g + lane < rows_valid)
-                    P.relu_mask[(item * 2 + warp) * 128 + 32 * g + lane] = mword;
+                    P.relu_mask[((int64_t)item * 2 + warp) * 128 + 32 * g + lane] = mword;
                 // bf16 pairs of adjacent hidden units: the even lane stores row e, the odd lane row e + 4 (the two rows
                 // fall on disjoint 16-byte chunks of the swizzle, so the 32 stores of a step hit 32 banks)
 #pragma unroll
@@ -1175,8 +1197,8 @@ __global__ void __launch_bounds__(fs::threads_for(fs::N_SLOTS_TS), 1) fc1_stream
             fence_proxy_async_smem();
             epi_bar_sync();
             if (threadIdx.x == 0) {
-                bulk_copy_s2g(P.x_on + item * A_STAGE_BYTES, xs, (uint32_t)rows_valid * 128u);
-                bulk_copy_s2g(P.x_tg + item * A_STAGE_BYTES, xs + A_STAGE_BYTES, (uint32_t)rows_valid * 128u);
+                bulk_copy_s2g(P.x_on + (int64_t)item * A_STAGE_BYTES, xs, (uint32_t)rows_valid * 128u);
+                bulk_copy_s2g(P.x_tg + (int64_t)item * A_STAGE_BYTES, xs + A_STAGE_BYTES, (uint32_t)rows_valid * 128u);
                 bulk_commit_group();
             }
             TADD(13, clock64() - pe2);                         // epilogue: TMEM loads, tables, ReLU, mask, x stage
@@ -1305,8 +1327,10 @@ extern "C" int pmb_debug_fc1_prof(unsigned long long* out, int reset) {
 #endif
 int tc_fc1_fwd_both(const pmb_dims* d, const pmb_batch* b, int t0, int nt, const AgentParams& on, const AgentParams& tg,
                     float* x_on, float* x_tg, int tile_images, uint8_t* obs_img_out, uint32_t* relu_mask, void* scratch,
-                    int64_t scratch_bytes, cudaStream_t s, int weights_packed) {
+                    int64_t scratch_bytes, cudaStream_t s, int weights_packed, const int32_t* live_items) {
     // scratch: packed W (128 x Kpad bf16) | tab_act | tab_id
+    // live_items (may be NULL): the live (t, tile) items of a padded-step skipping learner step, -1 after the last one
+    // (streaming kernels only)
     // weights_packed: the caller guarantees that `scratch` still holds the images / tables a previous call packed from
     // the SAME parameters (rollout steps between two learner updates): the pack launches are skipped
     const int D_in = d_in_of(d);
@@ -1377,6 +1401,7 @@ int tc_fc1_fwd_both(const pmb_dims* d, const pmb_batch* b, int t0, int nt, const
             Q.x_on = reinterpret_cast<uint8_t*>(x_on); Q.x_tg = reinterpret_cast<uint8_t*>(x_tg);
             Q.relu_mask = relu_mask; Q.use_act = d->obs_last_action;
             Q.n_nets = x_tg ? 2 : 1; Q.t0 = t0; Q.n_act = d->A;
+            Q.items = live_items;
             // L2 prefetch of the CTA's next tile(s): measured (round 2, same box, alternating) as a LOSS - rollout step 0.196 ms
             // with one tile ahead, 0.217 ms with two, 0.190 ms without; learner fc1 8.1-8.4 / 8.8 / 8.0 ms - the copies of the
             // ring already keep the memory system busy and the prefetch instructions cost the producers issue time.
@@ -1422,10 +1447,10 @@ int tc_fc1_fwd_both(const pmb_dims* d, const pmb_batch* b, int t0, int nt, const
             PMB_LAUNCH_CHECK("fc1_stream_kernel");
             return PMB_OK;
         }
-        if (b->ep_index) { set_error("tc_fc1: ep_index needs the streaming kernel (obs dim <= 320)"); return PMB_ERR_INVALID; }
+        if (b->ep_index || live_items) { set_error("tc_fc1: ep_index and live items need the streaming kernel (obs dim <= 320)"); return PMB_ERR_INVALID; }
         return tc::launch_tc_gemm(P, epi, s);
     }
-    if (b->ep_index) { set_error("tc_fc1: ep_index is not supported without tile images"); return PMB_ERR_INVALID; }
+    if (b->ep_index || live_items) { set_error("tc_fc1: ep_index and live items are not supported without tile images"); return PMB_ERR_INVALID; }
     tc::Fc1Epi epi{tab_act, tab_id, b->actions, b->actions_sb, b->filled, b->filled_sb, x_on, x_tg,
                    t0, nt, d->N, d->A, d->obs_last_action, (int64_t)d->B * d->N};
     return tc::launch_tc_gemm(P, epi, s);

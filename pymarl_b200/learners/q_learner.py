@@ -10,6 +10,8 @@ Data parallel: with torch.distributed initialised (one process per GPU, NCCL) ev
 trains on its shard of the episodes (train() slices the sampled batch itself); the un-normalised
 gradients and the five loss sums travel in ONE all-reduce per step and every rank applies the
 identical update.  args.cuda_graph = True replays the whole step as one CUDA graph.
+args.skip_padded_steps = True lets the step skip the padded timesteps of a ragged batch (pmb_dims.reserved
+bit 1; honoured on the fused tensor-core path, ignored elsewhere).
 """
 import copy
 import ctypes as C
@@ -96,7 +98,8 @@ class QLearner:
         return _lib.make_dims(B=B, T=T, N=a.n_agents, O=O, S=S, A=a.n_actions, H=a.rnn_hidden_dim,
                               E=getattr(a, "mixing_embed_dim", 1) if a.mixer == "qmix" else 1,
                               obs_last_action=a.obs_last_action, obs_agent_id=a.obs_agent_id, mixer=a.mixer,
-                              double_q=a.double_q, precision=self.precision)
+                              double_q=a.double_q, precision=self.precision,
+                              skip_padding=getattr(a, "skip_padded_steps", False))
 
     def _ensure_flat(self):
         """(Re)build the four flat buffers when the parameters are not views of them (first
@@ -180,6 +183,10 @@ class QLearner:
             for s in shp:
                 n *= s
             out[k] = f32[off:off + n].view(shp)
+        if v.ep_order:                  # padded-step skipping ran (args.skip_padded_steps where it is honoured)
+            n_tiles = (R + 127) // 128
+            out["ep_order"] = self._workspace[v.ep_order - base:v.ep_order - base + 8 * B].view(th.int64)
+            out["tile_steps"] = self._workspace[v.tile_steps - base:v.tile_steps - base + 4 * n_tiles].view(th.int32)
         return out
 
     # ---- the step ---------------------------------------------------------------------------
