@@ -76,9 +76,15 @@ typedef struct pmb_dims {
                                 * area only where the bit is honoured.  0 is always safe.                             */
 } pmb_dims;
 
-/* The EpisodeBatch fields the path reads.  *_sb = batch stride in ELEMENTS. */
+/* Element type of pmb_batch.obs.  BF16 (a scheme with "obs": {..., "dtype": th.bfloat16}, stored with torch's
+ * round-to-nearest-even) is read natively only where pmb_obs_bf16_supported() says so; every other entry point that reads
+ * obs returns PMB_ERR_INVALID for it.  The bf16 tier rounds obs to bf16 before its first use, so there a bf16-stored batch
+ * gives results bit-identical to an fp32-stored one holding the same (bf16-representable) values. */
+enum pmb_dtype { PMB_DTYPE_F32 = 0, PMB_DTYPE_BF16 = 1 };
+
+/* The EpisodeBatch fields the path reads.  *_sb = batch stride in ELEMENTS (of the field's own type). */
 typedef struct pmb_batch {
-    const float*   obs;        int64_t obs_sb;          /* [B,T,N,O] f32 */
+    const void*    obs;        int64_t obs_sb;          /* [B,T,N,O] f32, or bf16 (obs_dtype) */
     const float*   state;      int64_t state_sb;        /* [B,T,S]   f32 (QMIX only, else NULL) */
     const int64_t* actions;    int64_t actions_sb;      /* [B,T,N,1] i64 */
     const int32_t* avail;      int64_t avail_sb;        /* [B,T,N,A] i32 */
@@ -90,7 +96,18 @@ typedef struct pmb_batch {
      * (components/episode_buffer.py:205-217,291-298) without the gather copy.  Device array of B ids.  Supported by
      * the tensor-core tier of pmb_qlearner_train_step only. */
     const int64_t* ep_index;
+    int32_t obs_dtype;         /* enum pmb_dtype; 0 (fp32) is always accepted, any value but 0 and 1 is PMB_ERR_INVALID */
 } pmb_batch;
+
+/* 1 where the kernels of `entry` read PMB_DTYPE_BF16 obs natively for these dims, else 0 (host only, no device call):
+ *   PMB_ENTRY_TRAIN_STEP      pmb_qlearner_train_step on the fused tensor-core path (bf16 tier, H = 64, A <= 64, QMIX with
+ *                             E = 32 or VDN / IQL, O <= 320, agent id folding into the K padding of obs) where the
+ *                             streaming fc1 kernel runs (its staging ring fits shared memory)
+ *   PMB_ENTRY_SELECT_ACTIONS  pmb_select_actions_step on the tensor-core tier where the streaming fc1 kernel runs
+ * The fp32 tier, the generic tcgen05 fc1 GEMM, pmb_agent_fc1_fwd, pmb_agent_unroll_bwd and the COMA entry points read fp32
+ * obs only: convert first. */
+enum pmb_entry { PMB_ENTRY_TRAIN_STEP = 0, PMB_ENTRY_SELECT_ACTIONS = 1 };
+int pmb_obs_bf16_supported(const pmb_dims* d, int32_t entry);
 
 /* Flat parameter layout.  Agent tensors keep the reference order (modules/agents/rnn_agent.py:19-21);
  * the mixer puts the four hypernet weight matrices first so they form ONE [ (N+3)E, S ]

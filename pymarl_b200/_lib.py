@@ -23,6 +23,8 @@ PARAM_ORDER = [  # enum pmb_param_id
 ]
 STAT_IDS = dict(mask_sum=0, td2_sum=1, tdabs_sum=2, qtaken_sum=3, target_sum=4, grad_norm=5, loss=6, clip_coef=7)
 STATS_LEN = 16
+OBS_DTYPE_IDS = {th.float32: 0, th.bfloat16: 1}           # enum pmb_dtype
+ENTRY_TRAIN_STEP, ENTRY_SELECT_ACTIONS = 0, 1             # enum pmb_entry
 DP_TAIL_FLOATS = 16          # PMB_DP_TAIL_FLOATS
 
 
@@ -40,7 +42,8 @@ class Batch(C.Structure):
                 ("reward", C.c_void_p), ("reward_sb", C.c_int64),
                 ("terminated", C.c_void_p), ("terminated_sb", C.c_int64),
                 ("filled", C.c_void_p), ("filled_sb", C.c_int64),
-                ("ep_index", C.c_void_p)]
+                ("ep_index", C.c_void_p),
+                ("obs_dtype", C.c_int32)]          # enum pmb_dtype
 
 
 class Layout(C.Structure):
@@ -97,6 +100,7 @@ _SIGS = {
     "pmb_h2d_rows": (C.c_int, [_P, _P, C.c_int64, C.c_int64, C.c_int64, _P]),
     "pmb_device_info": (C.c_int, [C.POINTER(C.c_int32)] * 3 + [C.POINTER(C.c_int64)]),
     "pmb_flat_layout": (C.c_int, [C.POINTER(Dims), C.POINTER(Layout)]),
+    "pmb_obs_bf16_supported": (C.c_int, [C.POINTER(Dims), C.c_int32]),
     "pmb_learner_workspace_bytes": (C.c_int64, [C.POINTER(Dims)]),
     "pmb_learner_workspace_views": (C.c_int, [C.POINTER(Dims), _P, C.c_int64, C.POINTER(WsViews)]),
     "pmb_agent_fc1_fwd": (C.c_int, [C.POINTER(Dims), C.POINTER(Batch), C.c_int32, C.c_int32, _P, _P, _P]),
@@ -278,11 +282,19 @@ def gather_episodes(src_tensors, ep_ids, n_src):
     return out
 
 
-def make_batch(fields, need_state=True, keep=None, ep_index=None):
+def obs_bf16_supported(dims, entry):
+    """Whether the kernels of ``entry`` (ENTRY_TRAIN_STEP / ENTRY_SELECT_ACTIONS) read bf16 obs natively for ``dims``."""
+    return lib().pmb_obs_bf16_supported(C.byref(dims), int(entry)) == 1
+
+
+def make_batch(fields, need_state=True, keep=None, ep_index=None, dims=None, entry=None):
     """Build the pmb_batch view of an EpisodeBatch-like mapping (``fields[k]`` -> tensor).
     Tensors that are not on CUDA, have the wrong dtype or non-contiguous inner dims are
-    converted (the converted tensors are appended to ``keep`` so they outlive the call)."""
+    converted (the converted tensors are appended to ``keep`` so they outlive the call).
+    bf16 obs (a scheme with ``"obs": {..., "dtype": th.bfloat16}``) is passed through as it is when ``dims`` and
+    ``entry`` name a call whose kernels read it natively (obs_bf16_supported); otherwise it is converted to fp32."""
     b = Batch()
+    b.obs_dtype = 0
     names = [("obs", "obs"), ("state", "state"), ("actions", "actions"), ("avail", "avail_actions"),
              ("reward", "reward"), ("terminated", "terminated"), ("filled", "filled")]
     for cname, key in names:
@@ -292,7 +304,10 @@ def make_batch(fields, need_state=True, keep=None, ep_index=None):
             continue
         t = fields[key]
         require_cuda(t, "batch[%r]" % key)
-        if t.dtype != _FIELD_DTYPES[key]:
+        if key == "obs" and t.dtype == th.bfloat16 and dims is not None and entry is not None \
+                and obs_bf16_supported(dims, entry):
+            b.obs_dtype = OBS_DTYPE_IDS[th.bfloat16]
+        elif t.dtype != _FIELD_DTYPES[key]:
             t = t.to(_FIELD_DTYPES[key])
         inner = 1
         for s in t.shape[1:]:

@@ -52,11 +52,11 @@ class BasicMAC:
                               A=a.n_actions, H=a.rnn_hidden_dim, E=1, obs_last_action=a.obs_last_action,
                               obs_agent_id=a.obs_agent_id, mixer=None, precision=getattr(a, "precision", "fp32"))
 
-    def _step_batch(self, ep_batch, t, keep):
+    def _step_batch(self, ep_batch, t, keep, dims):
         """pmb_batch with just the fields a rollout step reads.  When the runner keeps its
         batch on the host (reference behaviour, basic_controller.py:32,105,113) only the
         timesteps the step needs are copied, re-based so that the kernel's index t maps onto
-        them."""
+        them.  bf16 obs stays bf16 where the rollout kernels read it natively for ``dims``."""
         dev = self._device()
         fields = {}
         if ep_batch["obs"].is_cuda:
@@ -79,7 +79,7 @@ class BasicMAC:
             self._dummies = (zero, zero.to(th.uint8))
         zero, zero_u8 = self._dummies
         fields.update(state=zero, reward=zero, terminated=zero_u8)
-        b = _lib.make_batch(fields, need_state=False, keep=keep)
+        b = _lib.make_batch(fields, need_state=False, keep=keep, dims=dims, entry=_lib.ENTRY_SELECT_ACTIONS)
         return b, t_local, T_local
 
     def _run_step(self, ep_batch, t, epsilon=None, u=None, expo=None, seed=0, offset=0, want_actions=False, want_q=True):
@@ -87,7 +87,7 @@ class BasicMAC:
         _lib.require_cuda(self.agent.fc1.weight, "agent parameters")
         keep = []
         dims = self._dims(ep_batch)
-        batch, t_local, T_local = self._step_batch(ep_batch, t, keep)
+        batch, t_local, T_local = self._step_batch(ep_batch, t, keep, dims)
         dims.T = T_local
         B, N, A, H = dims.B, dims.N, dims.A, dims.H
         flat = C.c_void_p(_flat.ensure_block(self.agent, "agent", dims))

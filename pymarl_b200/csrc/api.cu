@@ -71,6 +71,7 @@ int tc_gemm_atb_ti(const uint8_t* d_ti, int T, int N, int64_t R, int n_tiles, co
                    float* out, int64_t ldo, float* bias_out, void* scratch, int64_t scratch_bytes, cudaStream_t s);
 int64_t tc_atb_ti_scratch_bytes(int T, int n_tiles, int K);
 int64_t tc_fc1_scratch_bytes(const pmb_dims* d);
+bool tc_fc1_streams(const pmb_dims* d, int obs_dtype);
 
 static thread_local char g_err[512] = "";
 std::atomic<long long> g_launch_count{0};
@@ -221,6 +222,31 @@ bool fused_tc_path(const pmb_dims* d) {
 // pmb_dims.reserved bit 1 (pmb_qlearner_train_step): skip the padded steps of a ragged batch.  Ignored off the fused path.
 bool skip_padding(const pmb_dims* d) { return (d->reserved & 2) && fused_tc_path(d); }
 
+bool rollout_tc_ok(const pmb_dims* d) {
+    return d->precision == PMB_PREC_BF16 && d->H == 64 && d->A <= 64 && d->O <= 320;
+}
+
+// Where the kernels read bf16 obs (pmb_batch.obs_dtype) natively: the streaming fc1 kernels are the only obs readers of
+// the fused learner step (the fc1 / fc2 weight gradients read the obs tile images they write) and of the tensor-core
+// rollout step.
+bool obs_bf16_native(const pmb_dims* d, int entry) {
+    if (entry == PMB_ENTRY_TRAIN_STEP) return fused_tc_path(d) && tc_fc1_streams(d, PMB_DTYPE_BF16);
+    if (entry == PMB_ENTRY_SELECT_ACTIONS) return rollout_tc_ok(d) && tc_fc1_streams(d, PMB_DTYPE_BF16);
+    return false;
+}
+
+// batch.obs_dtype of a call to `who`: fp32 always, bf16 where `entry` reads it natively (entry < 0: nowhere)
+int check_obs_dtype(const pmb_dims* d, const pmb_batch* b, int entry, const char* who) {
+    PMB_REQUIRE(b->obs_dtype == PMB_DTYPE_F32 || b->obs_dtype == PMB_DTYPE_BF16, "%s: unknown batch.obs_dtype %d", who,
+                (int)b->obs_dtype);
+    PMB_REQUIRE(b->obs_dtype == PMB_DTYPE_F32 || (entry >= 0 && obs_bf16_native(d, entry)),
+                "%s: bf16 obs is not read natively for these dims (see pmb_obs_bf16_supported); convert obs to fp32", who);
+    return PMB_OK;
+}
+
+// batch.obs of an entry point that accepted fp32 obs only
+const float* obs_f32(const pmb_batch* b) { return static_cast<const float*>(b->obs); }
+
 int64_t agent_bwd_scratch(const pmb_dims* d) {
     const int64_t rows = (int64_t)d->T * d->B * d->N;
     int64_t a = atb_scratch_bytes(d->precision, 3 * d->H, d->H, rows);
@@ -334,7 +360,7 @@ int fc1_fwd(const pmb_dims* d, const pmb_batch* b, int t0, int nt, const AgentPa
     ep.T_batch = d->T; ep.t0 = t0; ep.nt = nt; ep.N = d->N; ep.O = d->O; ep.A = d->A; ep.H = d->H;
     ep.D_in = d_in_of(d); ep.use_act = d->obs_last_action; ep.use_id = d->obs_agent_id;
     ep.R = (int64_t)d->B * d->N;
-    return launch_fc1_gemm(b->obs + (int64_t)t0 * d->N * d->O, map, M, d->O, ap.fc1_w, ep.D_in, d->H, ep, s);
+    return launch_fc1_gemm(obs_f32(b) + (int64_t)t0 * d->N * d->O, map, M, d->O, ap.fc1_w, ep.D_in, d->H, ep, s);
 }
 
 int agent_bwd(const pmb_dims* d, const pmb_batch* b, const float* flat_agent, const float* x_on, const float* h_stash,
@@ -364,7 +390,7 @@ int agent_bwd(const pmb_dims* d, const pmb_batch* b, const float* flat_agent, co
     // fc1.weight[:, :O] / fc1.bias:  dpre1^T . obs   (dpre1 time major, obs batch major)
     RowMap dmap{(int64_t)d->N * H, R * H, (int64_t)H, d->T, d->N};
     RowMap omap{b->obs_sb, (int64_t)d->N * d->O, (int64_t)d->O, d->T, d->N};
-    rc = gemm_atb_any(prec, dpre1, dmap, H, b->obs, omap, d->O, rows, gr.fc1_w, d_in_of(d), gr.fc1_b, scratch,
+    rc = gemm_atb_any(prec, dpre1, dmap, H, obs_f32(b), omap, d->O, rows, gr.fc1_w, d_in_of(d), gr.fc1_b, scratch,
                       scratch_bytes, s);
     if (rc) return rc;
     PHASE(s, "agent_scatter_grads");
@@ -382,10 +408,6 @@ int pack_gru_images(const pmb_dims* d, const AgentParams& ap, char* base, cudaSt
     const float* p[4] = {ap.w_ih, ap.w_hh, ap.fc2_w, nullptr};
     int r[4] = {192, 192, d->A, 64 - d->A}, l[4] = {64, 64, 64, 64};
     return tc_pack_w(p, r, l, 4, 64, reinterpret_cast<__nv_bfloat16*>(base), s);
-}
-
-bool rollout_tc_ok(const pmb_dims* d) {
-    return d->precision == PMB_PREC_BF16 && d->H == 64 && d->A <= 64 && d->O <= 320;
 }
 
 }  // namespace
@@ -454,6 +476,11 @@ int pmb_flat_layout(const pmb_dims* d, pmb_layout* out) {
     return PMB_OK;
 }
 
+int pmb_obs_bf16_supported(const pmb_dims* d, int32_t entry) {
+    if (validate_dims(d)) return 0;
+    return obs_bf16_native(d, entry) ? 1 : 0;
+}
+
 int64_t pmb_learner_workspace_bytes(const pmb_dims* d) {
     if (validate_dims(d) || d->T < 2) return -1;
     return plan_workspace(d).total;
@@ -477,6 +504,7 @@ int pmb_agent_fc1_fwd(const pmb_dims* d, const pmb_batch* b, int32_t t0, int32_t
     PMB_REQUIRE(b == nullptr || b->ep_index == nullptr, "pmb_agent_fc1_fwd: batch.ep_index is only supported by pmb_qlearner_train_step");
     PMB_REQUIRE(t0 >= 0 && nt > 0 && t0 + nt <= d->T, "fc1_fwd: bad time range [%d, %d) for T = %d", t0, t0 + nt, d->T);
     PMB_REQUIRE(!d->obs_last_action || (b->actions && b->filled), "fc1_fwd: obs_last_action needs actions and filled");
+    if ((rc = check_obs_dtype(d, b, -1, "pmb_agent_fc1_fwd"))) return rc;
     return fc1_fwd(d, b, t0, nt, agent_params(d, flat_agent), x_out, (cudaStream_t)stream);
 }
 
@@ -566,6 +594,7 @@ int pmb_agent_unroll_bwd(const pmb_dims* d, const pmb_batch* b, const float* fla
     PMB_REQUIRE(b == nullptr || b->ep_index == nullptr, "pmb_agent_unroll_bwd: batch.ep_index is only supported by pmb_qlearner_train_step");
     PMB_REQUIRE(b && b->obs && b->actions && b->filled && flat_agent && x_on && h_stash && gates && d_chosen && dpre1 &&
                     flat_grad_agent && scratch, "agent_unroll_bwd: NULL pointer");
+    if ((rc = check_obs_dtype(d, b, -1, "pmb_agent_unroll_bwd"))) return rc;
     return agent_bwd(d, b, flat_agent, x_on, h_stash, gates, d_chosen, dpre1, flat_grad_agent, scratch, scratch_bytes,
                      (cudaStream_t)stream);
 }
@@ -615,6 +644,7 @@ int pmb_select_actions_step(const pmb_dims* d, const pmb_batch* b, int32_t t, co
     PMB_REQUIRE(b == nullptr || b->ep_index == nullptr, "pmb_select_actions_step: batch.ep_index is only supported by pmb_qlearner_train_step");
     PMB_REQUIRE(t >= 0 && t < d->T, "select_actions_step: t = %d outside [0, %d)", t, d->T);
     PMB_REQUIRE((u == nullptr) == (expo == nullptr), "select_actions_step: inject both u and expo or neither");
+    if ((rc = check_obs_dtype(d, b, PMB_ENTRY_SELECT_ACTIONS, "pmb_select_actions_step"))) return rc;
     if (scratch_bytes < pmb_select_actions_workspace_bytes(d)) { set_error("select_actions_step: scratch too small"); return PMB_ERR_WORKSPACE; }
     cudaStream_t s = (cudaStream_t)stream;
     const int64_t R = (int64_t)d->B * d->N;
@@ -695,6 +725,7 @@ int pmb_qlearner_train_step(const pmb_dims* d, const pmb_batch* b, const pmb_hpa
     PMB_REQUIRE(b && hp && flat_p && flat_g && flat_sq && flat_target && workspace && stats, "train_step: NULL pointer");
     PMB_REQUIRE(b->obs && b->actions && b->avail && b->reward && b->terminated && b->filled, "train_step: batch field is NULL");
     PMB_REQUIRE(d->mixer != PMB_MIXER_QMIX || b->state, "train_step: QMIX needs batch.state");
+    if ((rc = check_obs_dtype(d, b, PMB_ENTRY_TRAIN_STEP, "pmb_qlearner_train_step"))) return rc;
     cudaStream_t s = (cudaStream_t)stream;
     WsPlan plan = plan_workspace(d);
     if (workspace_bytes < plan.total) { set_error("workspace too small: %lld < %lld", (long long)workspace_bytes, (long long)plan.total); return PMB_ERR_WORKSPACE; }
@@ -874,7 +905,7 @@ int pmb_qlearner_train_step(const pmb_dims* d, const pmb_batch* b, const pmb_hpa
         } else {
             PHASE(s, "dW_fc1_tc");
             RowMap omap{b->obs_sb, (int64_t)d->N * d->O, (int64_t)d->O, d->T, d->N};
-            if ((rc = tc_gemm_atb_ti(x_tg_ti, d->T, d->N, R, n_tiles, b->obs, omap, d->O, gr.fc1_w, d_in_of(d), gr.fc1_b,
+            if ((rc = tc_gemm_atb_ti(x_tg_ti, d->T, d->N, R, n_tiles, obs_f32(b), omap, d->O, gr.fc1_w, d_in_of(d), gr.fc1_b,
                                      v.scratch, v.scratch_bytes, s))) return rc;
             PHASE(s, "agent_scatter_grads");
             if ((rc = scatter_grads_dispatch(d, b, v.h_stash, v.x_tg, v.d_chosen, gr, v.scratch, v.scratch_bytes, s,
@@ -1009,6 +1040,7 @@ int pmb_coma_train_step(const pmb_dims* d, const pmb_batch* b, const pmb_coma_hp
                 "coma_train_step: NULL pointer");
     PMB_REQUIRE(b->obs && b->state && b->actions && b->avail && b->reward && b->terminated && b->filled && !b->ep_index,
                 "coma_train_step: batch field is NULL (or ep_index given)");
+    if ((rc = check_obs_dtype(d, b, -1, "pmb_coma_train_step"))) return rc;
     cudaStream_t s = (cudaStream_t)stream;
     ComaPlan P = coma_plan(d);
     if (workspace_bytes < P.total) { set_error("coma workspace too small: %lld < %lld", (long long)workspace_bytes, (long long)P.total); return PMB_ERR_WORKSPACE; }
@@ -1074,6 +1106,7 @@ int pmb_coma_critic_fwd(const pmb_dims* d, const pmb_batch* b, const float* crit
     if (rc) return rc;
     PMB_REQUIRE(b && critic_p && q_out && workspace && b->obs && b->state && b->actions && b->filled && !b->ep_index,
                 "coma_critic_fwd: NULL pointer");
+    if ((rc = check_obs_dtype(d, b, -1, "pmb_coma_critic_fwd"))) return rc;
     PMB_REQUIRE(t0 >= 0 && nt > 0 && t0 + nt <= d->T, "coma_critic_fwd: bad time range");
     cudaStream_t s = (cudaStream_t)stream;
     ComaPlan P = coma_plan(d);

@@ -52,6 +52,7 @@ __global__ void __launch_bounds__(256) gather_episodes_kernel(GatherArgs A) {
             case 16: copy_span<uint4>(s, d, A.bytes[f] / 16); break;
             case 8: copy_span<uint2>(s, d, A.bytes[f] / 8); break;
             case 4: copy_span<uint32_t>(s, d, A.bytes[f] / 4); break;
+            case 2: copy_span<uint16_t>(s, d, A.bytes[f] / 2); break;
             default: copy_span<uint8_t>(s, d, A.bytes[f]); break;
         }
     }
@@ -122,6 +123,7 @@ __global__ void __launch_bounds__(128) batch_update_kernel(UpdateArgs A) {
                 case 16: copy_cell<uint4>(s, d, A.cell[f] / 16); break;
                 case 8: copy_cell<uint2>(s, d, A.cell[f] / 8); break;
                 case 4: copy_cell<uint32_t>(s, d, A.cell[f] / 4); break;
+                case 2: copy_cell<uint16_t>(s, d, A.cell[f] / 2); break;
                 default: copy_cell<uint8_t>(s, d, A.cell[f]); break;
             }
         }
@@ -135,6 +137,12 @@ __global__ void __launch_bounds__(128) batch_update_kernel(UpdateArgs A) {
 }  // namespace pmb
 
 using namespace pmb;
+
+// widest copy unit (16, 8, 4, 2 or 1 bytes) that divides every address and size of a field: a bf16 obs cell of an odd obs
+// dim (570 bytes at O = 285) moves in 2-byte words instead of bytes
+static int vec_width(uintptr_t bits) {
+    return (bits & 15) == 0 ? 16 : ((bits & 7) == 0 ? 8 : ((bits & 3) == 0 ? 4 : ((bits & 1) == 0 ? 2 : 1)));
+}
 
 extern "C" {
 
@@ -153,7 +161,7 @@ int pmb_gather_episodes(const pmb_gather_field* fields, int32_t n_fields, const 
         A.bytes[f] = fields[f].bytes_per_episode;
         const uintptr_t bits = reinterpret_cast<uintptr_t>(fields[f].src) | reinterpret_cast<uintptr_t>(fields[f].dst) |
                                (uintptr_t)fields[f].bytes_per_episode;
-        A.vec[f] = (bits & 15) == 0 ? 16 : ((bits & 7) == 0 ? 8 : ((bits & 3) == 0 ? 4 : 1));
+        A.vec[f] = vec_width(bits);
         if (A.bytes[f] > biggest) biggest = A.bytes[f];
     }
     // enough blocks per episode to give every thread ~32 vectors of the biggest field, at least 4 waves in total
@@ -186,7 +194,7 @@ int pmb_batch_update(const pmb_update_field* fields, int32_t n_fields, const int
         A.onehot[f] = u.onehot_dim;
         const uintptr_t bits = reinterpret_cast<uintptr_t>(u.src) | reinterpret_cast<uintptr_t>(u.dst) | (uintptr_t)u.cell_bytes |
                                (uintptr_t)u.dst_batch_stride_bytes | (uintptr_t)u.dst_time_stride_bytes;
-        A.vec[f] = (bits & 15) == 0 ? 16 : ((bits & 7) == 0 ? 8 : ((bits & 3) == 0 ? 4 : 1));
+        A.vec[f] = vec_width(bits);
     }
     batch_update_kernel<<<(unsigned)(nb * nt), 128, 0, (cudaStream_t)stream>>>(A);
     PMB_LAUNCH_CHECK("batch_update_kernel");

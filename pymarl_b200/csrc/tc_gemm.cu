@@ -506,33 +506,45 @@ int launch_tc_gemm(const GemmParams& P, const Epi& epi, cudaStream_t s) {
 // The generic kernel above feeds A through eight producer warps that load 8 bytes per lane (obs rows are 4-byte
 // aligned only: 285 floats) and convert synchronously, chunk by chunk: ~28 % of the HBM ceiling (ncu, profiles/).
 // Here the copy engine does the streaming:
-//   producer warp : walks the rows of a 16-row group (time-major tile order: a group is 1-2 contiguous runs of
-//                   [B,T,N,O] memory, one per episode), issues ONE cp.async.bulk per run for its 16-byte-aligned
-//                   interior and 4-byte cp.async for the <= 3 floats of head and tail, into a ring of fp32 staging
-//                   slots (never reads outside the run).  3 slots x 18 KB in flight per SM.
-//   8 converter warps : fp32 staging -> bf16 K-major/128B-swizzle A tile (all k-chunks of the tile, 80 KB).
+//   producer warp : walks the rows of a group (time-major tile order: a group is 1-2 contiguous runs of [B,T,N,O]
+//                   memory, one per episode), issues ONE cp.async.bulk per run, widened to 16-byte boundaries, into a
+//                   ring of staging slots in the obs element type.  3 slots x 18 KB in flight per SM.
+//                   A group is 16 rows of fp32 obs or 32 rows of bf16 obs (pmb_batch.obs_dtype): a slot holds about the
+//                   same bytes either way, and the stream is bound by the bytes in flight per SM.
+//   8 converter warps : staging -> bf16 K-major/128B-swizzle A tile (all k-chunks of the tile, 80 KB); fp32 obs is
+//                   rounded to nearest even here, bf16 obs is copied, and both give the same bytes for the same values.
 //   MMA thread    : W (both nets, 128 columns, all chunks) stays resident; 4 tcgen05.mma per chunk, 2 TMEM buffers.
 //   store thread  : the finished A tile IS the obs tile image the weight-gradient kernel wants: one 80 KB bulk store.
 //   4 epilogue warps : Fc1TiEpi (one-hot gathers, bias, ReLU, bf16 x tile images of both nets, ReLU bit mask).
 namespace fs {
 constexpr int MAX_CHUNKS = 5;
-constexpr int GROUP_ROWS = 16, GROUPS = BM / GROUP_ROWS;     // (8 rows x 6 slots measured no better: 8.5 vs 8.2 ms)
+// rows of a staging group (= one slot fill) for obs elements of ES bytes: 64 bytes of every row's 16-row share.
+// (fp32: 8 rows x 6 slots measured no better than 16 x 3: 8.5 vs 8.2 ms)
+// (bf16: 16 rows per group, half the bytes per slot, measured slower than 32: 8.61 against 8.08 ms, with the earlier
+// converter; profiles/r03_obs_bf16.json)
+constexpr int group_rows_of(int es) { return 64 / es; }
+template <int ES> constexpr int group_rows() { return group_rows_of(ES); }
+// staging bytes between two runs of a group: a run starts at the next 128-byte boundary (< 128) plus the 128-byte phase of
+// its source (< 128), and its copy is widened by < 16 bytes - under 272 bytes, so the copies of the runs stay disjoint
+constexpr int RUN_SLACK = 272;
 constexpr int N_SLOTS = 3;                                   // learner step (both nets: W is 16 KB per k-chunk)
 constexpr int N_SLOTS_1NET = 5;                              // rollout step: W of one net is half the size, two more slots fit
 #ifndef PMB_FC1_NCONV
 #define PMB_FC1_NCONV 8
 #endif
 constexpr int N_EPI = 4, MMA_W = 4, PROD_W = 5, N_CONV = PMB_FC1_NCONV;
-constexpr int RPW = GROUP_ROWS / N_CONV;                     // rows of a group per converter warp
 // NS staging slots, one producer warp each (every producer warp owns one staging slot: parity waits are only safe one
 // phase apart), then the converter warps
 constexpr int threads_for(int ns) { return 32 * (PROD_W + ns + N_CONV); }
-static_assert(RPW >= 1 && RPW * N_CONV == GROUP_ROWS, "group rows must divide over the converter warps");
+// a group's rows divide over the converter warps and into the 128-row tile, and the producer writes one row per lane
+static_assert(group_rows<4>() % N_CONV == 0 && group_rows<2>() % N_CONV == 0, "group rows must divide over the converter warps");
+static_assert(BM % group_rows<4>() == 0 && BM % group_rows<2>() == 0, "group rows must divide the tile");
+static_assert(group_rows<4>() <= 32 && group_rows<2>() <= 32, "the producer writes one row table entry per lane");
 }  // namespace fs
 
 struct Fc1StreamParams {
     const int64_t* ep_index;       // optional batch row -> buffer episode
-    const float* obs; int64_t obs_sb;
+    const uint8_t* obs; int64_t obs_sb;   // fp32 or bf16 (the kernels' ES template argument), obs_sb in elements
     const __nv_bfloat16* Wp;       // packed [chunk][128 x 128 B]
     uint8_t* obs_img;              // optional [T*n_tiles][n_chunks][16 KB]
     int64_t R;
@@ -565,6 +577,11 @@ __device__ __forceinline__ int fc1_item(const Fc1StreamParams& P, int k) { retur
 __device__ __forceinline__ float lds_f32(uint32_t addr) {
     float v;
     asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(addr));
+    return v;
+}
+__device__ __forceinline__ uint32_t lds_b32(uint32_t addr) {
+    uint32_t v;
+    asm volatile("ld.shared.b32 %0, [%1];" : "=r"(v) : "r"(addr));
     return v;
 }
 __device__ __forceinline__ void sts_b32(uint32_t addr, uint32_t v) {
@@ -602,33 +619,32 @@ __device__ unsigned long long g_fc1_prof[16];
 #define FC1_PROF_END(ns) do { } while (0)
 #endif
 // The two roles the learner and the rollout kernels below share: the producer warps that stream the obs runs of a
-// 16-row group into the fp32 staging ring, and the converter warps that turn a staged group into bf16 rows of the
-// K-major / 128B-swizzle obs tile (and of the obs image).
+// group into the staging ring, and the converter warps that turn a staged group into bf16 rows of the K-major /
+// 128B-swizzle obs tile (and of the obs image).  ES = bytes of an obs element: 4 (fp32) or 2 (bf16).
 struct Fc1Ring {
     uint8_t* stage;         // [NS][slot_bytes]
-    int* rowoff;            // [NS][16] byte offset of a row in its slot
-    int* rown;              // [NS][16] agent index of the row
+    int* rowinfo;           // [NS][group rows] byte offset of a row in its slot | agent index << 20 (fold_id only); -1: zeros
     uint64_t* st_full;      // [NS]
     uint64_t* st_empty;     // [NS]
 };
 
-template <int NC, int NS>
+template <int NC, int NS, int ES>
 __device__ __forceinline__ void fc1_produce(const Fc1StreamParams& P, const Fc1Ring& ring, int pw, int lane,
                                             long long (&prof_acc)[16]) {
     using namespace fs;
-    constexpr int N_SLOTS = NS;
+    constexpr int N_SLOTS = NS, GROUP_ROWS = group_rows<ES>(), GROUPS = BM / GROUP_ROWS;
     uint8_t* stage = ring.stage;
-    int* rowoff = ring.rowoff;
-    int* rown = ring.rown;
+    int* rowinfo = ring.rowinfo;
     uint64_t* st_full = ring.st_full;
     uint64_t* st_empty = ring.st_empty;
     const int n_items = P.T * P.n_tiles;
+    const uint32_t row_bytes = (uint32_t)P.O * ES;
 
     // Lane i owns the i-th contiguous run of a group (one episode each) and computes its descriptor - global
     // address, staging offset, head / interior / tail split - in closed form, in parallel with the other lanes
     // and BEFORE the slot is free; once it is, every lane just issues its copies.  (The first version walked the
     // runs serially after the wait: ~1.5 us of dependent integer code per group during which the slot sat empty,
-    // which bounded the stream at three slots per (walk + load + convert).)
+    // which bounded the stream at three slots per (walk + load + convert).)  A group has at most 32 runs (N = 1).
     uint32_t git = 0;
     for (int k = blockIdx.x; k < n_items; k += gridDim.x) {
         const int64_t item = fc1_item(P, k);
@@ -639,8 +655,7 @@ __device__ __forceinline__ void fc1_produce(const Fc1StreamParams& P, const Fc1R
             if (slot != pw) continue;
             TMARK(pp0);
             uint8_t* sl = stage + slot * P.slot_bytes;
-            int* ro = rowoff + slot * GROUP_ROWS;
-            int* rn = rown + slot * GROUP_ROWS;
+            int* ri = rowinfo + slot * GROUP_ROWS;
             const int64_t p0 = tile * BM + g * GROUP_ROWS;
             int rows_here = P.R - p0 < GROUP_ROWS ? (int)(P.R - p0) : GROUP_ROWS;     // rows of this group below R
             if (rows_here < 0) rows_here = 0;
@@ -653,21 +668,21 @@ __device__ __forceinline__ void fc1_produce(const Fc1StreamParams& P, const Fc1R
             int cnt = lane == 0 ? first_cnt : (rows_here - lr < P.N ? rows_here - lr : P.N);
             if (cnt < 0) cnt = 0;
             const int n0 = lane == 0 ? n00 : 0;
-            const char* ga = nullptr;
+            const uint8_t* ga = nullptr;
             uint32_t cur = 0, phase = 0, cp_bytes = 0;
             if (cnt > 0) {
-                ga = reinterpret_cast<const char*>(P.obs + ep_row(P.ep_index, (int64_t)b0 + lane) * P.obs_sb +
-                                                   ((t + P.t0) * P.N + n0) * (int64_t)P.O);
+                ga = P.obs + (ep_row(P.ep_index, (int64_t)b0 + lane) * P.obs_sb + ((t + P.t0) * P.N + n0) * (int64_t)P.O) * ES;
                 phase = (uint32_t)(reinterpret_cast<uintptr_t>(ga) & 15);
                 // staging offset: same 128-BYTE phase as the source (the copy engine then moves whole lines: with only the
-                // 16-byte phase matched every line is split and shifted); 320 bytes of slack per run keep the runs - and
+                // 16-byte phase matched every line is split and shifted); RUN_SLACK bytes per run keep the runs - and
                 // the up to 15 bytes copied before / after each of them - disjoint
-                cur = (((uint32_t)lr * P.O * 4u + 127u) & ~127u) + 320u * lane + (uint32_t)(reinterpret_cast<uintptr_t>(ga) & 127);
+                cur = (((uint32_t)lr * row_bytes + 127u) & ~127u) + (uint32_t)RUN_SLACK * lane +
+                      (uint32_t)(reinterpret_cast<uintptr_t>(ga) & 127);
                 // ONE bulk copy per run, widened to 16-byte boundaries on both sides (the extra bytes stay inside the
                 // 16-byte granules the run touches anyway - never another page - and land in the slack).  The first
                 // version copied the aligned interior and fetched head / tail with 4-byte cp.async: with the 32
                 // no-increment barrier arrivals that needs, publishing a slot took ~1600 cycles.
-                cp_bytes = (phase + (uint32_t)cnt * P.O * 4u + 15u) & ~15u;
+                cp_bytes = (phase + (uint32_t)cnt * row_bytes + 15u) & ~15u;
             }
             const uint32_t tx = __reduce_add_sync(0xffffffffu, cp_bytes);
             // L2 prefetch of the same group of this CTA's NEXT tile: the staging ring is all the shared memory that is
@@ -685,10 +700,10 @@ __device__ __forceinline__ void fc1_produce(const Fc1StreamParams& P, const Fc1R
                 const int lr2 = lane == 0 ? 0 : fc + (lane - 1) * P.N;
                 int cnt2 = lane == 0 ? fc : (rows2 - lr2 < P.N ? rows2 - lr2 : P.N);
                 if (cnt2 > 0) {
-                    const char* gb = reinterpret_cast<const char*>(P.obs + ep_row(P.ep_index, (int64_t)c0 + lane) * P.obs_sb +
-                                                                   ((t2 + P.t0) * P.N + (lane == 0 ? m00 : 0)) * (int64_t)P.O);
+                    const uint8_t* gb = P.obs + (ep_row(P.ep_index, (int64_t)c0 + lane) * P.obs_sb +
+                                                 ((t2 + P.t0) * P.N + (lane == 0 ? m00 : 0)) * (int64_t)P.O) * ES;
                     const uintptr_t a0 = (reinterpret_cast<uintptr_t>(gb) + 15) & ~(uintptr_t)15;
-                    const uintptr_t a1 = (reinterpret_cast<uintptr_t>(gb) + (uint64_t)cnt2 * P.O * 4) & ~(uintptr_t)15;
+                    const uintptr_t a1 = (reinterpret_cast<uintptr_t>(gb) + (uint64_t)cnt2 * row_bytes) & ~(uintptr_t)15;
                     if (a1 > a0)
                         asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(a0), "r"((uint32_t)(a1 - a0)) : "memory");
                 }
@@ -701,8 +716,9 @@ __device__ __forceinline__ void fc1_produce(const Fc1StreamParams& P, const Fc1R
             TWAIT(0, &st_empty[slot], ((git / N_SLOTS) & 1) ^ 1);
             TMARK(pp1);
             if (lane < GROUP_ROWS) {
-                ro[lane] = lane < rows_here ? (int)(cur_j + (uint32_t)(lane - lrj) * P.O * 4u) : -1;   // rows beyond R: zeros
-                rn[lane] = (rj == 0 ? n00 : 0) + (lane - lrj);
+                // the agent index is needed where one-hot(agent) goes into the K padding only (N < 64 there)
+                const int nj = P.fold_id ? (rj == 0 ? n00 : 0) + (lane - lrj) : 0;
+                ri[lane] = lane < rows_here ? (int)((cur_j + (uint32_t)(lane - lrj) * row_bytes) | ((uint32_t)nj << 20)) : -1;
             }
             if (cnt > 0) bulk_copy_g2s(sl + cur - phase, ga - phase, cp_bytes, &st_full[slot]);
             __syncwarp();
@@ -715,15 +731,14 @@ __device__ __forceinline__ void fc1_produce(const Fc1StreamParams& P, const Fc1R
 }
 
 // converter warp cw owns rows RPW cw .. RPW cw + RPW - 1 of every group; arrives on a_full once per finished tile
-template <int NC, int NS>
+template <int NC, int NS, int ES>
 __device__ __forceinline__ void fc1_convert(const Fc1StreamParams& P, const Fc1Ring& ring, uint8_t* a_s, uint64_t* a_free,
                                             uint64_t* a_full, int cw, int lane, long long (&prof_acc)[16]) {
     using namespace fs;
-    constexpr int N_SLOTS = NS;
+    constexpr int N_SLOTS = NS, GROUP_ROWS = group_rows<ES>(), GROUPS = BM / GROUP_ROWS, RPW = GROUP_ROWS / N_CONV;
     constexpr int tile_bytes = NC * A_STAGE_BYTES;
     uint8_t* stage = ring.stage;
-    int* rowoff = ring.rowoff;
-    int* rown = ring.rown;
+    int* rowinfo = ring.rowinfo;
     uint64_t* st_full = ring.st_full;
     uint64_t* st_empty = ring.st_empty;
     const int n_items = P.T * P.n_tiles;
@@ -741,42 +756,84 @@ __device__ __forceinline__ void fc1_convert(const Fc1StreamParams& P, const Fc1R
             const int slot = git % N_SLOTS;
             TWAIT(1, &st_full[slot], (git / N_SLOTS) & 1);
             TMARK(pt1);
-            const uint32_t sl = smem_u32(stage + slot * P.slot_bytes) + 8u * lane;
+            // the lane's column pair 2 lane, 2 lane + 1 of chunk c sits at byte 2 ES lane + 64 ES c of the staged row
+            const uint32_t sl = smem_u32(stage + slot * P.slot_bytes) + 2u * ES * lane;
             int offs[RPW], nns[RPW];
 #pragma unroll
             for (int rr = 0; rr < RPW; ++rr) {
-                offs[rr] = rowoff[slot * GROUP_ROWS + RPW * cw + rr];
-                nns[rr] = rown[slot * GROUP_ROWS + RPW * cw + rr];
+                const int info = rowinfo[slot * GROUP_ROWS + RPW * cw + rr];
+                offs[rr] = info < 0 ? -1 : (info & 0xfffff);
+                nns[rr] = info < 0 ? -1 : (info >> 20);
             }
-            float v0[RPW][NC], v1[RPW][NC];
             {
-#pragma unroll
-                for (int rr = 0; rr < RPW; ++rr) {           // all loads first
-                    const int off = offs[rr];
-                    const bool real = off >= 0;
-                    const uint32_t src = sl + (uint32_t)(real ? off : 0);
-#pragma unroll
-                    for (int c = 0; c < NC; ++c) {
-                        v0[rr][c] = 0.f; v1[rr][c] = 0.f;
-                        if (real && (c < c_last || okl0)) v0[rr][c] = lds_f32(src + c * 256);
-                        if (real && (c < c_last || okl1)) v1[rr][c] = lds_f32(src + c * 256 + 4);
-                    }
-                }
                 // pack first (consumes every loaded value), release the staging slot, then write the A tile
                 uint32_t pk[RPW][NC];
+                if constexpr (ES == 4) {
+                    float v0[RPW][NC], v1[RPW][NC];
 #pragma unroll
-                for (int rr = 0; rr < RPW; ++rr) {
-                    const int off = offs[rr];
-                    const int nn = nns[rr];
-                    // one-hot(agent) and the bias column live in the K padding of the last chunk
-                    const bool fold = P.fold_id && off >= 0;
-                    const bool hit0 = fold && j_pad >= 0 && (j_pad == nn || j_pad == P.N);
-                    const bool hit1 = fold && j_pad + 1 >= 0 && (j_pad + 1 == nn || j_pad + 1 == P.N);
+                    for (int rr = 0; rr < RPW; ++rr) {           // all loads first
+                        const int off = offs[rr];
+                        const bool real = off >= 0;
+                        const uint32_t src = sl + (uint32_t)(real ? off : 0);
 #pragma unroll
-                    for (int c = 0; c < NC; ++c) {
-                        float a = v0[rr][c], b = v1[rr][c];
-                        if (c == c_last) { a = hit0 ? 1.0f : a; b = hit1 ? 1.0f : b; }
-                        pk[rr][c] = pack_bf16x2(a, b);
+                        for (int c = 0; c < NC; ++c) {
+                            v0[rr][c] = 0.f; v1[rr][c] = 0.f;
+                            if (real && (c < c_last || okl0)) v0[rr][c] = lds_f32(src + c * 256);
+                            if (real && (c < c_last || okl1)) v1[rr][c] = lds_f32(src + c * 256 + 4);
+                        }
+                    }
+#pragma unroll
+                    for (int rr = 0; rr < RPW; ++rr) {
+                        const int off = offs[rr];
+                        const int nn = nns[rr];
+                        // one-hot(agent) and the bias column live in the K padding of the last chunk
+                        const bool fold = P.fold_id && off >= 0;
+                        const bool hit0 = fold && j_pad >= 0 && (j_pad == nn || j_pad == P.N);
+                        const bool hit1 = fold && j_pad + 1 >= 0 && (j_pad + 1 == nn || j_pad + 1 == P.N);
+#pragma unroll
+                        for (int c = 0; c < NC; ++c) {
+                            float a = v0[rr][c], b = v1[rr][c];
+                            if (c == c_last) { a = hit0 ? 1.0f : a; b = hit1 ? 1.0f : b; }
+                            pk[rr][c] = pack_bf16x2(a, b);
+                        }
+                    }
+                } else {
+                    // bf16: the column pair is one packed word already.  A row of odd O starts at 2 mod 4 every other
+                    // row, where the pair straddles two words: every lane loads the two aligned words around its pair and
+                    // a per-row byte selector picks it out.  (Choosing between one load and two per row compiled to a
+                    // branch around each chunk's loads, which serialised them: 8.1 against 6.5 ms for fp32 obs.)
+                    uint32_t lo[RPW][NC], hi[RPW][NC];
+#pragma unroll
+                    for (int rr = 0; rr < RPW; ++rr) {           // all loads first
+                        const int off = offs[rr];
+                        const bool real = off >= 0;
+                        const uint32_t src = sl + (uint32_t)(real ? (off & ~3) : 0);
+#pragma unroll
+                        for (int c = 0; c < NC; ++c) {
+                            lo[rr][c] = 0u; hi[rr][c] = 0u;
+                            if (real && (c < c_last || okl0)) {
+                                lo[rr][c] = lds_b32(src + c * 128);
+                                hi[rr][c] = lds_b32(src + c * 128 + 4);
+                            }
+                        }
+                    }
+#pragma unroll
+                    for (int rr = 0; rr < RPW; ++rr) {
+                        const int off = offs[rr];
+                        const int nn = nns[rr];
+                        const uint32_t sel = (off & 2) ? 0x5432u : 0x3210u;
+#pragma unroll
+                        for (int c = 0; c < NC; ++c) pk[rr][c] = __byte_perm(lo[rr][c], hi[rr][c], sel);
+                        const bool fold = P.fold_id && off >= 0;
+                        const bool hit0 = fold && j_pad >= 0 && (j_pad == nn || j_pad == P.N);
+                        const bool hit1 = fold && j_pad + 1 >= 0 && (j_pad + 1 == nn || j_pad + 1 == P.N);
+                        // last chunk: column O - 1 may share its word with the next row's first column; zero it, then
+                        // bf16 1.0 (0x3f80) for the one-hot and bias columns
+                        uint32_t w = pk[rr][c_last];
+                        w = okl1 ? w : (w & 0xffffu);
+                        w = hit0 ? ((w & 0xffff0000u) | 0x3f80u) : w;
+                        w = hit1 ? ((w & 0xffffu) | 0x3f800000u) : w;
+                        pk[rr][c_last] = w;
                     }
                 }
                 __syncwarp();
@@ -810,7 +867,7 @@ __device__ __forceinline__ void fc1_convert(const Fc1StreamParams& P, const Fc1R
     }
 }
 
-template <int NC, int NS>
+template <int NC, int NS, int ES>
 __global__ void __launch_bounds__(fs::threads_for(NS), 1) fc1_stream_kernel(Fc1StreamParams P) {
     FC1_PROF_BEGIN;
     using namespace fs;
@@ -823,9 +880,8 @@ __global__ void __launch_bounds__(fs::threads_for(NS), 1) fc1_stream_kernel(Fc1S
     uint8_t* w_s = smem;                                    // [n_chunks][w_chunk]
     uint8_t* a_s = smem + NC * w_chunk;                     // [n_chunks][16 KB]
     uint8_t* stage = a_s + tile_bytes;                      // [N_SLOTS][slot_bytes]
-    int* rowoff = reinterpret_cast<int*>(stage + N_SLOTS * P.slot_bytes);   // [N_SLOTS][16] byte offset of a row in its slot
-    int* rown = rowoff + N_SLOTS * GROUP_ROWS;                              // [N_SLOTS][16] agent index of the row
-    uint64_t* bars = reinterpret_cast<uint64_t*>(rown + N_SLOTS * GROUP_ROWS);
+    int* rowinfo = reinterpret_cast<int*>(stage + N_SLOTS * P.slot_bytes);  // [N_SLOTS][group rows] (Fc1Ring)
+    uint64_t* bars = reinterpret_cast<uint64_t*>(rowinfo + N_SLOTS * group_rows<ES>());
     uint64_t* w_full = bars;
     uint64_t* st_full = bars + 1;            // [N_SLOTS]
     uint64_t* st_empty = st_full + N_SLOTS;  // [N_SLOTS]
@@ -849,7 +905,7 @@ __global__ void __launch_bounds__(fs::threads_for(NS), 1) fc1_stream_kernel(Fc1S
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
     const int n_items = P.T * P.n_tiles;
-    const Fc1Ring ring{stage, rowoff, rown, st_full, st_empty};
+    const Fc1Ring ring{stage, rowinfo, st_full, st_empty};
     // programmatic dependent launch (rollout step only; see gru_rollout_kernel): the next kernel may be scheduled as the
     // CTAs of this grid leave; this kernel reads nothing its predecessor writes and only its epilogue warps write something
     // the predecessor (the GRU step of the previous rollout step) may still be reading - the x images
@@ -865,12 +921,12 @@ __global__ void __launch_bounds__(fs::threads_for(NS), 1) fc1_stream_kernel(Fc1S
             for (int c = 0; c < NC; ++c)
                 bulk_copy_g2s(w_s + c * w_chunk, reinterpret_cast<const uint8_t*>(P.Wp) + c * A_STAGE_BYTES, (uint32_t)w_chunk, w_full);
         }
-        fc1_produce<NC, NS>(P, ring, pw, lane, prof_acc);
+        fc1_produce<NC, NS, ES>(P, ring, pw, lane, prof_acc);
     } else if (warp >= FIRST_CONV_W) {
-        // ===== converters: warp cw owns rows 2cw, 2cw+1 of every group.  Everything that does not depend on the row
+        // ===== converters: warp cw owns rows RPW cw .. RPW cw + RPW - 1 of every group (RPW = 2 fp32, 4 bf16).  Everything that does not depend on the row
         // (which of a lane's two columns per chunk exist, where the one-hot padding columns are) is hoisted: the
         // first version spent ~2400 cycles per group in a serial chain of predicate / address arithmetic. =====
-        fc1_convert<NC, NS>(P, ring, a_s, a_free, a_full, warp - FIRST_CONV_W, lane, prof_acc);
+        fc1_convert<NC, NS, ES>(P, ring, a_s, a_free, a_full, warp - FIRST_CONV_W, lane, prof_acc);
     } else if (warp == MMA_W) {
         if (lane == 0) {
             const uint32_t idesc = umma_idesc_bf16(BM, 64 * P.n_nets, 0, 0);
@@ -1005,7 +1061,7 @@ constexpr int TS_TMEM_W = 256;            // first TMEM column of W
 
 __device__ __forceinline__ void epi_bar_sync() { asm volatile("bar.sync 1, 128;" ::: "memory"); }   // the 4 epilogue warps
 
-template <int NC>
+template <int NC, int ES>
 __global__ void __launch_bounds__(fs::threads_for(fs::N_SLOTS_TS), 1) fc1_stream_ts_kernel(Fc1StreamParams P) {
     FC1_PROF_BEGIN;
     using namespace fs;
@@ -1017,9 +1073,8 @@ __global__ void __launch_bounds__(fs::threads_for(fs::N_SLOTS_TS), 1) fc1_stream
     uint8_t* stage = xs + 2 * A_STAGE_BYTES;                // [NS][slot_bytes]
     float* tab_s = reinterpret_cast<float*>(stage + NS * P.slot_bytes);     // [A][128]: fc1.weight[h][O + a] of both nets
     int* prev_s = reinterpret_cast<int*>(tab_s + P.n_act * 128);            // [2][128] previous action of the tile's rows
-    int* rowoff = prev_s + 2 * BM;
-    int* rown = rowoff + NS * GROUP_ROWS;
-    uint64_t* bars = reinterpret_cast<uint64_t*>(rown + NS * GROUP_ROWS);
+    int* rowinfo = prev_s + 2 * BM;                         // [NS][group rows] (Fc1Ring)
+    uint64_t* bars = reinterpret_cast<uint64_t*>(rowinfo + NS * group_rows<ES>());
     uint64_t* w_full = bars;                 // W is in TMEM (arrivals of the 4 epilogue warps)
     uint64_t* st_full = bars + 1;            // [NS]
     uint64_t* st_empty = st_full + NS;       // [NS]
@@ -1042,12 +1097,12 @@ __global__ void __launch_bounds__(fs::threads_for(fs::N_SLOTS_TS), 1) fc1_stream
     __syncthreads();
     tc_fence_after();
     // (TMEM base and item count are read inside the roles: held across the role branch they spill at 112 registers)
-    const Fc1Ring ring{stage, rowoff, rown, st_full, st_empty};
+    const Fc1Ring ring{stage, rowinfo, st_full, st_empty};
 
     if (warp >= PROD_W && warp < PROD_W + NS) {
-        fc1_produce<NC, NS>(P, ring, warp - PROD_W, lane, prof_acc);
+        fc1_produce<NC, NS, ES>(P, ring, warp - PROD_W, lane, prof_acc);
     } else if (warp >= FIRST_CONV_W) {
-        fc1_convert<NC, NS>(P, ring, a_s, a_free, a_full, warp - FIRST_CONV_W, lane, prof_acc);
+        fc1_convert<NC, NS, ES>(P, ring, a_s, a_free, a_full, warp - FIRST_CONV_W, lane, prof_acc);
     } else if (warp == MMA_W) {
         if (lane == 0) {
             const uint32_t tmem_base = *tmem_slot;
@@ -1325,6 +1380,56 @@ extern "C" int pmb_debug_fc1_prof(unsigned long long* out, int reset) {
     return 0;
 }
 #endif
+// Shared-memory plan of the streaming fc1 kernels for obs elements of `es` bytes
+struct Fc1StreamPlan {
+    int n_chunks, slot_bytes, fold_id;
+    int64_t smem_need;   // fc1_stream_kernel, both nets, N_SLOTS slots
+    int64_t smem_1net;   // fc1_stream_kernel, one net (rollout), N_SLOTS_1NET slots
+    int64_t smem_ts;     // fc1_stream_ts_kernel
+    bool streams;        // tc_fc1_fwd_both with tile images runs a streaming kernel
+};
+static Fc1StreamPlan fc1_stream_plan(const pmb_dims* d, int es) {
+    using namespace tc::fs;
+    Fc1StreamPlan p;
+    const int gr = group_rows_of(es);
+    p.n_chunks = (d->O + tc::BK - 1) / tc::BK;
+    // a group is at most (gr - 1) / N + 2 contiguous runs, each displaced by < RUN_SLACK bytes (see the producer)
+    const int max_runs = std::min(gr, (gr - 1) / d->N + 2);
+    p.slot_bytes = (int)align_up((int64_t)gr * d->O * es + (int64_t)RUN_SLACK * max_runs + 128, 128);
+    p.fold_id = p.n_chunks * tc::BK - d->O >= d->N + 1;
+    const int64_t tab = (int64_t)gr * 4;                     // row table bytes per slot
+    p.smem_need = 1024 + 2 * (int64_t)p.n_chunks * tc::A_STAGE_BYTES + N_SLOTS * ((int64_t)p.slot_bytes + tab) + 256;
+    p.smem_1net = 1024 + (int64_t)p.n_chunks * (tc::A_STAGE_BYTES / 2) + (int64_t)p.n_chunks * tc::A_STAGE_BYTES +
+                  N_SLOTS_1NET * ((int64_t)p.slot_bytes + tab) + 256;
+    p.smem_ts = 1024 + (int64_t)(p.n_chunks + 2) * tc::A_STAGE_BYTES + N_SLOTS_TS * ((int64_t)p.slot_bytes + tab) +
+                (int64_t)d->A * 128 * 4 + 2 * tc::BM * 4 + 256;
+    p.streams = p.n_chunks <= MAX_CHUNKS && p.smem_need <= 232448;
+    return p;
+}
+
+bool tc_fc1_streams(const pmb_dims* d, int obs_dtype) {
+    return fc1_stream_plan(d, obs_dtype == PMB_DTYPE_BF16 ? 2 : 4).streams;
+}
+
+// kind: 0 fc1_stream_ts_kernel, 1 fc1_stream_kernel with N_SLOTS_1NET slots (rollout, PDL), 2 with N_SLOTS slots
+template <int NC, int ES>
+static int launch_fc1_stream(const tc::Fc1StreamParams& Q, int kind, int64_t smem, int grid, cudaStream_t s) {
+    using namespace tc::fs;
+    if (kind == 0) {
+        PMB_SMEM_ATTR((tc::fc1_stream_ts_kernel<NC, ES>), (int)smem);
+        tc::fc1_stream_ts_kernel<NC, ES><<<grid, threads_for(N_SLOTS_TS), (size_t)smem, s>>>(Q);
+    } else if (kind == 1) {
+        PMB_SMEM_ATTR((tc::fc1_stream_kernel<NC, N_SLOTS_1NET, ES>), (int)smem);
+        PMB_CUDA(launch_pdl(tc::fc1_stream_kernel<NC, N_SLOTS_1NET, ES>, dim3(grid), dim3(threads_for(N_SLOTS_1NET)),
+                            (size_t)smem, s, rollout_pdl_enabled(), Q));
+    } else {
+        PMB_SMEM_ATTR((tc::fc1_stream_kernel<NC, N_SLOTS, ES>), (int)smem);
+        tc::fc1_stream_kernel<NC, N_SLOTS, ES><<<grid, threads_for(N_SLOTS), (size_t)smem, s>>>(Q);
+    }
+    PMB_LAUNCH_CHECK("fc1_stream_kernel");
+    return PMB_OK;
+}
+
 int tc_fc1_fwd_both(const pmb_dims* d, const pmb_batch* b, int t0, int nt, const AgentParams& on, const AgentParams& tg,
                     float* x_on, float* x_tg, int tile_images, uint8_t* obs_img_out, uint32_t* relu_mask, void* scratch,
                     int64_t scratch_bytes, cudaStream_t s, int weights_packed, const int32_t* live_items) {
@@ -1341,16 +1446,12 @@ int tc_fc1_fwd_both(const pmb_dims* d, const pmb_batch* b, int t0, int nt, const
     __nv_bfloat16* wp = static_cast<__nv_bfloat16*>(scratch);
     float* tab_act = reinterpret_cast<float*>(static_cast<char*>(scratch) + wp_bytes);
     float* tab_id = reinterpret_cast<float*>(static_cast<char*>(scratch) + wp_bytes + ta_bytes);
+    const bool bf16_obs = b->obs_dtype == PMB_DTYPE_BF16;
     // the streaming kernel packs its own W (fc1_stream_pack_kernel) and needs the agent-id table only when the one-hot
     // columns do not fit the K padding
-    const int n_chunks_s = (d->O + tc::BK - 1) / tc::BK;
-    // a group is at most (GROUP_ROWS - 1) / N + 2 contiguous runs, each displaced by < 320 bytes (see the producer)
-    const int max_runs_s = std::min(tc::fs::GROUP_ROWS, (tc::fs::GROUP_ROWS - 1) / d->N + 2);
-    const int slot_bytes_s = (int)align_up((int64_t)tc::fs::GROUP_ROWS * d->O * 4 + 320 * max_runs_s + 128, 128);
-    const int64_t smem_need_s = 1024 + 2 * (int64_t)n_chunks_s * tc::A_STAGE_BYTES + tc::fs::N_SLOTS * (int64_t)slot_bytes_s +
-                                2 * tc::fs::N_SLOTS * tc::fs::GROUP_ROWS * 4 + 256;
-    const bool use_stream = tile_images && n_chunks_s <= tc::fs::MAX_CHUNKS && smem_need_s <= 232448;
-    const bool fold_id_s = n_chunks_s * tc::BK - d->O >= d->N + 1;
+    const Fc1StreamPlan sp = fc1_stream_plan(d, bf16_obs ? 2 : 4);
+    const bool use_stream = tile_images && sp.streams;
+    if (bf16_obs && !use_stream) { set_error("tc_fc1: bf16 obs needs the streaming fc1 kernel"); return PMB_ERR_INVALID; }
     int rc = PMB_OK;
     if (!use_stream) {
         const float* ptrs[2] = {on.fc1_w, tg.fc1_w};
@@ -1358,7 +1459,7 @@ int tc_fc1_fwd_both(const pmb_dims* d, const pmb_batch* b, int t0, int nt, const
         rc = tc_pack_w(ptrs, rows, lds, 2, d->O, wp, s);
         if (rc) return rc;
     }
-    if ((!use_stream || !fold_id_s) && !(weights_packed && use_stream)) {
+    if ((!use_stream || !sp.fold_id) && !(weights_packed && use_stream)) {
         int n_tab = 2 * (d->A + d->N) * 64;
         fc1_tables_kernel<<<(unsigned)ceil_div(n_tab, 256), 256, 0, s>>>(on.fc1_w, on.fc1_b, tg.fc1_w, tg.fc1_b, d->O, d->A,
                                                                          d->N, D_in, d->obs_last_action, d->obs_agent_id,
@@ -1367,7 +1468,8 @@ int tc_fc1_fwd_both(const pmb_dims* d, const pmb_batch* b, int t0, int nt, const
     }
     const int64_t M = (int64_t)d->B * nt * d->N;
     RowMap map{b->obs_sb, (int64_t)d->N * d->O, (int64_t)d->O, nt, d->N};
-    tc::GemmParams P{b->obs + (int64_t)t0 * d->N * d->O, map, M, d->O, (d->O + tc::BK - 1) / tc::BK, wp, 128,
+    const float* obs_f32 = static_cast<const float*>(b->obs);
+    tc::GemmParams P{obs_f32 + (int64_t)t0 * d->N * d->O, map, M, d->O, (d->O + tc::BK - 1) / tc::BK, wp, 128,
                      0, 0, 0, 0, nullptr, nullptr};
     if (tile_images) {
         // rows in time-major tiled order so that GEMM tiles coincide with the (t, tile) tile images
@@ -1379,12 +1481,8 @@ int tc_fc1_fwd_both(const pmb_dims* d, const pmb_batch* b, int t0, int nt, const
         tc::Fc1TiEpi epi{tab_act, tab_id, b->actions, b->actions_sb, b->filled, b->filled_sb,
                          reinterpret_cast<uint8_t*>(x_on), reinterpret_cast<uint8_t*>(x_tg), t0, nt, d->N, d->A,
                          d->obs_last_action, n_tiles, R, relu_mask};
-        const int n_chunks = (d->O + tc::BK - 1) / tc::BK;
-        const int slot_bytes = slot_bytes_s;
-        const int64_t smem_need = 1024 + 2 * (int64_t)n_chunks * tc::A_STAGE_BYTES + tc::fs::N_SLOTS * (int64_t)slot_bytes +
-                                  2 * tc::fs::N_SLOTS * tc::fs::GROUP_ROWS * 4 + 256;
-        if (n_chunks <= tc::fs::MAX_CHUNKS && smem_need <= 232448) {
-            const int fold_id = n_chunks * tc::BK - d->O >= d->N + 1;
+        if (use_stream) {
+            const int n_chunks = sp.n_chunks, fold_id = sp.fold_id;
             __nv_bfloat16* tab_act16 = reinterpret_cast<__nv_bfloat16*>(static_cast<char*>(scratch) + wp_bytes + ta_bytes + ti_bytes);
             const int64_t n_pack = (int64_t)128 * n_chunks * 8 + (int64_t)d->A * 128;
             if (!weights_packed) {
@@ -1394,8 +1492,9 @@ int tc_fc1_fwd_both(const pmb_dims* d, const pmb_batch* b, int t0, int nt, const
                 PMB_LAUNCH_CHECK("fc1_stream_pack_kernel");
             }
             tc::Fc1StreamParams Q;
-            Q.ep_index = b->ep_index; Q.obs = b->obs; Q.obs_sb = b->obs_sb; Q.Wp = wp; Q.obs_img = obs_img_out; Q.R = R;
-            Q.T = nt; Q.N = d->N; Q.O = d->O; Q.n_tiles = n_tiles; Q.n_chunks = n_chunks; Q.slot_bytes = slot_bytes;
+            Q.ep_index = b->ep_index; Q.obs = static_cast<const uint8_t*>(b->obs); Q.obs_sb = b->obs_sb; Q.Wp = wp;
+            Q.obs_img = obs_img_out; Q.R = R;
+            Q.T = nt; Q.N = d->N; Q.O = d->O; Q.n_tiles = n_tiles; Q.n_chunks = n_chunks; Q.slot_bytes = sp.slot_bytes;
             Q.fold_id = fold_id; Q.tab_act16 = reinterpret_cast<const uint4*>(tab_act16); Q.tab_id = tab_id;
             Q.actions = b->actions; Q.actions_sb = b->actions_sb; Q.filled = b->filled; Q.filled_sb = b->filled_sb;
             Q.x_on = reinterpret_cast<uint8_t*>(x_on); Q.x_tg = reinterpret_cast<uint8_t*>(x_tg);
@@ -1412,30 +1511,17 @@ int tc_fc1_fwd_both(const pmb_dims* d, const pmb_batch* b, int t0, int nt, const
             const int grid = (int)(n_items < sm_count() ? n_items : sm_count());
             // one net (rollout step): W takes half the shared memory, the staging ring gets two more slots when they fit -
             // the stream is bound by the bytes in flight per SM (slot turn-around ~3500 cycles: 3 x 18 KB give 4.6 TB/s)
-            const int64_t smem_1net = 1024 + (int64_t)n_chunks * (tc::A_STAGE_BYTES / 2) + (int64_t)n_chunks * tc::A_STAGE_BYTES +
-                                      tc::fs::N_SLOTS_1NET * (int64_t)slot_bytes + 2 * tc::fs::N_SLOTS_1NET * tc::fs::GROUP_ROWS * 4 + 256;
-            const bool wide_ring = Q.n_nets == 1 && smem_1net <= 232448;
+            const bool wide_ring = Q.n_nets == 1 && sp.smem_1net <= 232448;
             // learner step: W of both nets in tensor memory (fc1_stream_ts_kernel) when the agent id is folded into the K
             // padding and its ring, x stage and last-action table fit; PMB_FC1_TS=0 selects fc1_stream_kernel (A/B switch,
             // read on every call so that one process can run both)
-            const int64_t smem_ts = 1024 + (int64_t)(n_chunks + 2) * tc::A_STAGE_BYTES + tc::fs::N_SLOTS_TS * (int64_t)slot_bytes +
-                                    (int64_t)d->A * 128 * 4 + 2 * tc::BM * 4 + 2 * tc::fs::N_SLOTS_TS * tc::fs::GROUP_ROWS * 4 + 256;
             const char* e_ts = getenv("PMB_FC1_TS");
-            const bool use_ts = Q.n_nets == 2 && fold_id && smem_ts <= 232448 && !(e_ts && e_ts[0] == '0');
-#define PMB_FC1_STREAM_LAUNCH(NC)                                                                                            \
-    case NC:                                                                                                                 \
-        if (use_ts) {                                                                                                        \
-            PMB_SMEM_ATTR((tc::fc1_stream_ts_kernel<NC>), (int)smem_ts);                                                     \
-            tc::fc1_stream_ts_kernel<NC><<<grid, tc::fs::threads_for(tc::fs::N_SLOTS_TS), (size_t)smem_ts, s>>>(Q);          \
-        } else if (wide_ring) {                                                                                              \
-            PMB_SMEM_ATTR((tc::fc1_stream_kernel<NC, tc::fs::N_SLOTS_1NET>), (int)smem_1net);                               \
-            PMB_CUDA(launch_pdl(tc::fc1_stream_kernel<NC, tc::fs::N_SLOTS_1NET>, dim3(grid),                                 \
-                                dim3(tc::fs::threads_for(tc::fs::N_SLOTS_1NET)), (size_t)smem_1net, s, rollout_pdl_enabled(), Q)); \
-        } else {                                                                                                             \
-            PMB_SMEM_ATTR((tc::fc1_stream_kernel<NC, tc::fs::N_SLOTS>), (int)smem_need);                                     \
-            tc::fc1_stream_kernel<NC, tc::fs::N_SLOTS><<<grid, tc::fs::threads_for(tc::fs::N_SLOTS), (size_t)smem_need, s>>>(Q); \
-        }                                                                                                                    \
-        break;
+            const bool use_ts = Q.n_nets == 2 && fold_id && sp.smem_ts <= 232448 && !(e_ts && e_ts[0] == '0');
+            const int kind = use_ts ? 0 : (wide_ring ? 1 : 2);
+            const int64_t smem = use_ts ? sp.smem_ts : (wide_ring ? sp.smem_1net : sp.smem_need);
+#define PMB_FC1_STREAM_LAUNCH(NC)                                                                                          \
+    case NC:                                                                                                               \
+        return bf16_obs ? launch_fc1_stream<NC, 2>(Q, kind, smem, grid, s) : launch_fc1_stream<NC, 4>(Q, kind, smem, grid, s);
             switch (n_chunks) {
                 PMB_FC1_STREAM_LAUNCH(1)
                 PMB_FC1_STREAM_LAUNCH(2)
@@ -1444,8 +1530,8 @@ int tc_fc1_fwd_both(const pmb_dims* d, const pmb_batch* b, int t0, int nt, const
                 PMB_FC1_STREAM_LAUNCH(5)
             }
 #undef PMB_FC1_STREAM_LAUNCH
-            PMB_LAUNCH_CHECK("fc1_stream_kernel");
-            return PMB_OK;
+            set_error("tc_fc1: %d k-chunks", n_chunks);
+            return PMB_ERR_INVALID;
         }
         if (b->ep_index || live_items) { set_error("tc_fc1: ep_index and live items need the streaming kernel (obs dim <= 320)"); return PMB_ERR_INVALID; }
         return tc::launch_tc_gemm(P, epi, s);

@@ -317,7 +317,7 @@ class QLearner:
             main.wait_event(st["copied"][slot])
             fields = {k: st["bufs"][slot][k][:nb] for k in names}
             dims = self._layout_dims(B=nb, T=T, O=O, S=S)
-            pb = _lib.make_batch(fields, need_state=(a.mixer == "qmix"), keep=keep)
+            pb = _lib.make_batch(fields, need_state=(a.mixer == "qmix"), keep=keep, dims=dims, entry=_lib.ENTRY_TRAIN_STEP)
             need = self._ensure_workspace(self._layout_dims(B=chunk, T=T, O=O, S=S), dev)
             _lib.check(L.pmb_qlearner_train_step(C.byref(dims), C.byref(pb), C.byref(hp_chunk), _lib.ptr(f["p"]),
                                                  _lib.ptr(f["g"]), _lib.ptr(f["sq"]), _lib.ptr(f["target"]),
@@ -358,7 +358,8 @@ class QLearner:
                 S *= int(dim)
         dims = self._layout_dims(B=max(B, 1), T=T, O=O, S=S)
         dims.B = B
-        pb = _lib.make_batch(fields, need_state=(a.mixer == "qmix"), keep=keep, ep_index=ep_index)
+        pb = _lib.make_batch(fields, need_state=(a.mixer == "qmix"), keep=keep, ep_index=ep_index, dims=dims,
+                             entry=_lib.ENTRY_TRAIN_STEP)
         need = self._ensure_workspace(dims, dev) if B > 0 else 0
         if dp and (self._dp_scratch is None or self._dp_scratch.device != dev):
             self._dp_scratch = th.empty(4096, dtype=th.float32, device=dev)
