@@ -315,6 +315,34 @@ int pmb_gather_episodes(const pmb_gather_field* fields_host, int32_t n_fields, c
                         int64_t n_src_episodes, pmb_stream stream);
 int pmb_max_t_filled(const int64_t* filled, int64_t B, int32_t T, int64_t filled_sb, int64_t* out, pmb_stream stream);
 
+/* pmb_gather_episode_steps: the first `steps` timesteps of episodes ep_ids[j] of every field, for a replay buffer in HBM or
+ * in pinned host memory (then the GPU reads the sampled episodes over PCIe, nothing is staged on the host).
+ * Field f: src is [n_src_episodes][T_src][cell_bytes], either device memory or page-locked host memory mapped into the
+ * device's address space (cudaHostAlloc / pmb_host_alloc; the library uses its device alias).  Pageable host memory is
+ * PMB_ERR_INVALID.  dst is device memory [n_ids][dst_stride_bytes], 16-byte aligned, dst_stride_bytes a multiple of 16
+ * and >= steps * cell_bytes; row j receives steps * cell_bytes bytes, and the bytes of its last 16-byte word beyond them
+ * are written as zero (row padding).  At most 8 fields; ep_ids is a device array of n_ids ids (any count).
+ * trim != 0: episode j copies only its first F_j = min(steps, l_j + 2) timesteps, l_j = its last t < steps with
+ * filled[id][t] != 0 (F_j = 0 when there is none; filled is the buffer's int64 [n_src_episodes][T_src] field, device or
+ * mapped host memory, the same F as the padded-step skipping of the learner step), and the rest of its `steps` is
+ * written as zeros without reading the source.  trim == 0 copies all `steps` (filled may be NULL).  Ids outside
+ * [0, n_src_episodes) leave their row untouched. */
+typedef struct pmb_step_field {
+    const void* src;
+    void* dst;
+    int64_t cell_bytes;
+    int64_t dst_stride_bytes;
+} pmb_step_field;
+int pmb_gather_episode_steps(const pmb_step_field* fields_host, int32_t n_fields, const int64_t* ep_ids, int64_t n_ids,
+                             int64_t n_src_episodes, int32_t T_src, int32_t steps, const int64_t* filled, int32_t trim,
+                             pmb_stream stream);
+
+/* Page-locked host memory mapped into every device's address space (cudaHostAlloc, portable | mapped), for a replay
+ * buffer that pmb_gather_episode_steps reads in place.  These two are the only calls of the library that allocate, and
+ * only on request.  The memory is not zeroed. */
+int pmb_host_alloc(int64_t bytes, void** out);
+int pmb_host_free(void* p);
+
 /* pmb_batch_update: EpisodeBatch.update(data, bs, ts, mark_filled) (components/episode_buffer.py:98-154) for a batch that
  * lives in HBM, every field of the call in ONE launch.  Source field f is a dense device array [nb][nt][cell_bytes]; cell
  * (i, j) is written to episode b(i) = b_index[i] (device array, may be NULL: b0 + i * b_step), timestep t0 + j of the

@@ -5,6 +5,7 @@ an exception.  The library is built in-tree by ``pymarl_b200.build.build()`` (nv
 """
 import ctypes as C
 import os
+import weakref
 
 import torch as th
 
@@ -65,6 +66,10 @@ class GatherField(C.Structure):
     _fields_ = [("src", C.c_void_p), ("dst", C.c_void_p), ("bytes_per_episode", C.c_int64)]
 
 
+class StepField(C.Structure):
+    _fields_ = [("src", C.c_void_p), ("dst", C.c_void_p), ("cell_bytes", C.c_int64), ("dst_stride_bytes", C.c_int64)]
+
+
 class UpdateField(C.Structure):
     _fields_ = [("src", C.c_void_p), ("dst", C.c_void_p), ("cell_bytes", C.c_int64), ("dst_batch_stride_bytes", C.c_int64),
                 ("dst_time_stride_bytes", C.c_int64), ("onehot_dim", C.c_int32), ("reserved", C.c_int32)]
@@ -94,6 +99,10 @@ _SIGS = {
     "pmb_profile_begin": (C.c_int, []),
     "pmb_profile_end": (C.c_int, [C.POINTER(C.c_float), C.c_char_p, C.c_int32, C.c_int32, C.POINTER(C.c_int32)]),
     "pmb_gather_episodes": (C.c_int, [C.POINTER(GatherField), C.c_int32, _P, C.c_int64, C.c_int64, _P]),
+    "pmb_gather_episode_steps": (C.c_int, [C.POINTER(StepField), C.c_int32, _P, C.c_int64, C.c_int64, C.c_int32, C.c_int32,
+                                           _P, C.c_int32, _P]),
+    "pmb_host_alloc": (C.c_int, [C.c_int64, C.POINTER(C.c_void_p)]),
+    "pmb_host_free": (C.c_int, [_P]),
     "pmb_batch_update": (C.c_int, [C.POINTER(UpdateField), C.c_int32, _P, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_int64,
                                    C.c_int64, _P, C.c_int64, _P]),
     "pmb_max_t_filled": (C.c_int, [_P, C.c_int64, C.c_int32, C.c_int64, _P, _P]),
@@ -279,6 +288,63 @@ def gather_episodes(src_tensors, ep_ids, n_src):
                 raise PmbError("gather_episodes needs contiguous buffer fields (%r is not)" % k)
             arr[j] = GatherField(v.data_ptr(), out[k].data_ptr(), v[0].numel() * v.element_size())
         check(lib().pmb_gather_episodes(arr, len(chunk), ptr(ids), n, n_src, stream_ptr(dev)), "pmb_gather_episodes")
+    return out
+
+
+def host_empty(shape, dtype):
+    """Uninitialised host tensor in page-locked memory that is mapped into the device's address space (pmb_host_alloc),
+    so that gather_episode_steps reads it in place.  Freed when its last view dies.  torch's pinned allocator would
+    round every field of a replay buffer up to a power of two (a 28 GB obs field takes 32 GB); this does not."""
+    n = 1
+    for s in shape:
+        n *= int(s)
+    nbytes = n * th.empty((), dtype=dtype).element_size()
+    p = C.c_void_p()
+    check(lib().pmb_host_alloc(max(nbytes, 1), C.byref(p)), "pmb_host_alloc")
+    raw = (C.c_uint8 * max(nbytes, 1)).from_address(p.value)
+    weakref.finalize(raw, lib().pmb_host_free, C.c_void_p(p.value))      # runs when the storage lets go of `raw`
+    return th.frombuffer(raw, dtype=th.uint8)[:nbytes].view(dtype).view(tuple(shape))
+
+
+def episode_rows(n, shape, dtype, dev):
+    """Device tensor [n, *shape] whose rows start 16-byte aligned (the row stride is rounded up to 16 bytes): the
+    destination layout of gather_episode_steps.  The kernels take any batch stride."""
+    es = th.empty((), dtype=dtype).element_size()
+    inner = 1
+    for s in shape:
+        inner *= int(s)
+    row = -(-inner * es // 16) * 16 // es
+    buf = th.empty(max(n, 1) * row, dtype=dtype, device=dev)
+    return buf.as_strided((n,) + tuple(shape), (row,) + th.empty(tuple(shape), device="meta").stride())
+
+
+def gather_episode_steps(src, ep_ids, steps, out, filled=None):
+    """out[k][j] = src[k][ep_ids[j], :steps] for every key, one launch per 8 fields on the current stream.  src[k]:
+    contiguous [n_src, T_src, ...] buffer fields in HBM or in pinned mapped host memory; out[k]: device tensors from
+    episode_rows(n_ids, (steps, ...)); ep_ids: int64 device tensor.  With `filled` (the buffer's filled field), episode j
+    copies only its first min(steps, last filled step + 2) timesteps and the rest of its row is written as zeros."""
+    keys = list(src)
+    some = src[keys[0]]
+    n_src, T_src = int(some.shape[0]), int(some.shape[1])
+    n = int(ep_ids.numel())
+    dev = out[keys[0]].device
+    for k in keys:
+        v, o = src[k], out[k]
+        if not v.is_contiguous() or tuple(v.shape[:2]) != (n_src, T_src):
+            raise PmbError("gather_episode_steps needs contiguous [n_src, T, ...] buffer fields (%r is not)" % k)
+        if tuple(o.shape) != (n, steps) + tuple(v.shape[2:]) or o.dtype != v.dtype or not o[0].is_contiguous():
+            raise PmbError("gather_episode_steps: out[%r] must be episode_rows(%d, %r)" % (k, n, (steps,) + tuple(v.shape[2:])))
+    if filled is not None and (not filled.is_contiguous() or filled.dtype != th.int64 or tuple(filled.shape[:2]) != (n_src, T_src)):
+        raise PmbError("gather_episode_steps: filled must be the buffer's contiguous int64 [n_src, T] field")
+    for i in range(0, len(keys), 8):
+        chunk = keys[i:i + 8]
+        arr = (StepField * len(chunk))()
+        for j, k in enumerate(chunk):
+            v, o = src[k], out[k]
+            es = v.element_size()
+            arr[j] = StepField(v.data_ptr(), o.data_ptr(), v[0, 0].numel() * es, o.stride(0) * es)
+        check(lib().pmb_gather_episode_steps(arr, len(chunk), ptr(ep_ids), n, n_src, T_src, int(steps), ptr(filled),
+                                             int(filled is not None), stream_ptr(dev)), "pmb_gather_episode_steps")
     return out
 
 

@@ -19,6 +19,8 @@ def _as_tuple(v):
 
 
 class EpisodeBatch:
+    pinned = False          # fields live in page-locked host memory mapped into the device (ReplayBuffer(pin_memory=True))
+
     def __init__(self, scheme, groups, batch_size, max_seq_length, data=None, preprocess=None, device="cpu"):
         self.scheme = scheme.copy()
         self.groups = groups
@@ -55,10 +57,15 @@ class EpisodeBatch:
                 shape = (groups[group],) + shape
             dtype = info.get("dtype", th.float32)
             if info.get("episode_const", False):
-                self.data.episode_data[key] = th.zeros((batch_size,) + shape, dtype=dtype, device=self.device)
+                self.data.episode_data[key] = self._zeros((batch_size,) + shape, dtype)
             else:
-                self.data.transition_data[key] = th.zeros((batch_size, max_seq_length) + shape, dtype=dtype,
-                                                          device=self.device)
+                self.data.transition_data[key] = self._zeros((batch_size, max_seq_length) + shape, dtype)
+
+    def _zeros(self, shape, dtype):
+        if self.pinned:
+            from .. import _lib
+            return _lib.host_empty(shape, dtype).zero_()
+        return th.zeros(shape, dtype=dtype, device=self.device)
 
     def extend(self, scheme, groups=None):
         self._setup_data(scheme, self.groups if groups is None else groups, self.batch_size, self.max_seq_length, None)
@@ -292,18 +299,24 @@ class IndexedEpisodeBatch:
     sampled episodes plus a reference to the buffer, instead of a gathered copy (29 GB at 27m_vs_30m / 4096).
     ``QLearner.train`` hands the ids to the kernels (``pmb_batch.ep_index``), which read the episodes in place.  It
     quacks like the EpisodeBatch the reference's train loop handles (``run.py:207-219``): ``max_t_filled()``,
-    ``batch[:, :t]``, ``.to(device)``, ``batch[key]`` (materialises that field with the gather kernel)."""
+    ``batch[:, :t]``, ``.to(device)``, ``batch[key]`` (materialises that field with the gather kernel).
 
-    def __init__(self, buffer, ep_ids, max_seq_length=None):
+    The buffer may also live in pinned host memory (``ReplayBuffer(..., pin_memory=True)``); then ``host_ids`` holds the
+    ids on the host as well, and the learner's gather kernel pulls exactly the sampled episodes, fields and timesteps
+    over PCIe (pmb_gather_episode_steps): nothing is gathered on the host."""
+
+    def __init__(self, buffer, ep_ids, max_seq_length=None, host_ids=None):
         self.buffer = buffer
         self.ep_ids = ep_ids                       # int64 device tensor
+        self.host_ids = host_ids                   # int64 host tensor when the buffer lives in pinned host memory
         self.batch_size = int(ep_ids.numel())
         self.max_seq_length = buffer.max_seq_length if max_seq_length is None else int(max_seq_length)
         self.scheme, self.groups, self.device = buffer.scheme, buffer.groups, buffer.device
 
     def max_t_filled(self):
         f = self.buffer.data.transition_data["filled"]
-        return th.sum(f.index_select(0, self.ep_ids)[:, :self.max_seq_length], 1).max(0)[0]
+        ids = self.ep_ids if self.host_ids is None else self.host_ids
+        return th.sum(f.index_select(0, ids)[:, :self.max_seq_length], 1).max(0)[0]
 
     def __getitem__(self, item):
         if isinstance(item, str):
@@ -311,12 +324,16 @@ class IndexedEpisodeBatch:
             src = self.buffer.data.transition_data
             if item not in src:
                 raise ValueError(item)
+            if self.host_ids is not None:
+                T, v = self.max_seq_length, src[item]
+                out = {item: _lib.episode_rows(self.batch_size, (T,) + tuple(v.shape[2:]), v.dtype, self.ep_ids.device)}
+                return _lib.gather_episode_steps({item: v}, self.ep_ids, T, out)[item]
             return _lib.gather_episodes({item: src[item]}, self.ep_ids, self.buffer.batch_size)[item][:, :self.max_seq_length]
         if isinstance(item, tuple) and len(item) == 2 and item[0] == slice(None) and isinstance(item[1], slice):
             lo, hi, step = item[1].indices(self.max_seq_length)
             if lo != 0 or step != 1:
                 raise IndexError("an IndexedEpisodeBatch can only be truncated in time: batch[:, :t]")
-            return IndexedEpisodeBatch(self.buffer, self.ep_ids, hi)
+            return IndexedEpisodeBatch(self.buffer, self.ep_ids, hi, self.host_ids)
         raise IndexError("unsupported index for an IndexedEpisodeBatch: {!r}".format(item))
 
     def to(self, device):
@@ -331,15 +348,43 @@ class IndexedEpisodeBatch:
 class ReplayBuffer(EpisodeBatch):
     """Ring buffer of episodes with uniform sampling (episode_buffer.py:263-298).  Sampling
     draws ids on the legacy global numpy RandomState exactly like the reference, so a shared
-    ``np.random.seed`` yields the same episode ids."""
+    ``np.random.seed`` yields the same episode ids.
 
-    def __init__(self, scheme, groups, buffer_size, max_seq_length, preprocess=None, device="cpu"):
+    ``pin_memory=True`` (host buffers) allocates every field in page-locked host memory mapped into the device, which
+    lets ``zero_copy`` sampling read the buffer in place over PCIe; ``pin_memory_()`` moves an existing buffer there."""
+
+    def __init__(self, scheme, groups, buffer_size, max_seq_length, preprocess=None, device="cpu", pin_memory=False):
+        if pin_memory and th.device(device).type != "cpu":
+            raise ValueError("pin_memory is for a buffer in host memory (device='cpu')")
+        self.pinned = bool(pin_memory)
         super().__init__(scheme, groups, buffer_size, max_seq_length, preprocess=preprocess, device=device)
         self.buffer_size = buffer_size
         self.buffer_index = 0
         self.episodes_in_buffer = 0
         # opt-in: sample() returns an IndexedEpisodeBatch (ids only) instead of a gathered copy when the buffer is in HBM
+        # or in pinned host memory
         self.zero_copy = False
+        # CUDA event recorded after the learner's last reads of a zero-copy sample of this host buffer: train() returns
+        # before its gathers have read the episodes, so writes wait on it
+        self.device_reads = None
+
+    def pin_memory_(self):
+        """Move every field into page-locked host memory mapped into the device (one field at a time)."""
+        if th.device(self.device).type != "cpu":
+            raise ValueError("only a buffer in host memory can be pinned")
+        if not self.pinned:
+            from .. import _lib
+            for store in (self.data.transition_data, self.data.episode_data):
+                for k, v in store.items():
+                    store[k] = _lib.host_empty(v.shape, v.dtype).copy_(v)
+            self.pinned = True
+        return self
+
+    def update(self, data, bs=slice(None), ts=slice(None), mark_filled=True):
+        if self.device_reads is not None:
+            self.device_reads.synchronize()
+            self.device_reads = None
+        super().update(data, bs, ts, mark_filled)
 
     def insert_episode_batch(self, ep_batch):
         n = ep_batch.batch_size
@@ -366,6 +411,9 @@ class ReplayBuffer(EpisodeBatch):
         ep_ids = np.random.choice(self.episodes_in_buffer, batch_size, replace=False)
         if self.zero_copy and th.device(self.device).type == "cuda":
             return IndexedEpisodeBatch(self, th.as_tensor(ep_ids, dtype=th.int64).to(self.device))
+        if self.zero_copy and self.pinned:
+            ids = th.as_tensor(ep_ids, dtype=th.int64)
+            return IndexedEpisodeBatch(self, ids.to("cuda"), host_ids=ids)
         return self[ep_ids]
 
     def __repr__(self):

@@ -58,6 +58,116 @@ __global__ void __launch_bounds__(256) gather_episodes_kernel(GatherArgs A) {
     }
 }
 
+// ---- the first `steps` timesteps of sampled episodes, from HBM or over PCIe (pmb_gather_episode_steps) ----------------
+// A replay buffer in pinned host memory is read by this kernel through its device alias, so the copy is PCIe-bound and
+// the read side decides the rate.  One episode's timesteps of one field are ONE contiguous run in source and destination.
+// The source run is read in aligned 16-byte words only: a bf16 obs cell at odd O starts 2-byte aligned, and a narrower
+// read of mapped host memory is a PCIe request of its own.  The words of a tile are staged in shared memory and shifted
+// into place with funnel shifts; destination rows start 16-byte aligned, so every store is a full 16-byte word.  (The
+// copy loop of gather_episodes above needs both sides equally aligned, which these runs are not.)
+// A CTA's unit of work is a group of up to STEPS_TILES_PER_GROUP tiles of one episode, so trim mode reads the episode's
+// `filled` row once per group, not once per tile.  Tiles past the trimmed length F_j are zero-filled without a read.
+constexpr int STEPS_MAX_FIELDS = 8;
+constexpr int STEPS_THREADS = 256;
+constexpr int STEPS_UNROLL = 4;                                  // independent 16-byte loads in flight per thread
+constexpr int STEPS_TILE = STEPS_THREADS * STEPS_UNROLL;         // destination words of one tile (16 KB)
+constexpr int STEPS_TILES_PER_GROUP = 16;
+
+struct StepsArgs {
+    const char* src[STEPS_MAX_FIELDS];       // device addresses
+    char* dst[STEPS_MAX_FIELDS];
+    int64_t cell[STEPS_MAX_FIELDS];          // bytes of one timestep
+    int64_t src_ep[STEPS_MAX_FIELDS];        // T_src * cell
+    int64_t dst_sb[STEPS_MAX_FIELDS];        // destination row stride (bytes, multiple of 16)
+    int32_t tile0[STEPS_MAX_FIELDS + 1];     // first tile of field f in an episode's tile list; [n_fields] = tiles per episode
+    int32_t n_fields, groups_per_ep, steps;
+    const int64_t* ids;
+    int64_t n_ids, n_src;
+    const int64_t* filled;                   // trim mode: [n_src][filled_sb] int64; NULL: copy all `steps`
+    int64_t filled_sb;
+};
+
+__global__ void __launch_bounds__(STEPS_THREADS) gather_steps_kernel(StepsArgs A) {
+    __shared__ uint4 stage[STEPS_TILE + 1];
+    __shared__ int copy_steps;
+    const int tid = threadIdx.x;
+    const uint4 zero = make_uint4(0u, 0u, 0u, 0u);
+    const int64_t n_groups = A.n_ids * A.groups_per_ep;
+    for (int64_t g = blockIdx.x; g < n_groups; g += gridDim.x) {
+        const int64_t j = g / A.groups_per_ep;
+        const int q = (int)(g - j * A.groups_per_ep);
+        const int64_t id = __ldg(A.ids + j);
+        if (id < 0 || id >= A.n_src) continue;                    // invalid id: leave the row untouched (block-uniform)
+        if (tid < 32) {
+            int F = A.steps;
+            if (A.filled) {                                       // F_j = min(steps, l_j + 2), as skip_steps_kernel
+                const int64_t* fr = A.filled + id * A.filled_sb;
+                int last = -1;
+                for (int t0 = A.steps - 1; t0 >= 0 && last < 0; t0 -= 32) {
+                    const int t = t0 - tid;
+                    const unsigned m = __ballot_sync(0xffffffffu, t >= 0 && fr[t] != 0);
+                    if (m) last = t0 - (__ffs((int)m) - 1);
+                }
+                F = last < 0 ? 0 : min(A.steps, last + 2);
+            }
+            if (tid == 0) copy_steps = F;
+        }
+        __syncthreads();
+        const int F = copy_steps;
+        const int r_end = min((q + 1) * STEPS_TILES_PER_GROUP, A.tile0[A.n_fields]);
+        int f = 0;
+        for (int r = q * STEPS_TILES_PER_GROUP; r < r_end; ++r) {
+            while (r >= A.tile0[f + 1]) ++f;
+            const int64_t k0 = (int64_t)(r - A.tile0[f]) * STEPS_TILE;     // first destination word of the tile
+            const int64_t n_copy = (int64_t)F * A.cell[f];
+            const int64_t n_words = ceil_div((int64_t)A.steps * A.cell[f], 16);
+            uint4* d = reinterpret_cast<uint4*>(A.dst[f] + j * A.dst_sb[f]);
+            if (16 * k0 >= n_copy) {                              // trimmed tail: zeros, no read
+                for (int i = tid; i < STEPS_TILE && k0 + i < n_words; i += STEPS_THREADS) d[k0 + i] = zero;
+                continue;
+            }
+            const char* s = A.src[f] + id * A.src_ep[f];
+            const int a = (int)(reinterpret_cast<uintptr_t>(s) & 15);
+            const uint4* sv = reinterpret_cast<const uint4*>(s - a);
+            const int64_t n_src_words = ceil_div(a + n_copy, 16);          // aligned words holding a byte of the copy
+            uint4 v[STEPS_UNROLL];
+#pragma unroll
+            for (int u = 0; u < STEPS_UNROLL; ++u) {
+                const int64_t m = k0 + tid + u * STEPS_THREADS;
+                v[u] = m < n_src_words ? __ldcs(sv + m) : zero;
+            }
+            if (tid == 0) stage[STEPS_TILE] = k0 + STEPS_TILE < n_src_words ? __ldcs(sv + k0 + STEPS_TILE) : zero;
+#pragma unroll
+            for (int u = 0; u < STEPS_UNROLL; ++u) stage[tid + u * STEPS_THREADS] = v[u];
+            __syncthreads();
+            // destination word k = source bytes [a + 16 k, a + 16 k + 16) of the aligned stream
+            const uint32_t* w32 = reinterpret_cast<const uint32_t*>(stage);
+            const unsigned sh = 8u * (unsigned)(a & 3);
+#pragma unroll
+            for (int u = 0; u < STEPS_UNROLL; ++u) {
+                const int i = tid + u * STEPS_THREADS;
+                const int64_t k = k0 + i;
+                if (k >= n_words) break;
+                const int w = 4 * i + (a >> 2);
+                uint32_t o[4];
+#pragma unroll
+                for (int e = 0; e < 4; ++e) o[e] = __funnelshift_r(w32[w + e], w32[w + e + 1], sh);
+                const int64_t valid = n_copy - 16 * k;            // bytes of this word inside the copied prefix
+                if (valid < 16) {
+#pragma unroll
+                    for (int e = 0; e < 4; ++e) {
+                        const int64_t keep = valid - 4 * e;
+                        o[e] = keep <= 0 ? 0u : (keep >= 4 ? o[e] : o[e] & ((1u << (8 * keep)) - 1u));
+                    }
+                }
+                d[k] = make_uint4(o[0], o[1], o[2], o[3]);
+            }
+            __syncthreads();
+        }
+        __syncthreads();                                          // copy_steps is rewritten by the next group
+    }
+}
+
 // max_b sum_t filled[b, t]  (episode_buffer.py:255-256), one block per 256 episodes + atomicMax
 __global__ void __launch_bounds__(256) max_t_filled_kernel(const int64_t* __restrict__ filled, int64_t B, int T, int64_t sb,
                                                            unsigned long long* __restrict__ out) {
@@ -176,7 +286,91 @@ int pmb_gather_episodes(const pmb_gather_field* fields, int32_t n_fields, const 
     return PMB_OK;
 }
 
-int pmb_batch_update(const pmb_update_field* fields, int32_t n_fields, const int64_t* b_index, int64_t b0, int64_t b_step,
+// The address the device reads `p` at: device memory as it is, pinned host memory through its mapped alias.  Pageable
+// host memory has no device address; a kernel that read it would fault, so it is refused here.
+static int device_alias(const void* p, bool host_ok, const void** out, const char* what, int f) {
+    cudaPointerAttributes at;
+    PMB_CUDA(cudaPointerGetAttributes(&at, p));
+    if (at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged) {
+        *out = p;
+        return PMB_OK;
+    }
+    PMB_REQUIRE(at.type == cudaMemoryTypeHost || at.type == cudaMemoryTypeUnregistered,
+                "gather_episode_steps: %s of field %d: unknown memory type", what, f);
+    PMB_REQUIRE(host_ok, "gather_episode_steps: %s of field %d must be device memory", what, f);
+    PMB_REQUIRE(at.type == cudaMemoryTypeHost,
+                "gather_episode_steps: %s of field %d is pageable host memory; the GPU reads a host buffer only when it "
+                "is pinned and mapped (ReplayBuffer(..., pin_memory=True) or pin_memory_())", what, f);
+    void* d = at.devicePointer;
+    if (!d && cudaHostGetDevicePointer(&d, const_cast<void*>(p), 0) != cudaSuccess) {
+        (void)cudaGetLastError();
+        d = nullptr;
+    }
+    PMB_REQUIRE(d, "gather_episode_steps: %s of field %d is pinned host memory that is not mapped into the device", what, f);
+    *out = d;
+    return PMB_OK;
+}
+
+int pmb_gather_episode_steps(const pmb_step_field* fields, int32_t n_fields, const int64_t* ep_ids, int64_t n_ids,
+                             int64_t n_src_episodes, int32_t T_src, int32_t steps, const int64_t* filled, int32_t trim,
+                             pmb_stream stream) {
+    PMB_REQUIRE(fields && n_fields > 0 && n_fields <= STEPS_MAX_FIELDS, "gather_episode_steps: 1..%d fields", STEPS_MAX_FIELDS);
+    PMB_REQUIRE(n_ids >= 0 && n_src_episodes > 0 && steps > 0 && steps <= T_src, "gather_episode_steps: need n_ids >= 0, "
+                "n_src_episodes > 0 and 0 < steps <= T_src");
+    PMB_REQUIRE(!trim || filled, "gather_episode_steps: trim mode needs the buffer's filled field");
+    if (n_ids == 0) return PMB_OK;
+    PMB_REQUIRE(ep_ids, "gather_episode_steps: ep_ids is NULL");
+    StepsArgs A;
+    A.n_fields = n_fields; A.steps = steps; A.ids = ep_ids; A.n_ids = n_ids; A.n_src = n_src_episodes;
+    A.filled = nullptr; A.filled_sb = T_src;
+    if (trim) {
+        const void* fd = nullptr;
+        if (int rc = device_alias(filled, true, &fd, "filled", -1)) return rc;
+        A.filled = static_cast<const int64_t*>(fd);
+    }
+    int64_t tiles = 0;
+    for (int f = 0; f < n_fields; ++f) {
+        const pmb_step_field& u = fields[f];
+        PMB_REQUIRE(u.src && u.dst && u.cell_bytes > 0, "gather_episode_steps: field %d is NULL or empty", f);
+        PMB_REQUIRE(u.dst_stride_bytes % 16 == 0 && reinterpret_cast<uintptr_t>(u.dst) % 16 == 0 &&
+                    u.dst_stride_bytes >= steps * u.cell_bytes,
+                    "gather_episode_steps: field %d: dst must be 16-byte aligned with a stride that is a multiple of 16 "
+                    "and holds steps * cell_bytes", f);
+        const void* s = nullptr;
+        const void* d = nullptr;
+        if (int rc = device_alias(u.src, true, &s, "src", f)) return rc;
+        if (int rc = device_alias(u.dst, false, &d, "dst", f)) return rc;
+        A.src[f] = static_cast<const char*>(s);
+        A.dst[f] = static_cast<char*>(const_cast<void*>(d));
+        A.cell[f] = u.cell_bytes; A.src_ep[f] = (int64_t)T_src * u.cell_bytes; A.dst_sb[f] = u.dst_stride_bytes;
+        A.tile0[f] = (int32_t)tiles;
+        tiles += ceil_div(ceil_div((int64_t)steps * u.cell_bytes, 16), STEPS_TILE);
+    }
+    PMB_REQUIRE(tiles < ((int64_t)1 << 30), "gather_episode_steps: episodes too large");
+    A.tile0[n_fields] = (int32_t)tiles;
+    A.groups_per_ep = (int32_t)ceil_div(tiles, STEPS_TILES_PER_GROUP);
+    // one CTA per SM: 16 KB of loads in flight per SM covers the PCIe round trip many times over, and the CTAs leave
+    // room on every SM for the compute kernels of the other chunk of a streamed learner step
+    const int64_t n_groups = n_ids * A.groups_per_ep;
+    const unsigned grid = (unsigned)(n_groups < sm_count() ? n_groups : sm_count());
+    gather_steps_kernel<<<grid, STEPS_THREADS, 0, (cudaStream_t)stream>>>(A);
+    PMB_LAUNCH_CHECK("gather_steps_kernel");
+    return PMB_OK;
+}
+
+int pmb_host_alloc(int64_t bytes, void** out) {
+    PMB_REQUIRE(out && bytes > 0, "host_alloc: bytes must be > 0");
+    *out = nullptr;
+    PMB_CUDA(cudaHostAlloc(out, (size_t)bytes, cudaHostAllocPortable | cudaHostAllocMapped));
+    return PMB_OK;
+}
+
+int pmb_host_free(void* p) {
+    if (p) PMB_CUDA(cudaFreeHost(p));
+    return PMB_OK;
+}
+
+int pmb_batch_update(const pmb_update_field* fields,int32_t n_fields, const int64_t* b_index, int64_t b0, int64_t b_step,
                      int64_t nb, int64_t n_rows, int64_t t0, int64_t nt, int64_t* filled, int64_t filled_sb, pmb_stream stream) {
     PMB_REQUIRE(fields && n_fields > 0 && n_fields <= UPDATE_MAX_FIELDS, "batch_update: 1..%d fields", UPDATE_MAX_FIELDS);
     PMB_REQUIRE(nb >= 0 && nt > 0 && t0 >= 0 && n_rows > 0 && nb * nt < ((int64_t)1 << 31), "batch_update: bad index range");

@@ -83,6 +83,9 @@ class COMALearner:
         return new
 
     def train(self, batch, t_env: int, episode_num: int):
+        if getattr(batch, "host_ids", None) is not None:
+            raise TypeError("COMALearner does not take zero-copy samples of a host replay buffer; "
+                            "set buffer.zero_copy = False for COMA")
         a = self.args
         f = self._ensure_flat()
         dev = f["ap"].device

@@ -12,6 +12,8 @@ gradients and the five loss sums travel in ONE all-reduce per step and every ran
 identical update.  args.cuda_graph = True replays the whole step as one CUDA graph.
 args.skip_padded_steps = True lets the step skip the padded timesteps of a ragged batch (pmb_dims.reserved
 bit 1; honoured on the fused tensor-core path, ignored elsewhere).
+A zero-copy sample of a replay buffer in pinned host memory (IndexedEpisodeBatch with host_ids) is pulled over PCIe by
+the gather kernel (pmb_gather_episode_steps): chunk by chunk into the streamed step's chunk buffers, or in one piece.
 """
 import copy
 import ctypes as C
@@ -53,6 +55,18 @@ class FusedRMSprop:
             for k in ("lr", "alpha", "eps"):
                 if k in g:
                     self.defaults[k] = g[k]
+
+
+def _host_sample(batch):
+    """A zero-copy sample of a replay buffer that lives in pinned host memory."""
+    return getattr(batch, "host_ids", None) is not None
+
+
+def _mark_buffer_read(batch, stream):
+    """Record on `stream`, after its last gather from the host buffer, the event the buffer's writes wait on."""
+    ev = th.cuda.Event()
+    ev.record(stream)
+    batch.buffer.device_reads = ev
 
 
 class QLearner:
@@ -202,6 +216,16 @@ class QLearner:
         if hasattr(batch, "ep_ids") and hasattr(batch, "buffer"):
             # zero-copy replay sample (IndexedEpisodeBatch): the kernels read the buffer's episodes in place
             ep_index = batch.ep_ids if lo is None else batch.ep_ids[lo:hi]
+            if _host_sample(batch):
+                # buffer in pinned host memory, in one piece: the (rank's) episodes cross PCIe into device rows
+                src, T = batch.buffer.data.transition_data, batch.max_seq_length
+                n = int(ep_index.numel())
+                for k in names:
+                    fields[k] = _lib.episode_rows(n, (T,) + tuple(src[k].shape[2:]), src[k].dtype, dev)
+                trim = src["filled"] if getattr(self.args, "skip_padded_steps", False) else None
+                _lib.gather_episode_steps({k: src[k] for k in names}, ep_index.contiguous(), T, fields, filled=trim)
+                _mark_buffer_read(batch, th.cuda.current_stream(dev))
+                return fields, None, n, T
             for k in names:
                 fields[k] = batch.buffer.data.transition_data[k]
             return fields, ep_index, int(ep_index.numel()), batch.max_seq_length
@@ -256,16 +280,19 @@ class QLearner:
     # the chunk gradients and sums are added up and ONE exchange / clip / RMSprop update follows - the same arithmetic as
     # the data-parallel path with the chunks in the role of the ranks.  The device then holds two chunks and a chunk-sized
     # workspace instead of the whole batch (7 GB + 6.5 GB instead of 29 GB + 52 GB) and the compute hides under the copy.
+    # A zero-copy sample of a pinned host buffer streams the same way; its chunks are gathered from the buffer by the
+    # gather kernel on the copy stream (with args.skip_padded_steps it leaves out each episode's padded tail).
     def _host_stream_plan(self, batch, dp):
         a = self.args
         chunk = int(getattr(a, "host_stream_chunk", 512))
-        if chunk <= 0 or getattr(a, "cuda_graph", False) or (hasattr(batch, "ep_ids") and hasattr(batch, "buffer")):
+        indexed = hasattr(batch, "ep_ids") and hasattr(batch, "buffer")
+        if chunk <= 0 or getattr(a, "cuda_graph", False) or (indexed and not _host_sample(batch)):
             return None
-        if dp and not getattr(a, "host_stream_dp", False):
+        if dp and (indexed or not getattr(a, "host_stream_dp", False)):
             return None        # with data parallelism every rank holds 1/world of the batch already; opt-in (not measured on GPUs)
-        if batch["obs"].is_cuda:
+        if not indexed and batch["obs"].is_cuda:
             return None
-        n_ep = int(batch["obs"].shape[0])
+        n_ep = batch.batch_size if indexed else int(batch["obs"].shape[0])
         lo, hi = 0, n_ep
         if dp and getattr(a, "dp_shard_batch", True):
             lo, hi = data_parallel.shard_slice(n_ep, data_parallel.rank(), data_parallel.world_size())
@@ -286,18 +313,28 @@ class QLearner:
                                  g=None, sums=th.zeros(5, dtype=th.float64, device=dev))
         if st["g"] is None or st["g"].numel() != n:
             st["g"] = th.zeros(n, dtype=th.float32, device=dev)
-        src = {k: batch[k] for k in names}
+        host = _host_sample(batch)
+        if host:                                 # chunk rows of the gather kernel: 16-byte aligned
+            src, T = batch.buffer.data.transition_data, batch.max_seq_length
+            src = {k: src[k] for k in names}
+            shapes = {k: (T,) + tuple(src[k].shape[2:]) for k in names}
+            trim = src["filled"] if getattr(a, "skip_padded_steps", False) else None
+        else:
+            src = {k: batch[k] for k in names}
+            shapes = {k: tuple(src[k].shape[1:]) for k in names}
+            T = src["obs"].shape[1]
+        if st.get("host") != host:
+            st["bufs"], st["host"] = [{}, {}], host
         for slot in st["bufs"]:
             for k in names:
                 t = src[k]
-                shape = (chunk,) + tuple(t.shape[1:])
-                if k not in slot or slot[k].shape != shape or slot[k].dtype != t.dtype:
-                    slot[k] = th.empty(shape, dtype=t.dtype, device=dev)
+                if k not in slot or tuple(slot[k].shape) != (chunk,) + shapes[k] or slot[k].dtype != t.dtype:
+                    slot[k] = _lib.episode_rows(chunk, shapes[k], t.dtype, dev) if host else \
+                        th.empty((chunk,) + shapes[k], dtype=t.dtype, device=dev)
         st["g"].zero_()
         st["sums"].zero_()
         st["copy"].wait_stream(main)             # the chunk buffers may still be read by the previous call's kernels
         hp_chunk = _lib.HParams(hp.gamma, hp.lr, hp.alpha, hp.eps, hp.grad_norm_clip, 0, 1, hp.keep_q)
-        T = src["obs"].shape[1]
         N, O = src["obs"].shape[2], src["obs"].shape[3]
         S = 1
         if "state" in src:
@@ -311,8 +348,12 @@ class QLearner:
             with th.cuda.stream(st["copy"]):
                 if i >= 2:
                     st["copy"].wait_event(st["done"][slot])
-                for k in names:
-                    st["bufs"][slot][k][:nb].copy_(src[k][s0:s1], non_blocking=True)
+                if host:
+                    _lib.gather_episode_steps(src, batch.ep_ids[s0:s1], T, {k: st["bufs"][slot][k][:nb] for k in names},
+                                              filled=trim)
+                else:
+                    for k in names:
+                        st["bufs"][slot][k][:nb].copy_(src[k][s0:s1], non_blocking=True)
                 st["copied"][slot].record(st["copy"])
             main.wait_event(st["copied"][slot])
             fields = {k: st["bufs"][slot][k][:nb] for k in names}
@@ -326,6 +367,9 @@ class QLearner:
             st["g"].add_(f["g"][:n])
             st["sums"].add_(self._stats[:5])
             st["done"][slot].record(main)
+        if host:
+            batch.ep_ids.record_stream(st["copy"])
+            _mark_buffer_read(batch, st["copy"])
         f["g"][:n].copy_(st["g"])
         self._stats[:5].copy_(st["sums"])
         if not dp:
