@@ -80,14 +80,14 @@ typedef struct pmb_dims {
  * round-to-nearest-even) is read natively only where pmb_obs_bf16_supported() says so; every other entry point that reads
  * obs returns PMB_ERR_INVALID for it.  The bf16 tier rounds obs to bf16 before its first use, so there a bf16-stored batch
  * gives results bit-identical to an fp32-stored one holding the same (bf16-representable) values. */
-enum pmb_dtype { PMB_DTYPE_F32 = 0, PMB_DTYPE_BF16 = 1 };
+enum pmb_dtype { PMB_DTYPE_F32 = 0, PMB_DTYPE_BF16 = 1, PMB_DTYPE_U8 = 2 };
 
 /* The EpisodeBatch fields the path reads.  *_sb = batch stride in ELEMENTS (of the field's own type). */
 typedef struct pmb_batch {
     const void*    obs;        int64_t obs_sb;          /* [B,T,N,O] f32, or bf16 (obs_dtype) */
-    const float*   state;      int64_t state_sb;        /* [B,T,S]   f32 (QMIX only, else NULL) */
+    const void*    state;      int64_t state_sb;        /* [B,T,S]   f32, or bf16 (state_dtype) (QMIX only, else NULL) */
     const int64_t* actions;    int64_t actions_sb;      /* [B,T,N,1] i64 */
-    const int32_t* avail;      int64_t avail_sb;        /* [B,T,N,A] i32 */
+    const void*    avail;      int64_t avail_sb;        /* [B,T,N,A] i32, or u8 (avail_dtype) */
     const float*   reward;     int64_t reward_sb;       /* [B,T,1]   f32 */
     const uint8_t* terminated; int64_t terminated_sb;   /* [B,T,1]   u8  */
     const int64_t* filled;     int64_t filled_sb;       /* [B,T,1]   i64 */
@@ -97,6 +97,14 @@ typedef struct pmb_batch {
      * the tensor-core tier of pmb_qlearner_train_step only. */
     const int64_t* ep_index;
     int32_t obs_dtype;         /* enum pmb_dtype; 0 (fp32) is always accepted, any value but 0 and 1 is PMB_ERR_INVALID */
+    /* Compact state / avail storage ("state": {..., "dtype": th.bfloat16}, "avail_actions": {..., "dtype": th.uint8} or
+     * th.bool, passed as uint8).  Read natively only where pmb_field_dtype_supported() says so; elsewhere, and for any
+     * other value, PMB_ERR_INVALID.  The tensor-core mixer rounds state to bf16 before its first use and avail holds 0 / 1,
+     * so the results are bit-identical to fp32 / i32 storage of the same values.
+     * The two fields take what was the struct's tail padding: sizeof(pmb_batch) stays 128 and a zero-initialised struct
+     * laid out by an earlier header keeps its meaning. */
+    int16_t state_dtype;       /* 0 = f32 (always accepted), PMB_DTYPE_BF16 */
+    int16_t avail_dtype;       /* 0 = i32, the reference's th.int (always accepted), PMB_DTYPE_U8 */
 } pmb_batch;
 
 /* 1 where the kernels of `entry` read PMB_DTYPE_BF16 obs natively for these dims, else 0 (host only, no device call):
@@ -108,6 +116,17 @@ typedef struct pmb_batch {
  * obs only: convert first. */
 enum pmb_entry { PMB_ENTRY_TRAIN_STEP = 0, PMB_ENTRY_SELECT_ACTIONS = 1 };
 int pmb_obs_bf16_supported(const pmb_dims* d, int32_t entry);
+
+/* 1 where the kernels of `entry` accept `field` stored as `dtype` for these dims, else 0 (host only, no device call).
+ * dtype 0 (the reference's type: f32 obs / state, i32 avail) is accepted everywhere.  Besides that:
+ *   PMB_FIELD_OBS,   PMB_DTYPE_BF16  as pmb_obs_bf16_supported()
+ *   PMB_FIELD_STATE, PMB_DTYPE_BF16  PMB_ENTRY_TRAIN_STEP where the tensor-core mixer runs (bf16 tier, QMIX with E = 32)
+ *   PMB_FIELD_AVAIL, PMB_DTYPE_U8    PMB_ENTRY_TRAIN_STEP where the tensor-core agent runs (bf16 tier, H = 64, A <= 64);
+ *                                    PMB_ENTRY_SELECT_ACTIONS on the tensor-core tier (bf16 tier, H = 64, A <= 64, O <= 320)
+ * The fp32 tier, pmb_target_select, pmb_epsilon_greedy, pmb_mixer_* and the COMA entry points read f32 state and i32
+ * avail only: convert first. */
+enum pmb_field { PMB_FIELD_OBS = 0, PMB_FIELD_STATE = 1, PMB_FIELD_AVAIL = 2 };
+int pmb_field_dtype_supported(const pmb_dims* d, int32_t entry, int32_t field, int32_t dtype);
 
 /* Flat parameter layout.  Agent tensors keep the reference order (modules/agents/rnn_agent.py:19-21);
  * the mixer puts the four hypernet weight matrices first so they form ONE [ (N+3)E, S ]

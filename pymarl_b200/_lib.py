@@ -25,7 +25,9 @@ PARAM_ORDER = [  # enum pmb_param_id
 STAT_IDS = dict(mask_sum=0, td2_sum=1, tdabs_sum=2, qtaken_sum=3, target_sum=4, grad_norm=5, loss=6, clip_coef=7)
 STATS_LEN = 16
 OBS_DTYPE_IDS = {th.float32: 0, th.bfloat16: 1}           # enum pmb_dtype
+DTYPE_F32, DTYPE_BF16, DTYPE_U8 = 0, 1, 2                 # enum pmb_dtype (0 is the reference type: f32, i32 avail)
 ENTRY_TRAIN_STEP, ENTRY_SELECT_ACTIONS = 0, 1             # enum pmb_entry
+FIELD_IDS = {"obs": 0, "state": 1, "avail_actions": 2}    # enum pmb_field
 DP_TAIL_FLOATS = 16          # PMB_DP_TAIL_FLOATS
 
 
@@ -45,6 +47,24 @@ class Batch(C.Structure):
                 ("filled", C.c_void_p), ("filled_sb", C.c_int64),
                 ("ep_index", C.c_void_p),
                 ("obs_dtype", C.c_int32)]          # enum pmb_dtype
+
+
+class _BatchTail(C.Structure):
+    """pmb_batch from obs_dtype on: state_dtype and avail_dtype are int16 in the tail padding of Batch (sizeof stays 128)."""
+    _fields_ = [("obs_dtype", C.c_int32), ("state_dtype", C.c_int16), ("avail_dtype", C.c_int16)]
+
+
+def _tail_field(name):
+    def get(self):
+        return getattr(_BatchTail.from_buffer(self, Batch.obs_dtype.offset), name)
+
+    def put(self, value):
+        setattr(_BatchTail.from_buffer(self, Batch.obs_dtype.offset), name, value)
+    return property(get, put)
+
+
+Batch.state_dtype = _tail_field("state_dtype")           # enum pmb_dtype (0: f32)
+Batch.avail_dtype = _tail_field("avail_dtype")           # enum pmb_dtype (0: i32)
 
 
 class Layout(C.Structure):
@@ -110,6 +130,7 @@ _SIGS = {
     "pmb_device_info": (C.c_int, [C.POINTER(C.c_int32)] * 3 + [C.POINTER(C.c_int64)]),
     "pmb_flat_layout": (C.c_int, [C.POINTER(Dims), C.POINTER(Layout)]),
     "pmb_obs_bf16_supported": (C.c_int, [C.POINTER(Dims), C.c_int32]),
+    "pmb_field_dtype_supported": (C.c_int, [C.POINTER(Dims), C.c_int32, C.c_int32, C.c_int32]),
     "pmb_learner_workspace_bytes": (C.c_int64, [C.POINTER(Dims)]),
     "pmb_learner_workspace_views": (C.c_int, [C.POINTER(Dims), _P, C.c_int64, C.POINTER(WsViews)]),
     "pmb_agent_fc1_fwd": (C.c_int, [C.POINTER(Dims), C.POINTER(Batch), C.c_int32, C.c_int32, _P, _P, _P]),
@@ -353,14 +374,27 @@ def obs_bf16_supported(dims, entry):
     return lib().pmb_obs_bf16_supported(C.byref(dims), int(entry)) == 1
 
 
+def field_dtype_supported(dims, entry, field, dtype):
+    """Whether the kernels of ``entry`` read ``field`` ("obs", "state" or "avail_actions") stored as ``dtype`` (DTYPE_*)
+    natively for ``dims`` (pmb_field_dtype_supported)."""
+    return lib().pmb_field_dtype_supported(C.byref(dims), int(entry), FIELD_IDS[field], int(dtype)) == 1
+
+
+# the compact cell types a kernel may read natively: (field, torch dtype) -> enum pmb_dtype.  bool avail is passed as
+# its uint8 view (one byte holding 0 or 1).
+_COMPACT = {("obs", th.bfloat16): DTYPE_BF16, ("state", th.bfloat16): DTYPE_BF16,
+            ("avail_actions", th.uint8): DTYPE_U8, ("avail_actions", th.bool): DTYPE_U8}
+
+
 def make_batch(fields, need_state=True, keep=None, ep_index=None, dims=None, entry=None):
     """Build the pmb_batch view of an EpisodeBatch-like mapping (``fields[k]`` -> tensor).
     Tensors that are not on CUDA, have the wrong dtype or non-contiguous inner dims are
     converted (the converted tensors are appended to ``keep`` so they outlive the call).
-    bf16 obs (a scheme with ``"obs": {..., "dtype": th.bfloat16}``) is passed through as it is when ``dims`` and
-    ``entry`` name a call whose kernels read it natively (obs_bf16_supported); otherwise it is converted to fp32."""
+    Compact storage chosen in the scheme - bf16 obs or state, uint8 or bool avail_actions - is passed through as it is
+    when ``dims`` and ``entry`` name a call whose kernels read it natively (field_dtype_supported); otherwise it is
+    converted to the reference type."""
     b = Batch()
-    b.obs_dtype = 0
+    b.obs_dtype = b.state_dtype = b.avail_dtype = 0
     names = [("obs", "obs"), ("state", "state"), ("actions", "actions"), ("avail", "avail_actions"),
              ("reward", "reward"), ("terminated", "terminated"), ("filled", "filled")]
     for cname, key in names:
@@ -370,9 +404,11 @@ def make_batch(fields, need_state=True, keep=None, ep_index=None, dims=None, ent
             continue
         t = fields[key]
         require_cuda(t, "batch[%r]" % key)
-        if key == "obs" and t.dtype == th.bfloat16 and dims is not None and entry is not None \
-                and obs_bf16_supported(dims, entry):
-            b.obs_dtype = OBS_DTYPE_IDS[th.bfloat16]
+        code = _COMPACT.get((key, t.dtype))
+        if code is not None and dims is not None and entry is not None and field_dtype_supported(dims, entry, key, code):
+            setattr(b, cname + "_dtype", code)
+            if t.dtype == th.bool:
+                t = t.view(th.uint8)
         elif t.dtype != _FIELD_DTYPES[key]:
             t = t.to(_FIELD_DTYPES[key])
         inner = 1

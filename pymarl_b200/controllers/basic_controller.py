@@ -56,7 +56,7 @@ class BasicMAC:
         """pmb_batch with just the fields a rollout step reads.  When the runner keeps its
         batch on the host (reference behaviour, basic_controller.py:32,105,113) only the
         timesteps the step needs are copied, re-based so that the kernel's index t maps onto
-        them.  bf16 obs stays bf16 where the rollout kernels read it natively for ``dims``."""
+        them.  bf16 obs and uint8 / bool avail stay as they are where the rollout kernels read them natively for ``dims``."""
         dev = self._device()
         fields = {}
         if ep_batch["obs"].is_cuda:

@@ -235,17 +235,46 @@ bool obs_bf16_native(const pmb_dims* d, int entry) {
     return false;
 }
 
-// batch.obs_dtype of a call to `who`: fp32 always, bf16 where `entry` reads it natively (entry < 0: nowhere)
-int check_obs_dtype(const pmb_dims* d, const pmb_batch* b, int entry, const char* who) {
+static_assert(sizeof(pmb_batch) == 128, "pmb_batch: state_dtype / avail_dtype live in the former tail padding");
+
+// Where the kernels read compact state / avail natively: the q-select epilogue is the only avail reader of the
+// tensor-core agent's learner step, state_to_images_kernel the only state reader of the tensor-core mixer, and the
+// rollout kernel the only avail reader of the tensor-core rollout step.
+bool field_dtype_native(const pmb_dims* d, int entry, int field, int dtype) {
+    if (field < PMB_FIELD_OBS || field > PMB_FIELD_AVAIL) return false;
+    if (dtype == PMB_DTYPE_F32) return entry == PMB_ENTRY_TRAIN_STEP || entry == PMB_ENTRY_SELECT_ACTIONS;
+    const bool tc_agent = d->precision == PMB_PREC_BF16 && d->H == 64 && d->A <= 64;
+    const bool tc_mixer = d->precision == PMB_PREC_BF16 && d->mixer == PMB_MIXER_QMIX && d->E == 32;
+    if (field == PMB_FIELD_OBS) return dtype == PMB_DTYPE_BF16 && obs_bf16_native(d, entry);
+    if (field == PMB_FIELD_STATE) return dtype == PMB_DTYPE_BF16 && entry == PMB_ENTRY_TRAIN_STEP && tc_mixer;
+    if (field == PMB_FIELD_AVAIL && dtype == PMB_DTYPE_U8)
+        return (entry == PMB_ENTRY_TRAIN_STEP && tc_agent) || (entry == PMB_ENTRY_SELECT_ACTIONS && rollout_tc_ok(d));
+    return false;
+}
+
+// batch.{obs,state,avail}_dtype of a call to `who`: the reference types always, compact ones where `entry` reads them
+// natively (entry < 0: nowhere)
+int check_dtypes(const pmb_dims* d, const pmb_batch* b, int entry, const char* who) {
     PMB_REQUIRE(b->obs_dtype == PMB_DTYPE_F32 || b->obs_dtype == PMB_DTYPE_BF16, "%s: unknown batch.obs_dtype %d", who,
                 (int)b->obs_dtype);
     PMB_REQUIRE(b->obs_dtype == PMB_DTYPE_F32 || (entry >= 0 && obs_bf16_native(d, entry)),
                 "%s: bf16 obs is not read natively for these dims (see pmb_obs_bf16_supported); convert obs to fp32", who);
+    PMB_REQUIRE(b->state_dtype == PMB_DTYPE_F32 || b->state_dtype == PMB_DTYPE_BF16, "%s: unknown batch.state_dtype %d",
+                who, (int)b->state_dtype);
+    PMB_REQUIRE(b->state_dtype == PMB_DTYPE_F32 || field_dtype_native(d, entry, PMB_FIELD_STATE, b->state_dtype),
+                "%s: bf16 state is not read natively for these dims (see pmb_field_dtype_supported); convert state to fp32",
+                who);
+    PMB_REQUIRE(b->avail_dtype == PMB_DTYPE_F32 || b->avail_dtype == PMB_DTYPE_U8, "%s: unknown batch.avail_dtype %d",
+                who, (int)b->avail_dtype);
+    PMB_REQUIRE(b->avail_dtype == PMB_DTYPE_F32 || field_dtype_native(d, entry, PMB_FIELD_AVAIL, b->avail_dtype),
+                "%s: uint8 avail is not read natively for these dims (see pmb_field_dtype_supported); convert avail to int32",
+                who);
     return PMB_OK;
 }
 
-// batch.obs of an entry point that accepted fp32 obs only
+// the fields of an entry point that accepted the reference types only
 const float* obs_f32(const pmb_batch* b) { return static_cast<const float*>(b->obs); }
+const int32_t* avail_i32(const pmb_batch* b) { return static_cast<const int32_t*>(b->avail); }
 
 int64_t agent_bwd_scratch(const pmb_dims* d) {
     const int64_t rows = (int64_t)d->T * d->B * d->N;
@@ -481,6 +510,11 @@ int pmb_obs_bf16_supported(const pmb_dims* d, int32_t entry) {
     return obs_bf16_native(d, entry) ? 1 : 0;
 }
 
+int pmb_field_dtype_supported(const pmb_dims* d, int32_t entry, int32_t field, int32_t dtype) {
+    if (validate_dims(d)) return 0;
+    return field_dtype_native(d, entry, field, dtype) ? 1 : 0;
+}
+
 int64_t pmb_learner_workspace_bytes(const pmb_dims* d) {
     if (validate_dims(d) || d->T < 2) return -1;
     return plan_workspace(d).total;
@@ -504,7 +538,7 @@ int pmb_agent_fc1_fwd(const pmb_dims* d, const pmb_batch* b, int32_t t0, int32_t
     PMB_REQUIRE(b == nullptr || b->ep_index == nullptr, "pmb_agent_fc1_fwd: batch.ep_index is only supported by pmb_qlearner_train_step");
     PMB_REQUIRE(t0 >= 0 && nt > 0 && t0 + nt <= d->T, "fc1_fwd: bad time range [%d, %d) for T = %d", t0, t0 + nt, d->T);
     PMB_REQUIRE(!d->obs_last_action || (b->actions && b->filled), "fc1_fwd: obs_last_action needs actions and filled");
-    if ((rc = check_obs_dtype(d, b, -1, "pmb_agent_fc1_fwd"))) return rc;
+    if ((rc = check_dtypes(d, b, -1, "pmb_agent_fc1_fwd"))) return rc;
     return fc1_fwd(d, b, t0, nt, agent_params(d, flat_agent), x_out, (cudaStream_t)stream);
 }
 
@@ -537,6 +571,7 @@ int pmb_target_select(const pmb_dims* d, const pmb_batch* b, const float* q_on, 
     PMB_REQUIRE(d->T >= 2, "target_select: T must be >= 2");
     PMB_REQUIRE(b && b->avail && b->actions && q_on && q_tg && chosen && tmax, "target_select: NULL pointer");
     PMB_REQUIRE(b == nullptr || b->ep_index == nullptr, "pmb_target_select: batch.ep_index is only supported by pmb_qlearner_train_step");
+    if ((rc = check_dtypes(d, b, -1, "pmb_target_select"))) return rc;
     return launch_target_select(d, b, q_on, q_tg, chosen, tmax, cur_max, (cudaStream_t)stream);
 }
 
@@ -547,6 +582,7 @@ int pmb_mixer_fwd(const pmb_dims* d, const pmb_batch* b, const float* flat_mixer
     PMB_REQUIRE(d->T >= 2 && (t_off == 0 || t_off == 1), "mixer_fwd: bad T / t_off");
     PMB_REQUIRE(agent_qs && q_tot, "mixer_fwd: NULL pointer");
     PMB_REQUIRE(b == nullptr || b->ep_index == nullptr, "mixer_fwd: batch.ep_index is only supported by pmb_qlearner_train_step");
+    if (b && (rc = check_dtypes(d, b, -1, "pmb_mixer_fwd"))) return rc;
     return launch_mixer_fwd(d, b, flat_mixer, agent_qs, t_off, raw, q_tot, (cudaStream_t)stream);
 }
 
@@ -561,6 +597,7 @@ int pmb_td_loss(const pmb_dims* d, const pmb_batch* b, const float* q_tot, const
     if (rc) return rc;
     PMB_REQUIRE(d->T >= 2, "td_loss: T must be >= 2");
     PMB_REQUIRE(b && b->reward && b->terminated && b->filled && q_tot && t_tot && g_out && stats, "td_loss: NULL pointer");
+    if ((rc = check_dtypes(d, b, -1, "pmb_td_loss"))) return rc;
     return launch_td_loss(d, b, q_tot, t_tot, gamma, g_out, stats, (cudaStream_t)stream);
 }
 
@@ -576,6 +613,7 @@ int pmb_mixer_bwd(const pmb_dims* d, const pmb_batch* b, const float* flat_mixer
     if (rc) return rc;
     PMB_REQUIRE(d->T >= 2 && g && d_agent_qs, "mixer_bwd: bad arguments");
     PMB_REQUIRE(b == nullptr || b->ep_index == nullptr, "mixer_bwd: batch.ep_index is only supported by pmb_qlearner_train_step");
+    if (b && (rc = check_dtypes(d, b, -1, "pmb_mixer_bwd"))) return rc;
     return launch_mixer_bwd(d, b, flat_mixer, agent_qs, raw, g, d_agent_qs, flat_grad_mixer, scratch, scratch_bytes,
                             (cudaStream_t)stream);
 }
@@ -594,7 +632,7 @@ int pmb_agent_unroll_bwd(const pmb_dims* d, const pmb_batch* b, const float* fla
     PMB_REQUIRE(b == nullptr || b->ep_index == nullptr, "pmb_agent_unroll_bwd: batch.ep_index is only supported by pmb_qlearner_train_step");
     PMB_REQUIRE(b && b->obs && b->actions && b->filled && flat_agent && x_on && h_stash && gates && d_chosen && dpre1 &&
                     flat_grad_agent && scratch, "agent_unroll_bwd: NULL pointer");
-    if ((rc = check_obs_dtype(d, b, -1, "pmb_agent_unroll_bwd"))) return rc;
+    if ((rc = check_dtypes(d, b, -1, "pmb_agent_unroll_bwd"))) return rc;
     return agent_bwd(d, b, flat_agent, x_on, h_stash, gates, d_chosen, dpre1, flat_grad_agent, scratch, scratch_bytes,
                      (cudaStream_t)stream);
 }
@@ -644,7 +682,7 @@ int pmb_select_actions_step(const pmb_dims* d, const pmb_batch* b, int32_t t, co
     PMB_REQUIRE(b == nullptr || b->ep_index == nullptr, "pmb_select_actions_step: batch.ep_index is only supported by pmb_qlearner_train_step");
     PMB_REQUIRE(t >= 0 && t < d->T, "select_actions_step: t = %d outside [0, %d)", t, d->T);
     PMB_REQUIRE((u == nullptr) == (expo == nullptr), "select_actions_step: inject both u and expo or neither");
-    if ((rc = check_obs_dtype(d, b, PMB_ENTRY_SELECT_ACTIONS, "pmb_select_actions_step"))) return rc;
+    if ((rc = check_dtypes(d, b, PMB_ENTRY_SELECT_ACTIONS, "pmb_select_actions_step"))) return rc;
     if (scratch_bytes < pmb_select_actions_workspace_bytes(d)) { set_error("select_actions_step: scratch too small"); return PMB_ERR_WORKSPACE; }
     cudaStream_t s = (cudaStream_t)stream;
     const int64_t R = (int64_t)d->B * d->N;
@@ -674,7 +712,8 @@ int pmb_select_actions_step(const pmb_dims* d, const pmb_batch* b, int32_t t, co
         fp.x_ti = x_ti; fp.h0 = hidden; fp.h_ti = nullptr; fp.g_ti = nullptr; fp.q = q; fp.h_last = hidden;
         fp.R = R; fp.nt = 1; fp.A = d->A; fp.n_tiles = n_tiles;
         // epsilon-greedy fused into the q epilogue (no q round trip through HBM); q itself only when the caller wants it
-        fp.avail = b->avail + (int64_t)t * d->N * d->A; fp.avail_sb = b->avail_sb; fp.N = d->N; fp.epsilon = epsilon;
+        fp.avail = static_cast<const uint8_t*>(b->avail) + ((int64_t)t * d->N * d->A << (b->avail_dtype == PMB_DTYPE_U8 ? 0 : 2));
+        fp.avail_u8 = b->avail_dtype == PMB_DTYPE_U8; fp.avail_sb = b->avail_sb; fp.N = d->N; fp.epsilon = epsilon;
         fp.u = u; fp.expo = expo; fp.seed = seed; fp.offset = offset; fp.actions_out = actions_out;
         if (actions_out && !q_out) fp.q = nullptr;
         if ((rc = tc_gru_fwd(fp, s))) return rc;
@@ -686,7 +725,7 @@ int pmb_select_actions_step(const pmb_dims* d, const pmb_batch* b, int32_t t, co
         if (rc) return rc;
     }
     if (!actions_out) return PMB_OK;
-    return launch_epsilon_greedy(R, d->N, d->A, q, b->avail + (int64_t)t * d->N * d->A, b->avail_sb, epsilon, u, expo,
+    return launch_epsilon_greedy(R, d->N, d->A, q, avail_i32(b) + (int64_t)t * d->N * d->A, b->avail_sb, epsilon, u, expo,
                                  seed, offset, actions_out, s);
 }
 
@@ -725,7 +764,7 @@ int pmb_qlearner_train_step(const pmb_dims* d, const pmb_batch* b, const pmb_hpa
     PMB_REQUIRE(b && hp && flat_p && flat_g && flat_sq && flat_target && workspace && stats, "train_step: NULL pointer");
     PMB_REQUIRE(b->obs && b->actions && b->avail && b->reward && b->terminated && b->filled, "train_step: batch field is NULL");
     PMB_REQUIRE(d->mixer != PMB_MIXER_QMIX || b->state, "train_step: QMIX needs batch.state");
-    if ((rc = check_obs_dtype(d, b, PMB_ENTRY_TRAIN_STEP, "pmb_qlearner_train_step"))) return rc;
+    if ((rc = check_dtypes(d, b, PMB_ENTRY_TRAIN_STEP, "pmb_qlearner_train_step"))) return rc;
     cudaStream_t s = (cudaStream_t)stream;
     WsPlan plan = plan_workspace(d);
     if (workspace_bytes < plan.total) { set_error("workspace too small: %lld < %lld", (long long)workspace_bytes, (long long)plan.total); return PMB_ERR_WORKSPACE; }
@@ -1040,7 +1079,7 @@ int pmb_coma_train_step(const pmb_dims* d, const pmb_batch* b, const pmb_coma_hp
                 "coma_train_step: NULL pointer");
     PMB_REQUIRE(b->obs && b->state && b->actions && b->avail && b->reward && b->terminated && b->filled && !b->ep_index,
                 "coma_train_step: batch field is NULL (or ep_index given)");
-    if ((rc = check_obs_dtype(d, b, -1, "pmb_coma_train_step"))) return rc;
+    if ((rc = check_dtypes(d, b, -1, "pmb_coma_train_step"))) return rc;
     cudaStream_t s = (cudaStream_t)stream;
     ComaPlan P = coma_plan(d);
     if (workspace_bytes < P.total) { set_error("coma workspace too small: %lld < %lld", (long long)workspace_bytes, (long long)P.total); return PMB_ERR_WORKSPACE; }
@@ -1106,7 +1145,7 @@ int pmb_coma_critic_fwd(const pmb_dims* d, const pmb_batch* b, const float* crit
     if (rc) return rc;
     PMB_REQUIRE(b && critic_p && q_out && workspace && b->obs && b->state && b->actions && b->filled && !b->ep_index,
                 "coma_critic_fwd: NULL pointer");
-    if ((rc = check_obs_dtype(d, b, -1, "pmb_coma_critic_fwd"))) return rc;
+    if ((rc = check_dtypes(d, b, -1, "pmb_coma_critic_fwd"))) return rc;
     PMB_REQUIRE(t0 >= 0 && nt > 0 && t0 + nt <= d->T, "coma_critic_fwd: bad time range");
     cudaStream_t s = (cudaStream_t)stream;
     ComaPlan P = coma_plan(d);

@@ -368,7 +368,7 @@ __global__ void multinomial_kernel(int64_t rows, int A, const float* __restrict_
 int coma_launch_inputs(const pmb_dims* d, const pmb_batch* b, int t0, int nt, float* out, cudaStream_t s) {
     const int64_t rows = (int64_t)d->B * nt * d->N;
     if (rows <= 0) return PMB_OK;
-    coma_inputs_kernel<<<(unsigned)rows, 256, 0, s>>>(d->B, d->N, d->O, d->S, d->A, t0, nt, b->state, b->state_sb, static_cast<const float*>(b->obs), b->obs_sb,
+    coma_inputs_kernel<<<(unsigned)rows, 256, 0, s>>>(d->B, d->N, d->O, d->S, d->A, t0, nt, static_cast<const float*>(b->state), b->state_sb, static_cast<const float*>(b->obs), b->obs_sb,
                                                       b->actions, b->actions_sb, b->filled, b->filled_sb, out);
     PMB_LAUNCH_CHECK("coma_inputs_kernel");
     return PMB_OK;
@@ -431,7 +431,7 @@ int coma_launch_policy(const pmb_dims* d, const pmb_batch* b, float eps, const f
     if (total <= 0) return PMB_OK;
     int64_t grid = ceil_div(total, 8);
     if (grid > 8 * sm_count()) grid = 8 * sm_count();
-    coma_policy_kernel<<<(unsigned)grid, 256, 0, s>>>(d->B, d->T, d->N, d->A, eps, logits, q_vals, b->avail, b->avail_sb,
+    coma_policy_kernel<<<(unsigned)grid, 256, 0, s>>>(d->B, d->T, d->N, d->A, eps, logits, q_vals, static_cast<const int32_t*>(b->avail), b->avail_sb,
                                                      b->actions, b->actions_sb, b->terminated, b->terminated_sb, b->filled,
                                                      b->filled_sb, dlogits, pi_out, stats_row, partials);
     PMB_LAUNCH_CHECK("coma_policy_kernel");

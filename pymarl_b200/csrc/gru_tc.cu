@@ -120,7 +120,8 @@ namespace ro {
 constexpr int WIH = 0, WHH = 24576, W2 = 49152;
 constexpr int SLOT0 = 57344;
 constexpr int S_X = 0, S_HT = 16384, S_HS = 32768, S_AV = S_HS + 32768;      // S_HS: two fp32 tiles (columns 0-31, 32-63)
-constexpr int AV_BYTES = 18432;                               // staged avail rows: 128 * A * 4 <= this (A <= 36)
+constexpr int AV_BYTES = 18432;                               // staged avail rows: 128 * A * 4 <= this (i32, A <= 36)
+constexpr int AV8_SLACK = 48;                                 // u8: bytes per env run beyond its cells (av8_run)
 constexpr int S_XC = S_AV + AV_BYTES;                         // 16 bytes per row: selection hand-over between the two threads of a row
 constexpr int SLOT_BYTES = S_XC + 2048;                       // 86016 = 84 KB (multiple of 1024)
 constexpr int BIAS = SLOT0 + 2 * SLOT_BYTES;
@@ -143,6 +144,73 @@ __device__ unsigned long long g_ro_prof[16];
 #define RMARK(var)
 #define RADD(idx, expr)
 #endif
+// u8 avail staging.  A bulk copy moves 16-byte-aligned, 16-byte-granular runs, and an env's N x A bytes (972 at 27m) are
+// neither, so the loader copies the aligned superset of each env's run [lo, hi): every 16-byte word of it holds a byte
+// of the run, so no word lies outside the allocation.  Env e of the tile (k = e - e0) lands at the 16-aligned
+// dst = 16 floor(x / 16) + 48 k, x = (first row of e in the tile - row0) * A; with L <= len + 30 bytes per superset the
+// next env starts at least len + 33 bytes later, so the runs never overlap, and the whole area is under
+// 128 A + 48 (envs per tile).  A row's cells sit at dst + (start & 15) + (row - ra) A: same alignment as in memory.
+struct Av8Run { const uint8_t* lo; uint32_t dst, bytes, phase; };
+__device__ __forceinline__ Av8Run av8_run(const GruFwdParams& P, int64_t e, int64_t row0, int64_t row_end) {
+    const int64_t ra = e * P.N > row0 ? e * P.N : row0;                        // rows of env e inside the tile
+    const int64_t rb = (e + 1) * P.N < row_end ? (e + 1) * P.N : row_end;
+    const uintptr_t start = reinterpret_cast<uintptr_t>(P.avail) + e * P.avail_sb + (ra - e * P.N) * P.A;
+    const uintptr_t lo = start & ~(uintptr_t)15, hi = (start + (rb - ra) * P.A + 15) & ~(uintptr_t)15;
+    const int64_t e0 = (int64_t)((uint32_t)row0 / (uint32_t)P.N);
+    Av8Run run;
+    run.lo = reinterpret_cast<const uint8_t*>(lo);
+    run.dst = (uint32_t)((((ra - row0) * P.A) & ~(int64_t)15) + ro::AV8_SLACK * (e - e0));
+    run.bytes = (uint32_t)(hi - lo);
+    run.phase = (uint32_t)(start & 15);
+    return run;
+}
+
+// availability bits of cells c0 .. c0 + 15 of a row (generic pointer: staged in shared memory or in global memory);
+// cells >= A read as 0 and are not read.  vec (i32): the row is 16-byte aligned and A % 4 == 0.
+template <int AVB>
+__device__ __forceinline__ uint32_t avail_bits16(const uint8_t* row, int c0, int A, bool vec) {
+    uint32_t oks = 0u;
+    if (AVB == 4) {
+        const int32_t* av = reinterpret_cast<const int32_t*>(row);
+        int avj[16];
+        if (vec && c0 + 16 <= A) {
+#pragma unroll
+            for (int j4 = 0; j4 < 4; ++j4) {
+                const int4 w4 = *(reinterpret_cast<const int4*>(av + c0) + j4);
+                avj[4 * j4] = w4.x; avj[4 * j4 + 1] = w4.y; avj[4 * j4 + 2] = w4.z; avj[4 * j4 + 3] = w4.w;
+            }
+        } else {
+#pragma unroll
+            for (int j = 0; j < 16; ++j) avj[j] = c0 + j < A ? av[c0 + j] : 0;
+        }
+#pragma unroll
+        for (int j = 0; j < 16; ++j) oks |= (avj[j] != 0 ? 1u : 0u) << j;
+    } else {
+        const uint8_t* av = row + c0;
+        const uintptr_t al = reinterpret_cast<uintptr_t>(av);
+        uint32_t w[4] = {0u, 0u, 0u, 0u};
+        if (c0 + 16 <= A && (al & 15) == 0) {
+            const uint4 v = *reinterpret_cast<const uint4*>(av);
+            w[0] = v.x; w[1] = v.y; w[2] = v.z; w[3] = v.w;
+        } else {
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                const int c = c0 + 4 * k;
+                if (c + 4 <= A && (al & 3) == 0) w[k] = *reinterpret_cast<const uint32_t*>(av + 4 * k);
+                else {
+#pragma unroll
+                    for (int e = 0; e < 4; ++e)
+                        if (c + e < A) w[k] |= (uint32_t)av[4 * k + e] << (8 * e);
+                }
+            }
+        }
+#pragma unroll
+        for (int j = 0; j < 16; ++j) oks |= (((w[j >> 2] >> (8 * (j & 3))) & 0xffu) != 0u ? 1u : 0u) << j;
+    }
+    return oks;
+}
+
+template <int AVB>
 __global__ void __launch_bounds__(ro::THREADS, 1) gru_rollout_kernel(GruFwdParams P, int av_smem,
                                                                      const __grid_constant__ CUtensorMap tmap_h0,
                                                                      const __grid_constant__ CUtensorMap tmap_h1) {
@@ -267,14 +335,27 @@ __global__ void __launch_bounds__(ro::THREADS, 1) gru_rollout_kernel(GruFwdParam
                 const int64_t row0 = tile * TILE_ROWS;
                 const int rows_here = (int)(P.R - row0 < TILE_ROWS ? P.R - row0 : TILE_ROWS);
                 RWAIT(1, &av_free[s], (uint32_t)((u & 1) ^ 1));
-                if (lane == 0) mbar_arrive_expect_tx(&av_full[s], (uint32_t)(rows_here * P.A * 4));
-                __syncwarp();
                 const int64_t e0 = (int64_t)((uint32_t)row0 / (uint32_t)P.N);
-                for (int64_t e = e0 + lane; e * P.N < row0 + rows_here; e += 32) {
-                    const int64_t ra = e * P.N > row0 ? e * P.N : row0;                  // rows of env e inside the tile
-                    const int64_t rb = (e + 1) * P.N < row0 + rows_here ? (e + 1) * P.N : row0 + rows_here;
-                    bulk_copy_g2s(sl + S_AV + (ra - row0) * P.A * 4, P.avail + e * P.avail_sb + (ra - e * P.N) * P.A,
-                                  (uint32_t)((rb - ra) * P.A * 4), &av_full[s]);
+                if (AVB == 4) {
+                    if (lane == 0) mbar_arrive_expect_tx(&av_full[s], (uint32_t)(rows_here * P.A * 4));
+                    __syncwarp();
+                    const int32_t* avail = static_cast<const int32_t*>(P.avail);
+                    for (int64_t e = e0 + lane; e * P.N < row0 + rows_here; e += 32) {
+                        const int64_t ra = e * P.N > row0 ? e * P.N : row0;                  // rows of env e inside the tile
+                        const int64_t rb = (e + 1) * P.N < row0 + rows_here ? (e + 1) * P.N : row0 + rows_here;
+                        bulk_copy_g2s(sl + S_AV + (ra - row0) * P.A * 4, avail + e * P.avail_sb + (ra - e * P.N) * P.A,
+                                      (uint32_t)((rb - ra) * P.A * 4), &av_full[s]);
+                    }
+                } else {
+                    uint32_t bytes = 0;
+                    for (int64_t e = e0 + lane; e * P.N < row0 + rows_here; e += 32) bytes += av8_run(P, e, row0, row0 + rows_here).bytes;
+                    bytes = __reduce_add_sync(0xffffffffu, bytes);
+                    if (lane == 0) mbar_arrive_expect_tx(&av_full[s], bytes);
+                    __syncwarp();
+                    for (int64_t e = e0 + lane; e * P.N < row0 + rows_here; e += 32) {
+                        const Av8Run run = av8_run(P, e, row0, row0 + rows_here);
+                        bulk_copy_g2s(sl + S_AV + run.dst, run.lo, run.bytes, &av_full[s]);
+                    }
                 }
             }
         }
@@ -468,7 +549,7 @@ __global__ void __launch_bounds__(ro::THREADS, 1) gru_rollout_kernel(GruFwdParam
             const bool valid = row < P.R;
             const bool select = P.actions_out != nullptr && valid;
             float* qo = P.q ? P.q + row * P.A : nullptr;
-            const int32_t* av = nullptr;
+            const uint8_t* av = nullptr;
             bool av_vec = true;
             // first what the gate group will wait for next: the h_0 operand of the next tile (its inputs landed while this
             // group selected for the previous tile)
@@ -478,30 +559,22 @@ __global__ void __launch_bounds__(ro::THREADS, 1) gru_rollout_kernel(GruFwdParam
             uint32_t oks2[2] = {0u, 0u};                           // availability bits of the own chunks ch, ch + 2
             uint32_t rnd_x = 0u, rnd_y = 0u;
             if (select) {
-                if (av_smem) av = reinterpret_cast<const int32_t*>(sl + S_AV) + r * P.A;
-                else {
-                    const int64_t bb = (int64_t)((uint32_t)row / (uint32_t)P.N);
-                    av = P.avail + bb * P.avail_sb + (row - bb * P.N) * P.A;
+                const int64_t bb = (int64_t)((uint32_t)row / (uint32_t)P.N);
+                if (av_smem && AVB == 4) av = sl + S_AV + r * P.A * 4;
+                else if (av_smem) {
+                    const int64_t row0 = tile * TILE_ROWS;
+                    const Av8Run run = av8_run(P, bb, row0, row0 + TILE_ROWS);
+                    const int64_t ra = bb * P.N > row0 ? bb * P.N : row0;
+                    av = sl + S_AV + run.dst + run.phase + (row - ra) * P.A;
+                } else {
+                    av = static_cast<const uint8_t*>(P.avail) + (bb * P.avail_sb + (row - bb * P.N) * P.A) * AVB;
                     av_vec = (P.A & 3) == 0 && (P.avail_sb & 3) == 0 && (reinterpret_cast<uintptr_t>(P.avail) & 15) == 0;
                 }
 #pragma unroll
                 for (int i = 0; i < 2; ++i) {
                     const int c0 = 16 * (ch + 2 * i);
                     if (c0 < A_pad) {
-                        int avj[16];
-                        if (av_vec && c0 + 16 <= P.A) {
-#pragma unroll
-                            for (int j4 = 0; j4 < 4; ++j4) {
-                                const int4 w4 = *(reinterpret_cast<const int4*>(av + c0) + j4);
-                                avj[4 * j4] = w4.x; avj[4 * j4 + 1] = w4.y; avj[4 * j4 + 2] = w4.z; avj[4 * j4 + 3] = w4.w;
-                            }
-                        } else {
-#pragma unroll
-                            for (int j = 0; j < 16; ++j) avj[j] = c0 + j < P.A ? av[c0 + j] : 0;
-                        }
-                        uint32_t oks = 0u;
-#pragma unroll
-                        for (int j = 0; j < 16; ++j) oks |= (avj[j] != 0 ? 1u : 0u) << j;
+                        uint32_t oks = avail_bits16<AVB>(av, c0, P.A, av_vec);
                         const int left = P.A - c0;                                   // actions of this chunk that exist
                         oks &= left >= 16 ? 0xffffu : ((1u << (left > 0 ? left : 0)) - 1u);
                         oks2[i] = oks;
@@ -915,9 +988,13 @@ int tc_gru_fwd(const tc::GruFwdParams& P, cudaStream_t s) {
         set_error("tc_gru_fwd: hidden state must be 16-byte aligned");
         return PMB_ERR_INVALID;
     }
-    // avail rows are staged through shared memory by bulk copies when they fit and are 16-byte granular
-    const int av_smem = P.actions_out && P.avail && (P.A & 3) == 0 && 128 * P.A * 4 <= tc::ro::AV_BYTES && (P.avail_sb & 3) == 0 &&
-                        ((int64_t)P.N * P.A & 3) == 0 && (reinterpret_cast<uintptr_t>(P.avail) & 15) == 0;
+    // avail rows are staged through shared memory by bulk copies when they fit and (i32) are 16-byte granular; u8 rows
+    // are staged as the aligned superset of each env's run, which fits for every A <= 64
+    const int envs_per_tile = 127 / P.N + 2 < 128 ? 127 / P.N + 2 : 128;
+    const int av_smem = P.actions_out && P.avail &&
+                        (P.avail_u8 ? 128 * P.A + tc::ro::AV8_SLACK * envs_per_tile <= tc::ro::AV_BYTES
+                                    : (P.A & 3) == 0 && 128 * P.A * 4 <= tc::ro::AV_BYTES && (P.avail_sb & 3) == 0 &&
+                                          ((int64_t)P.N * P.A & 3) == 0 && (reinterpret_cast<uintptr_t>(P.avail) & 15) == 0);
     // tensor maps of the fp32 hidden state [R][64], in and out: boxes of 128 rows x 32 columns, 128-byte swizzle; loads
     // fill rows beyond R with zeros, stores clip them
     CUtensorMap tmap, tmap_out;
@@ -950,9 +1027,10 @@ int tc_gru_fwd(const tc::GruFwdParams& P, cudaStream_t s) {
             if (cr != CUDA_SUCCESS) { set_error("tc_gru_fwd: cuTensorMapEncodeTiled failed"); return PMB_ERR_CUDA; }
         }
     }
-    PMB_SMEM_ATTR(tc::gru_rollout_kernel, tc::ro::SMEM_BYTES);
+    const auto kern = P.avail_u8 ? tc::gru_rollout_kernel<1> : tc::gru_rollout_kernel<4>;
+    PMB_SMEM_ATTR(kern, tc::ro::SMEM_BYTES);
     const int grid = P.n_tiles < sm_count() ? P.n_tiles : sm_count();
-    PMB_CUDA(launch_pdl(tc::gru_rollout_kernel, dim3(grid), dim3(tc::ro::THREADS), tc::ro::SMEM_BYTES, s, rollout_pdl_enabled(), P, av_smem, tmap, tmap_out));
+    PMB_CUDA(launch_pdl(kern, dim3(grid), dim3(tc::ro::THREADS), tc::ro::SMEM_BYTES, s, rollout_pdl_enabled(), P, av_smem, tmap, tmap_out));
     PMB_LAUNCH_CHECK("gru_rollout_kernel");
     return PMB_OK;
 }

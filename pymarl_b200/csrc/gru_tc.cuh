@@ -23,8 +23,9 @@ struct GruFwdParams {
     int nt, A, n_tiles;
     // optional fused epsilon-greedy selection on the q of the LAST step (components/action_selectors.py:44-62; same
     // arithmetic and Philox indexing as epsilon_greedy_kernel in select.cu): actions_out == nullptr disables it
-    const int32_t* avail;            // already offset to the step: row (b, n) at avail + b*avail_sb + n*A
+    const void* avail;               // already offset to the step: row (b, n) at cell b*avail_sb + n*A of avail
     int64_t avail_sb;
+    int avail_u8;                    // cells are u8 (else i32)
     int N;
     float epsilon;
     const float* u;                  // injected draws [R] / [R][A], or null -> Philox(seed, offset)

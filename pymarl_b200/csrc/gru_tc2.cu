@@ -344,7 +344,7 @@ struct QSelectParams {
     const float *b2_on, *b2_tg;
     const uint8_t* h_on_ti;          // [(T+1)][n_tiles][16 KB]
     const uint8_t* h_tg_ti;
-    const int32_t* avail; int64_t avail_sb;
+    const void* avail; int64_t avail_sb;   // i32, or u8 (the kernel's AVB = 1)
     const int64_t* actions; int64_t actions_sb;
     const int64_t* ep_index;         // optional batch row -> buffer episode
     float* chosen;                   // [B][T-1][N]
@@ -360,6 +360,70 @@ struct QSelectParams {
     const int32_t* tile_steps;
 };
 
+// One row's avail, columns c of [0, 64) as 16 words of 4 cells each.  i32 cells (AVB = 4): avv[c] is the cell; u8 cells
+// (AVB = 1): byte c & 3 of word c >> 2.  The row's cells are loaded with the widest words its alignment allows, and no
+// byte past column A - 1 is read; columns >= A read as 0.
+template <int AVB> struct AvailRow;
+template <> struct AvailRow<4> {
+    int4 avv[16];
+    __device__ __forceinline__ void load(const void* row, bool want, int A, bool vec_ok) {
+        const int32_t* av = static_cast<const int32_t*>(row);
+        const int n_q4 = (A + 3) >> 2;
+#pragma unroll
+        for (int q = 0; q < 16; ++q) {
+            avv[q] = make_int4(0, 0, 0, 0);
+            if (want && q < n_q4) {
+                if (vec_ok) avv[q] = __ldg(reinterpret_cast<const int4*>(av) + q);
+                else {
+                    avv[q].x = __ldg(av + 4 * q);
+                    if (4 * q + 1 < A) avv[q].y = __ldg(av + 4 * q + 1);
+                    if (4 * q + 2 < A) avv[q].z = __ldg(av + 4 * q + 2);
+                    if (4 * q + 3 < A) avv[q].w = __ldg(av + 4 * q + 3);
+                }
+            }
+        }
+    }
+    __device__ __forceinline__ bool ok(int a) const {
+        const int4 w = avv[a >> 2];
+        return ((a & 3) == 0 ? w.x : ((a & 3) == 1 ? w.y : ((a & 3) == 2 ? w.z : w.w))) != 0;
+    }
+};
+template <> struct AvailRow<1> {
+    uint32_t w[16];
+    __device__ __forceinline__ void load(const void* row, bool want, int A, bool) {
+        const uint8_t* av = static_cast<const uint8_t*>(row);
+        const uintptr_t al = reinterpret_cast<uintptr_t>(av);
+#pragma unroll
+        for (int q = 0; q < 16; ++q) w[q] = 0u;
+        if (!want) return;
+#pragma unroll
+        for (int g = 0; g < 4; ++g) {                      // 16-byte groups of columns
+            const int c0 = 16 * g;
+            if (c0 >= A) break;
+            if (c0 + 16 <= A && (al & 15) == 0) {
+                const uint4 v = __ldg(reinterpret_cast<const uint4*>(av + c0));
+                w[4 * g] = v.x; w[4 * g + 1] = v.y; w[4 * g + 2] = v.z; w[4 * g + 3] = v.w;
+            } else if (c0 + 16 <= A && (al & 7) == 0) {
+                const uint2 v0 = __ldg(reinterpret_cast<const uint2*>(av + c0)), v1 = __ldg(reinterpret_cast<const uint2*>(av + c0 + 8));
+                w[4 * g] = v0.x; w[4 * g + 1] = v0.y; w[4 * g + 2] = v1.x; w[4 * g + 3] = v1.y;
+            } else {
+#pragma unroll
+                for (int k = 0; k < 4; ++k) {
+                    const int c = c0 + 4 * k;
+                    if (c + 4 <= A && (al & 3) == 0) w[4 * g + k] = __ldg(reinterpret_cast<const uint32_t*>(av + c));
+                    else {
+#pragma unroll
+                        for (int e = 0; e < 4; ++e)
+                            if (c + e < A) w[4 * g + k] |= (uint32_t)__ldg(av + c + e) << (8 * e);
+                    }
+                }
+            }
+        }
+    }
+    __device__ __forceinline__ bool ok(int a) const { return ((w[a >> 2] >> (8 * (a & 3))) & 0xffu) != 0u; }
+};
+
+template <int AVB>
 __global__ void __launch_bounds__(qs::THREADS, 2) q_select_kernel(QSelectParams P) {
     using namespace qs;
     extern __shared__ uint8_t smem_raw[];
@@ -440,7 +504,6 @@ __global__ void __launch_bounds__(qs::THREADS, 2) q_select_kernel(QSelectParams 
         const uint32_t tl = tmem_base + ((uint32_t)(warp * 32) << 16);
         const bool vec_ok = (P.A & 3) == 0 && (P.avail_sb & 3) == 0 && (reinterpret_cast<uintptr_t>(P.avail) & 15) == 0;
         const uint32_t bias_s = smem_u32(bias);
-        const int n_q4 = (P.A + 3) >> 2;
         uint32_t it = 0;
         for (int64_t k = blockIdx.x; k < n_items; k += gridDim.x, ++it) {
             const int64_t item = P.items ? (int64_t)__ldg(P.items + k) : k;
@@ -455,23 +518,11 @@ __global__ void __launch_bounds__(qs::THREADS, 2) q_select_kernel(QSelectParams 
             int a_taken = -1;
             const int64_t be = ep_row(P.ep_index, b);
             if (valid && t < P.T - 1) a_taken = (int)__ldg(P.actions + be * P.actions_sb + (int64_t)t * P.N + n);
-            const int32_t* av = P.avail + be * P.avail_sb + ((int64_t)t * P.N + n) * P.A;
+            const void* av = static_cast<const uint8_t*>(P.avail) + (be * P.avail_sb + ((int64_t)t * P.N + n) * P.A) * AVB;
             const bool want_t = valid && t >= 1;
             // the whole avail row goes to registers (16-byte loads when the layout allows); columns >= A read as 0
-            int4 avv[16];
-#pragma unroll
-            for (int q = 0; q < 16; ++q) {
-                avv[q] = make_int4(0, 0, 0, 0);
-                if (want_t && q < n_q4) {
-                    if (vec_ok) avv[q] = __ldg(reinterpret_cast<const int4*>(av) + q);
-                    else {
-                        avv[q].x = __ldg(av + 4 * q);
-                        if (4 * q + 1 < P.A) avv[q].y = __ldg(av + 4 * q + 1);
-                        if (4 * q + 2 < P.A) avv[q].z = __ldg(av + 4 * q + 2);
-                        if (4 * q + 3 < P.A) avv[q].w = __ldg(av + 4 * q + 3);
-                    }
-                }
-            }
+            AvailRow<AVB> avr;
+            avr.load(av, want_t, P.A, vec_ok);
             mbar_wait(&tfull[b2], (it >> 1) & 1);
             tc_fence_after();
             // padding columns (a >= A) have zero weights, zero bias and avail = 0: they are masked like unavailable
@@ -498,9 +549,7 @@ __global__ void __launch_bounds__(qs::THREADS, 2) q_select_kernel(QSelectParams 
                         const float q_on = __uint_as_float(von[j]) + bo[j];
                         const float q_tg = __uint_as_float(vtg[j]) + bt[j];
                         chosen = a == a_taken ? q_on : chosen;
-                        const int4 w = avv[4 * cc + (j >> 2)];
-                        const int avj = (j & 3) == 0 ? w.x : ((j & 3) == 1 ? w.y : ((j & 3) == 2 ? w.z : w.w));
-                        const bool ok = avj != 0;
+                        const bool ok = avr.ok(a);
                         const float mt = ok ? q_tg : kMaskValue;
                         const float v = P.double_q ? (ok ? q_on : kMaskValue) : mt;
                         if (a == 0) mt0 = mt;
@@ -994,8 +1043,13 @@ int tc_q_select(const pmb_dims* d, const pmb_batch* b, const __nv_bfloat16* w2_o
     const int64_t n_items = (int64_t)d->T * n_tiles;
     int grid = 2 * sm_count();
     if (grid > n_items) grid = (int)n_items;
-    PMB_SMEM_ATTR(tc::q_select_kernel, tc::qs::SMEM_BYTES);
-    tc::q_select_kernel<<<grid, tc::qs::THREADS, tc::qs::SMEM_BYTES, s>>>(P);
+    if (b->avail_dtype == PMB_DTYPE_U8) {
+        PMB_SMEM_ATTR(tc::q_select_kernel<1>, tc::qs::SMEM_BYTES);
+        tc::q_select_kernel<1><<<grid, tc::qs::THREADS, tc::qs::SMEM_BYTES, s>>>(P);
+    } else {
+        PMB_SMEM_ATTR(tc::q_select_kernel<4>, tc::qs::SMEM_BYTES);
+        tc::q_select_kernel<4><<<grid, tc::qs::THREADS, tc::qs::SMEM_BYTES, s>>>(P);
+    }
     PMB_LAUNCH_CHECK("q_select_kernel");
     return PMB_OK;
 }

@@ -148,7 +148,7 @@ int launch_mixer_fwd(const pmb_dims* d, const pmb_batch* b, const float* flat_mi
     MixerParams mp = mixer_params(d, flat_mixer);
     const int C = (d->N + 3) * d->E;
     RowMap smap{b->state_sb, (int64_t)d->S, 0, d->T - 1, 1};
-    int rc = launch_gemm_tn(b->state + (int64_t)t_off * d->S, smap, M, d->S, mp.w_cat, d->S, C, mp.b_cat, raw, C, 0, s);
+    int rc = launch_gemm_tn(static_cast<const float*>(b->state) + (int64_t)t_off * d->S, smap, M, d->S, mp.w_cat, d->S, C, mp.b_cat, raw, C, 0, s);
     if (rc) return rc;
     qmix_mix_fwd_kernel<<<(unsigned)ceil_div(M * 32, 256), 256, 0, s>>>(M, d->N, d->E, raw, agent_qs, mp.v2_w, mp.v2_b,
                                                                        q_tot);
@@ -193,7 +193,7 @@ int launch_mixer_bwd(const pmb_dims* d, const pmb_batch* b, const float* flat_mi
     PMB_LAUNCH_CHECK("v2_reduce_kernel");
     // hypernet weights and biases:  dW_cat = d_raw^T . state[:, :-1],  db_cat = column sums
     RowMap smap{b->state_sb, (int64_t)d->S, 0, d->T - 1, 1};
-    return gemm_atb_any(d->precision, raw, dense_map(C), C, b->state, smap, d->S, M, gbase + L.offset[PMB_P_HW1_W],
+    return gemm_atb_any(d->precision, raw, dense_map(C), C, static_cast<const float*>(b->state), smap, d->S, M, gbase + L.offset[PMB_P_HW1_W],
                         d->S, gbase + L.offset[PMB_P_HW1_B], atb_scratch, atb_bytes, s);
 }
 

@@ -160,7 +160,7 @@ int launch_target_select(const pmb_dims* d, const pmb_batch* b, const float* q_o
     int64_t n_rows = (int64_t)d->B * (d->T - 1) * d->N;
     if (n_rows <= 0) return PMB_OK;
     unsigned grid = (unsigned)ceil_div(n_rows * GL, 256);
-    target_select_kernel<<<grid, 256, 0, s>>>(d->B, d->T, d->N, d->A, d->double_q, q_on, q_tg, b->avail, b->avail_sb,
+    target_select_kernel<<<grid, 256, 0, s>>>(d->B, d->T, d->N, d->A, d->double_q, q_on, q_tg, static_cast<const int32_t*>(b->avail), b->avail_sb,
                                               b->actions, b->actions_sb, chosen, tmax, cur_max);
     PMB_LAUNCH_CHECK("target_select_kernel");
     return PMB_OK;

@@ -1562,12 +1562,15 @@ int64_t tc_mixer_scratch_bytes(const pmb_dims* d) {
 }
 
 // ---- image-fed mixer path -------------------------------------------------------------------------
-// state [B, T, S] fp32 -> bf16 tile images [ceil(B*T/128)][ceil((S+1)/64)][16 KB] over ALL (b, t) rows, m' = b*T + t.
-// Column S of every real row holds 1.0 (the bias-gradient column of the hypernet weight-gradient GEMM; the packed
-// forward weights are zero there), everything else beyond S and all padding rows are zero.
+// state [B, T, S] fp32 or bf16 (ES = element size) -> bf16 tile images [ceil(B*T/128)][ceil((S+1)/64)][16 KB] over ALL
+// (b, t) rows, m' = b*T + t.  Column S of every real row holds 1.0 (the bias-gradient column of the hypernet
+// weight-gradient GEMM; the packed forward weights are zero there), everything else beyond S and all padding rows are
+// zero.  fp32 state is rounded to bf16 here, so bf16 storage of the same rounded values gives the same images.
+template <int ES>
 __global__ void __launch_bounds__(256)
-state_to_images_kernel(const float* __restrict__ state, int64_t state_sb, const int64_t* __restrict__ ep_index, int64_t BT,
+state_to_images_kernel(const uint8_t* __restrict__ state, int64_t state_sb, const int64_t* __restrict__ ep_index, int64_t BT,
                        int T, int S, int n_chunks, uint8_t* __restrict__ img) {
+    static_assert(ES == 4 || ES == 2, "fp32 or bf16 state");
     // one thread per 16-byte chunk
     const int64_t total = ((BT + 127) / 128) * 128 * (int64_t)n_chunks * 8;
     int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -1583,19 +1586,35 @@ state_to_images_kernel(const float* __restrict__ state, int64_t state_sb, const 
     if (m < BT) {
         const int64_t b = m / T;
         const int t = (int)(m - b * T);
-        const float* src = state + ep_row(ep_index, b) * state_sb + (int64_t)t * S + c * 64 + j * 8;
+        const uint8_t* src = state + (ep_row(ep_index, b) * state_sb + (int64_t)t * S + c * 64 + j * 8) * ES;
         const int nv = S - (c * 64 + j * 8);
-        if (nv >= 8 && (reinterpret_cast<uintptr_t>(src) & 7) == 0) {        // the common case: four 8-byte loads
+        const uintptr_t al = reinterpret_cast<uintptr_t>(src);
+        if (ES == 4 && nv >= 8 && (al & 7) == 0) {                          // the common fp32 case: four 8-byte loads
 #pragma unroll
             for (int e = 0; e < 4; ++e) {
                 const float2 v = __ldg(reinterpret_cast<const float2*>(src) + e);
                 f[2 * e] = v.x; f[2 * e + 1] = v.y;
             }
+        } else if (ES == 2 && nv >= 8 && (al & 15) == 0) {                   // bf16: the whole chunk in one 16-byte load
+            const uint4 v = __ldg(reinterpret_cast<const uint4*>(src));
+            const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+            for (int e = 0; e < 4; ++e) { f[2 * e] = __uint_as_float(w[e] << 16); f[2 * e + 1] = __uint_as_float(w[e] & 0xffff0000u); }
+        } else if (ES == 2 && nv >= 8 && (al & 3) == 0) {                    // rows of 2 * S bytes, S even (27m: 2340)
+#pragma unroll
+            for (int e = 0; e < 4; ++e) {
+                const uint32_t w = __ldg(reinterpret_cast<const uint32_t*>(src) + e);
+                f[2 * e] = __uint_as_float(w << 16); f[2 * e + 1] = __uint_as_float(w & 0xffff0000u);
+            }
         } else {
 #pragma unroll
             for (int e = 0; e < 8; ++e) {
-                if (e < nv) f[e] = __ldg(src + e);
-                else if (e == nv) f[e] = 1.0f;
+                if (e < nv) {
+                    if (ES == 4) f[e] = __ldg(reinterpret_cast<const float*>(src) + e);
+                    else f[e] = __uint_as_float((uint32_t)__ldg(reinterpret_cast<const unsigned short*>(src) + e) << 16);
+                } else if (e == nv) {
+                    f[e] = 1.0f;
+                }
             }
         }
     }
@@ -1608,8 +1627,13 @@ int tc_state_to_images(const pmb_dims* d, const pmb_batch* b, uint8_t* img, cuda
     const int64_t BT = (int64_t)d->B * d->T;
     const int n_chunks = tc_state_chunks(d);
     const int64_t total = ((BT + 127) / 128) * 128 * (int64_t)n_chunks * 8;
-    state_to_images_kernel<<<(unsigned)ceil_div(total, 256), 256, 0, s>>>(b->state, b->state_sb, b->ep_index, BT, d->T, d->S, n_chunks,
-                                                                                  img);
+    const uint8_t* state = static_cast<const uint8_t*>(b->state);
+    if (b->state_dtype == PMB_DTYPE_BF16)
+        state_to_images_kernel<2><<<(unsigned)ceil_div(total, 256), 256, 0, s>>>(state, b->state_sb, b->ep_index, BT, d->T,
+                                                                                 d->S, n_chunks, img);
+    else
+        state_to_images_kernel<4><<<(unsigned)ceil_div(total, 256), 256, 0, s>>>(state, b->state_sb, b->ep_index, BT, d->T,
+                                                                                 d->S, n_chunks, img);
     PMB_LAUNCH_CHECK("state_to_images_kernel");
     return PMB_OK;
 }

@@ -462,7 +462,7 @@ class QLearner:
     # same stream.
     def _run_graphed(self, dims, pb, hp, f, need, dev, keep):
         key = (tuple(getattr(dims, k) for k, _ in dims._fields_), tuple(getattr(pb, k) for k, _ in pb._fields_),
-               tuple(getattr(hp, k) for k, _ in hp._fields_), f["p"].data_ptr(), self._workspace.data_ptr(),
+               pb.state_dtype, pb.avail_dtype, tuple(getattr(hp, k) for k, _ in hp._fields_), f["p"].data_ptr(), self._workspace.data_ptr(),
                self._stats.data_ptr())
         entry = self._graphs.get(key)
         if entry is None:
