@@ -177,9 +177,9 @@ def _train_twice(shape, mixer, batch, **over):
     return _state(lr)
 
 
-def _forward_workspace(shape, mixer, batch):
+def _forward_workspace(shape, mixer, batch, **over):
     """keep_q = 3: forward + loss sums only, every intermediate (obs / x images, ReLU mask, q) left in the workspace."""
-    lr = _learner(shape, mixer, keep_q=3)
+    lr = _learner(shape, mixer, keep_q=3, **over)
     lr.train(batch, 0, 0)
     lr._workspace.zero_()
     lr.train(batch, 0, 0)
@@ -190,19 +190,21 @@ def _forward_workspace(shape, mixer, batch):
 CASES = [("27m_vs_30m", "qmix", 256, 12), ("27m_vs_30m", "qmix", 100, 12),
          ("3m", "vdn", 40, 30), ("3m", None, 40, 30), ("2s3z", "vdn", 60, 20), ("2s3z", None, 60, 20),
          ("MMM2", "vdn", 50, 16), ("MMM2", None, 50, 16)]
+NO_INPUTS = dict(obs_last_action=False, obs_agent_id=False)     # pack and stream kernels without the act and id blocks
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("ts", [1, 0])
-@pytest.mark.parametrize("name,mixer,B,T", CASES)
-def test_train_step_bit_identical(name, mixer, B, T, ts):
+@pytest.mark.parametrize("name,mixer,B,T,over", [c + ({},) for c in CASES] + [("2s3z", "qmix", 60, 20, NO_INPUTS)],
+                         ids=["-".join(map(str, c)) for c in CASES] + ["2s3z-qmix-60-20-no_inputs"])
+def test_train_step_bit_identical(name, mixer, B, T, over, ts):
     shape = SMAC_SHAPES[name]
     b32, b16 = _pair(shape, B, T)
-    a = _with_ts(ts, lambda: _train_twice(shape, mixer, b32))
-    b = _with_ts(ts, lambda: _train_twice(shape, mixer, b16))
+    a = _with_ts(ts, lambda: _train_twice(shape, mixer, b32, **over))
+    b = _with_ts(ts, lambda: _train_twice(shape, mixer, b16, **over))
     _assert_equal(a, b)
-    w32 = _with_ts(ts, lambda: _forward_workspace(shape, mixer, b32))
-    w16 = _with_ts(ts, lambda: _forward_workspace(shape, mixer, b16))
+    w32 = _with_ts(ts, lambda: _forward_workspace(shape, mixer, b32, **over))
+    w16 = _with_ts(ts, lambda: _forward_workspace(shape, mixer, b16, **over))
     assert th.equal(w32, w16)
 
 

@@ -198,14 +198,18 @@ def test_same_order_with_and_without_skipping(shape, mixer, B, T):
 # ---- 4. against today's unsorted step ---------------------------------------------------------------------------------
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("shape,mixer,B,T", [("27m_vs_30m", "qmix", 256, 100), ("MMM2", "vdn", 128, 80)])
-def test_against_unsorted_step(shape, mixer, B, T):
+@pytest.mark.parametrize("shape,mixer,B,T,over", [
+    ("27m_vs_30m", "qmix", 256, 100, {}), ("MMM2", "vdn", 128, 80, {}),
+    # the live-item walk and the zero fill of the skipped items in the q-select epilogue with the flags off
+    ("MMM2", "qmix", 128, 80, dict(double_q=False, obs_last_action=False))],
+    ids=["27m_vs_30m-qmix-256-100", "MMM2-vdn-128-80", "MMM2-qmix-128-80-no_double_q-no_last_action"])
+def test_against_unsorted_step(shape, mixer, B, T, over):
     from cuda_utils import to_batch
     shape = SMAC_SHAPES[shape]
     batch = to_batch(shape, _fields(shape, B, T, seed=21))
     st = []
     for skip in (False, True):
-        learner = _learner(shape, mixer, skip=skip)
+        learner = _learner(shape, mixer, skip=skip, **over)
         learner.train(batch, 0, 0)
         st.append((learner, _state(learner)))
     (l0, a), (l1, b) = st
