@@ -131,8 +131,8 @@ class OracleCOMALearner:
         self.n_target_updates = 0
 
     def _train_critic(self, batch, rewards, terminated, actions, mask):
-        """coma_learner.py:103-148.  Returns q_vals [B, T-1, N, A] (each timestep with the critic of that moment) and
-        the per-step logs."""
+        """coma_learner.py:103-148.  Returns q_vals [B, T-1, N, A] (each timestep with the critic of that moment), the
+        per-step logs (log["t"]: the timestep of each entry), the td-lambda targets and the target critic's Q [B, T, N, A]."""
         a = self.args
         B, T, N = batch["obs"].shape[:3]
         dt = self.critic["fc1.weight"].dtype
@@ -141,7 +141,7 @@ class OracleCOMALearner:
         targets = td_lambda_targets(rewards, terminated, mask, targets_taken, a.gamma, a.td_lambda)
         A = tq.shape[-1]
         q_vals = np.zeros((B, T - 1, N, A), dtype=dt)
-        log = {k: [] for k in ("critic_loss", "critic_grad_norm", "td_error_abs", "target_mean", "q_taken_mean")}
+        log = {k: [] for k in ("t", "critic_loss", "critic_grad_norm", "td_error_abs", "target_mean", "q_taken_mean")}
         for t in reversed(range(T - 1)):
             mask_t = np.broadcast_to(mask[:, t], (B, N))
             if mask_t.sum() == 0:
@@ -161,11 +161,12 @@ class OracleCOMALearner:
             orc.rmsprop_step(self.critic, grads, self.sq_critic, CRITIC_PARAM_NAMES, a.critic_lr, a.optim_alpha, a.optim_eps)
             self.critic_training_steps += 1
             me = float(msum)
+            log["t"].append(t)
             log["critic_loss"].append(float(loss)); log["critic_grad_norm"].append(float(gn))
             log["td_error_abs"].append(float(np.abs(mtd).sum()) / me)
             log["q_taken_mean"].append(float((q_taken * mask_t).sum()) / me)
             log["target_mean"].append(float((targets[:, t] * mask_t).sum()) / me)
-        return q_vals, log, targets
+        return q_vals, log, targets, tq
 
     def train(self, batch, t_env, episode_num, epsilon):
         """coma_learner.py:32-101.  `epsilon` = mac.action_selector.epsilon at the time of the call (the epsilon floor of
@@ -179,7 +180,7 @@ class OracleCOMALearner:
         mask = batch["filled"][:, :-1].astype(dt)
         mask[:, 1:] = mask[:, 1:] * (1 - terminated[:, :-1])
         avail = batch["avail_actions"][:, :-1]
-        q_vals, clog, targets = self._train_critic(batch, rewards, terminated, actions, mask)
+        q_vals, clog, targets, tq = self._train_critic(batch, rewards, terminated, actions, mask)
         actions = actions[:, :-1]
         A = q_vals.shape[-1]
         # agent unroll over t = 0 .. T-2 (coma_learner.py:55-60)
@@ -232,12 +233,12 @@ class OracleCOMALearner:
             self.last_target_update_step = self.critic_training_steps
             self.n_target_updates += 1
         n_log = max(1, len(clog["critic_loss"]))
-        stats = {k: sum(v) / n_log for k, v in clog.items()}
+        stats = {k: sum(v) / n_log for k, v in clog.items() if k != "t"}
         me = float(msum)
         stats.update(advantage_mean=float((adv * m).sum()) / me, coma_loss=float(coma_loss), agent_grad_norm=float(gn),
                      pi_max=float((pi.max(axis=1) * m).sum()) / me)
         return stats, raw, dict(q_vals=q_vals, pi=pi.reshape(B, T - 1, N, A), targets=targets, advantages=adv.reshape(B, T - 1, N),
-                                logits=logits)
+                                logits=logits, target_q=tq, critic_log=clog)
 
 
 def agent_bptt_dense(p, cache, dq_full, B, N):
