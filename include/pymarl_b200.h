@@ -54,7 +54,7 @@ typedef struct pmb_dims {
     int32_t O;                 /* obs dim                                                 */
     int32_t S;                 /* state dim                                               */
     int32_t A;                 /* n_actions                                               */
-    int32_t H;                 /* rnn_hidden_dim  (16, 32 or 64)                          */
+    int32_t H;                 /* rnn_hidden_dim  (16, 32, 64 or 128)                     */
     int32_t E;                 /* mixing_embed_dim (8, 16, 32 or 64)                      */
     int32_t obs_last_action;   /* controllers/basic_controller.py:111                     */
     int32_t obs_agent_id;      /* controllers/basic_controller.py:118                     */
@@ -191,7 +191,9 @@ int pmb_agent_fc1_dense_fwd(const pmb_dims* d, int64_t rows, int32_t d_in, const
 /* GRUCell + fc2 unrolled over nt steps for R = rows (rnn_agent.py:33-36, the t loops of
  * q_learner.py:47-52,58-62).  h0 NULL = zeros (basic_controller.py:77-81).
  * h_stash [(nt+1)][R][H] (slot 0 = h0) and gates [nt][R][4H] (r,z,n,W_hn h+b_hn) are
- * written when non-NULL (needed by the backward); q [nt][R][A]; h_last [R][H] optional. */
+ * written when non-NULL (needed by the backward); q [nt][R][A]; h_last [R][H] optional.
+ * H = 128: gates is required (it first receives the input gates x W_ih^T + b_ih), and so is
+ * h_stash unless nt == 1 and h_last is given (q is computed from the stashed hidden states). */
 int pmb_agent_gru_unroll_fwd(const pmb_dims* d, int64_t rows, int32_t nt, const float* flat_agent,
                              const float* x, const float* h0, float* h_stash, float* gates,
                              float* q, float* h_last, pmb_stream stream);

@@ -516,6 +516,13 @@ int scatter_ctas(int64_t items) {
 
 }  // namespace
 
+// gru_h128.cu: rnn_hidden_dim 128 (W_ih and W_hh do not both fit in shared memory there)
+int h128_fwd(const pmb_dims* d, int prec, const AgentParams& p, int64_t R, int nt, const float* x, const float* h0,
+             float* h_seq, float* gates, int64_t ldg, int keep_gates, float* q, float* h_last, void* scratch,
+             int64_t scratch_bytes, cudaStream_t s);
+int h128_bwd(const pmb_dims* d, const pmb_batch* b, const AgentParams& p, const float* h_stash, float* gates,
+             const float* d_chosen, cudaStream_t s, const float* dq_full);
+
 int gru_fwd_dispatch(const pmb_dims* d, const AgentParams& p, int64_t R, int nt, const float* x, const float* h0,
                      float* h_stash, float* gates, float* q, float* h_last, cudaStream_t s) {
     int rw = pick_rw(R);
@@ -526,9 +533,12 @@ int gru_fwd_dispatch(const pmb_dims* d, const AgentParams& p, int64_t R, int nt,
         case 16: PMB_FWD(16);
         case 32: PMB_FWD(32);
         case 64: PMB_FWD(64);
+        // input gates in `gates`, q from `h_stash`: both buffers are required (CUDA-core GEMMs on every tier, as the
+        // unroll kernels above are fp32 on every tier)
+        case 128: return h128_fwd(d, PMB_PREC_FP32, p, R, nt, x, h0, h_stash, gates, 4 * d->H, 1, q, h_last, nullptr, 0, s);
     }
 #undef PMB_FWD
-    set_error("rnn_hidden_dim %d unsupported (16, 32, 64)", d->H);
+    set_error("rnn_hidden_dim %d unsupported (16, 32, 64, 128)", d->H);
     return PMB_ERR_INVALID;
 }
 
@@ -546,9 +556,10 @@ int gru_bwd_dispatch(const pmb_dims* d, const pmb_batch* b, const AgentParams& p
         case 16: PMB_BWD(16);
         case 32: PMB_BWD(32);
         case 64: PMB_BWD(64);
+        case 128: return h128_bwd(d, b, p, h_stash, gates, d_chosen, s, dq_full);     // dpre1: agent_bwd, after it
     }
 #undef PMB_BWD
-    set_error("rnn_hidden_dim %d unsupported (16, 32, 64)", d->H);
+    set_error("rnn_hidden_dim %d unsupported (16, 32, 64, 128)", d->H);
     return PMB_ERR_INVALID;
 }
 
@@ -584,7 +595,8 @@ int scatter_grads_dispatch(const pmb_dims* d, const pmb_batch* b, const float* h
         case 16: PMB_SC(16);
         case 32: PMB_SC(32);
         case 64: PMB_SC(64);
-        default: set_error("rnn_hidden_dim %d unsupported", d->H); return PMB_ERR_INVALID;
+        case 128: PMB_SC(128);
+        default: set_error("rnn_hidden_dim %d unsupported (16, 32, 64, 128)", d->H); return PMB_ERR_INVALID;
     }
 #undef PMB_SC
     PMB_LAUNCH_CHECK("agent_scatter_grads_kernel");

@@ -72,6 +72,14 @@ int tc_gemm_atb_ti(const uint8_t* d_ti, int T, int N, int64_t R, int n_tiles, co
 int64_t tc_atb_ti_scratch_bytes(int T, int n_tiles, int K);
 int64_t tc_fc1_scratch_bytes(const pmb_dims* d);
 bool tc_fc1_streams(const pmb_dims* d, int obs_dtype);
+// gru_h128.cu (rnn_hidden_dim 128)
+int64_t h128_fwd_scratch_bytes(const pmb_dims* d, int prec);
+int64_t h128_dpre1_scratch_bytes(int prec);
+int h128_fwd(const pmb_dims* d, int prec, const AgentParams& p, int64_t R, int nt, const float* x, const float* h0,
+             float* h_seq, float* gates, int64_t ldg, int keep_gates, float* q, float* h_last, void* scratch,
+             int64_t scratch_bytes, cudaStream_t s);
+int h128_dpre1(int prec, const AgentParams& p, int64_t rows, const float* gates, const float* x, float* dpre1,
+               void* scratch, int64_t scratch_bytes, cudaStream_t s);
 
 static thread_local char g_err[512] = "";
 std::atomic<long long> g_launch_count{0};
@@ -91,7 +99,7 @@ struct PhaseTimer {
 };
 static thread_local PhaseTimer g_timer;
 
-static void phase_mark(cudaStream_t s, const char* name) {
+void phase_mark(cudaStream_t s, const char* name) {
     PhaseTimer& t = g_timer;
     if (!t.armed) return;
     if (t.n > kMaxPhases) return;
@@ -176,7 +184,8 @@ static int side_stream(SideStream** out) {
 int validate_dims(const pmb_dims* d) {
     PMB_REQUIRE(d != nullptr, "dims is NULL");
     PMB_REQUIRE(d->B > 0 && d->T > 0 && d->N > 0 && d->O > 0 && d->A > 0, "B, T, N, O, A must be positive");
-    PMB_REQUIRE(d->H == 16 || d->H == 32 || d->H == 64, "rnn_hidden_dim %d unsupported (16, 32, 64)", d->H);
+    PMB_REQUIRE(d->H == 16 || d->H == 32 || d->H == 64 || d->H == 128, "rnn_hidden_dim %d unsupported (16, 32, 64, 128)",
+                d->H);
     PMB_REQUIRE(d->mixer >= PMB_MIXER_NONE && d->mixer <= PMB_MIXER_QMIX, "unknown mixer id %d", d->mixer);
     if (d->mixer == PMB_MIXER_QMIX) {
         PMB_REQUIRE(d->S > 0, "QMIX needs a positive state dim");
@@ -282,6 +291,7 @@ int64_t agent_bwd_scratch(const pmb_dims* d) {
     int64_t b = atb_scratch_bytes(d->precision, d->H, d->O, rows);
     int64_t c = scatter_scratch_bytes(d);
     int64_t m = a > b ? a : b;
+    if (d->H == 128 && h128_dpre1_scratch_bytes(d->precision) > m) m = h128_dpre1_scratch_bytes(d->precision);
     return m > c ? m : c;
 }
 
@@ -326,6 +336,7 @@ WsPlan plan_workspace(const pmb_dims* d) {
         off += align_up(sizes[i] * 4, 256);
     }
     int64_t sc = agent_bwd_scratch(d);
+    if (d->H == 128 && h128_fwd_scratch_bytes(d, d->precision) > sc) sc = h128_fwd_scratch_bytes(d, d->precision);
     int64_t mb = mixer_bwd_scratch_bytes(d);
     if (mb > sc) sc = mb;
     if (d->precision == PMB_PREC_BF16) {
@@ -402,9 +413,13 @@ int agent_bwd(const pmb_dims* d, const pmb_batch* b, const float* flat_agent, co
     PHASE(s, "gru_unroll_bwd");
     int rc = gru_bwd_dispatch(d, b, ap, x_on, h_stash, gates, d_chosen, dpre1, s, dq_full);
     if (rc) return rc;
+    const int prec = d->precision;
+    if (H == 128) {
+        PHASE(s, "h128_dpre1_gemm");
+        if ((rc = h128_dpre1(prec, ap, rows, gates, x_on, dpre1, scratch, scratch_bytes, s))) return rc;
+    }
     PHASE(s, "dW_rnn_gemm_atb");
     // rnn.weight_ih / bias_ih:  [da_r | da_z | da_n]^T . x
-    const int prec = d->precision;
     rc = gemm_atb_any(prec, gates, dense_map(4 * H), 3 * H, x_on, dense_map(H), H, rows, gr.w_ih, H, gr.b_ih, scratch,
                       scratch_bytes, s);
     if (rc) return rc;
@@ -669,6 +684,8 @@ int64_t pmb_select_actions_workspace_bytes(const pmb_dims* d) {
     int64_t n = align_up(R * d->H * 4, 256) + align_up(R * d->A * 4, 256);
     if (rollout_tc_ok(d))          // x tile images | GRU weight images | fc1 scratch
         n += align_up(ceil_div(R, 128) * 16384, 256) + 65536 + align_up(tc_fc1_scratch_bytes(d), 256);
+    if (d->H == 128)               // input gates [R][3H] | packed GEMM weights (bf16 tier)
+        n += align_up(R * 3 * d->H * 4, 256) + h128_fwd_scratch_bytes(d, d->precision);
     return n;
 }
 
@@ -718,6 +735,12 @@ int pmb_select_actions_step(const pmb_dims* d, const pmb_batch* b, int32_t t, co
         if (actions_out && !q_out) fp.q = nullptr;
         if ((rc = tc_gru_fwd(fp, s))) return rc;
         return PMB_OK;
+    } else if (d->H == 128) {
+        char* gi = static_cast<char*>(scratch) + align_up(R * d->H * 4, 256) + align_up(R * d->A * 4, 256);
+        char* gemm_scr = gi + align_up(R * 3 * d->H * 4, 256);
+        if ((rc = fc1_fwd(d, b, t, 1, ap, x, s))) return rc;
+        if ((rc = h128_fwd(d, d->precision, ap, R, 1, x, hidden, nullptr, reinterpret_cast<float*>(gi), 3 * d->H, 0, q, hidden,
+                           gemm_scr, h128_fwd_scratch_bytes(d, d->precision), s))) return rc;
     } else {
         rc = fc1_fwd(d, b, t, 1, ap, x, s);
         if (rc) return rc;
@@ -857,7 +880,14 @@ int pmb_qlearner_train_step(const pmb_dims* d, const pmb_batch* b, const pmb_hpa
         PHASE(s, "fc1_fwd_target");
         if ((rc = fc1_fwd(d, b, 0, d->T, tg, v.x_tg, s))) return rc;
     }
-    if (!tc_agent) {
+    if (!tc_agent && d->H == 128) {
+        // Target net first: its input gates and hidden states pass through `gates` and `h_stash`, which the online net
+        // then overwrites with what its backward needs - one set of buffers serves both nets.
+        if ((rc = h128_fwd(d, d->precision, tg, R, d->T, v.x_tg, nullptr, v.h_stash, v.gates, 4 * d->H, 0, v.q_tg, nullptr,
+                           v.scratch, v.scratch_bytes, s))) return rc;
+        if ((rc = h128_fwd(d, d->precision, on, R, d->T, v.x_on, nullptr, v.h_stash, v.gates, 4 * d->H, 1, v.q_on, nullptr,
+                           v.scratch, v.scratch_bytes, s))) return rc;
+    } else if (!tc_agent) {
         PHASE(s, "gru_unroll_fwd_online");
         if ((rc = gru_fwd_dispatch(d, on, R, d->T, v.x_on, nullptr, v.h_stash, v.gates, v.q_on, nullptr, s))) return rc;
         PHASE(s, "gru_unroll_fwd_target");

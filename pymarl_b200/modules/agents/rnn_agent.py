@@ -54,10 +54,12 @@ class RNNAgent(nn.Module):
         x = th.empty(rows, H, dtype=th.float32, device=x_in.device)
         q = th.empty(rows, A, dtype=th.float32, device=x_in.device)
         h = th.empty(rows, H, dtype=th.float32, device=x_in.device)
+        # H = 128 computes the input gates of all rows as one GEMM before the recurrence: they need a buffer
+        gates = th.empty(rows, 4 * H, dtype=th.float32, device=x_in.device) if H == 128 else None
         s = _lib.stream_ptr(x_in.device)
         L = _lib.lib()
         _lib.check(L.pmb_agent_fc1_dense_fwd(C.byref(dims), rows, self.d_in, _lib.ptr(x_in), flat,
                                              _lib.ptr(x), s), "pmb_agent_fc1_dense_fwd")
         _lib.check(L.pmb_agent_gru_unroll_fwd(C.byref(dims), rows, 1, flat, _lib.ptr(x), _lib.ptr(h_in),
-                                              None, None, _lib.ptr(q), _lib.ptr(h), s), "pmb_agent_gru_unroll_fwd")
+                                              None, _lib.ptr(gates), _lib.ptr(q), _lib.ptr(h), s), "pmb_agent_gru_unroll_fwd")
         return q, h
