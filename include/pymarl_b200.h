@@ -236,6 +236,23 @@ int pmb_agent_unroll_bwd(const pmb_dims* d, const pmb_batch* b, const float* fla
                          const float* h_stash, float* gates, const float* d_chosen, float* dpre1,
                          float* flat_grad_agent, void* scratch, int64_t scratch_bytes, pmb_stream stream);
 
+/* ---- K5b: backward of ONE agent step, for autograd through RNNAgent / BasicMAC (a user's learner calling
+ * loss.backward(); rnn_agent.py:27-36, basic_controller.py:40-49,100-135) ------------------------------------------------
+ * The step is pmb_agent_fc1_fwd (batch at time t) or pmb_agent_fc1_dense_fwd (inputs [rows][O], d->O = D_in and both
+ * one-hot flags 0), then pmb_agent_gru_unroll_fwd with nt = 1, which saved x [R][H] (fc1 output), h_stash [2][R][H]
+ * (h_prev | h) and gates [R][4H].  fp32 kernels on every precision tier (pmb_dims.precision is ignored).
+ * dq [R][A] = dL/dq and dh [R][H] = dL/dh may be NULL (no gradient reached them).  Writes dh_prev [R][H] = dL/dh_prev
+ * (may be NULL) and OVERWRITES flat_grad_agent, an n_agent-float block in the flat agent layout, with the step's eight
+ * parameter gradients: fc1.weight over the whole D_in (obs, last-action and agent-id columns), every other tensor
+ * dense.  Pass exactly one of b (with t the batch time the forward read) and inputs.  2 launches (3 when the rows are
+ * split into slices), no float atomics: identical calls give identical bits.  scratch >=
+ * pmb_agent_step_bwd_workspace_bytes(d, rows). */
+int64_t pmb_agent_step_bwd_workspace_bytes(const pmb_dims* d, int64_t rows);
+int pmb_agent_step_bwd(const pmb_dims* d, const pmb_batch* b, int32_t t, const float* inputs, int64_t rows,
+                       const float* flat_agent, const float* x, const float* h_stash, const float* gates, const float* dq,
+                       const float* dh, float* dh_prev, float* flat_grad_agent, void* scratch, int64_t scratch_bytes,
+                       pmb_stream stream);
+
 /* ---- K6: grad-norm clip + RMSprop + optional hard target sync (q_learner.py:102-107) --- */
 /* g is the un-normalised gradient; stats[PMB_S_MASK_SUM] supplies the 1/sum(mask) factor.
  * clip_grad_norm_: coef = min(1, clip / (norm + 1e-6)); RMSprop: v = a v + (1-a) g^2,

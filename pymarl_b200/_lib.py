@@ -144,6 +144,9 @@ _SIGS = {
     "pmb_mixer_bwd": (C.c_int, [C.POINTER(Dims), C.POINTER(Batch), _P, _P, _P, _P, _P, _P, _P, C.c_int64, _P]),
     "pmb_agent_bwd_workspace_bytes": (C.c_int64, [C.POINTER(Dims)]),
     "pmb_agent_unroll_bwd": (C.c_int, [C.POINTER(Dims), C.POINTER(Batch), _P, _P, _P, _P, _P, _P, _P, _P, C.c_int64, _P]),
+    "pmb_agent_step_bwd_workspace_bytes": (C.c_int64, [C.POINTER(Dims), C.c_int64]),
+    "pmb_agent_step_bwd": (C.c_int, [C.POINTER(Dims), C.POINTER(Batch), C.c_int32, _P, C.c_int64, _P, _P, _P, _P, _P, _P,
+                                     _P, _P, _P, C.c_int64, _P]),
     "pmb_clip_rmsprop_update": (C.c_int, [C.c_int64, _P, _P, _P, _P, C.c_int32, _P, C.c_float, C.c_float, C.c_float,
                                           C.c_float, _P, _P]),
     "pmb_dp_pack": (C.c_int, [C.c_int64, _P, _P, _P]),
@@ -228,6 +231,18 @@ def stream_ptr(device=None):
 def require_cuda(t, name):
     if not t.is_cuda:
         raise PmbError("%s must live on a CUDA device (pymarl_b200 has no CPU path); got %s" % (name, t.device))
+
+
+def autograd_mode(args):
+    """True when a module called with these args builds an autograd graph: the ``autograd_modules`` key is set and grad
+    mode is on (not under th.no_grad() / th.inference_mode()).  Otherwise the modules run their inference kernels."""
+    return bool(getattr(args, "autograd_modules", False)) and th.is_grad_enabled()
+
+
+def no_double_backward(what):
+    """Called at the top of a module Function's backward: the hand-written backward kernels are not differentiable."""
+    if th.is_grad_enabled():
+        raise PmbError("%s: double backward (create_graph=True) is not supported by the pymarl_b200 kernels" % what)
 
 
 def make_dims(B, T, N, O, S, A, H, E, obs_last_action=True, obs_agent_id=True, mixer="qmix", double_q=True,

@@ -8,6 +8,13 @@ the GRU cell, fc2, avail masking and epsilon-greedy selection.
 Only the upstream configuration is implemented: agent "rnn", agent_output_type "q",
 obs_decoder None, action_input_representation None (SURVEY.md section 2, row 3b).
 
+With ``args.autograd_modules = True`` and grad mode on, forward() builds one autograd node per timestep instead
+(modules.agents.rnn_agent.AgentStep: pmb_agent_fc1_fwd + pmb_agent_gru_unroll_fwd, backward pmb_agent_step_bwd) on
+the same virtual input, and ``hidden_states`` carries the graph from step to step, so a user's learner can unroll
+``mac.forward(batch, t)`` over t and call loss.backward() (BPTT falls out of autograd).  The pi_logits policy head is
+then restated in torch ops.  That mode runs the fp32 kernels whatever ``args.precision`` says.  select_actions() never
+builds a graph.
+
 Note on the last-action input: the reference reads ``actions_onehot[:, t-1]``; this package
 reads ``actions[:, t-1]`` and ``filled[:, t-1]`` instead (the one-hot row is all-zero exactly
 when the step was never written), so ``actions_onehot`` is never touched on the device.
@@ -19,6 +26,7 @@ import torch as th
 from .. import _lib, flat as _flat
 from ..components.action_selectors import REGISTRY as action_REGISTRY
 from ..modules.agents import REGISTRY as agent_REGISTRY
+from ..modules.agents.rnn_agent import AgentStep
 
 
 class BasicMAC:
@@ -45,21 +53,28 @@ class BasicMAC:
     def _device(self):
         return self.agent.fc1.weight.device
 
-    def _dims(self, ep_batch):
+    def _dims(self, ep_batch, precision=None):
         a = self.args
         obs = ep_batch["obs"]
         return _lib.make_dims(B=ep_batch.batch_size, T=obs.shape[1], N=self.n_agents, O=obs.shape[-1], S=1,
                               A=a.n_actions, H=a.rnn_hidden_dim, E=1, obs_last_action=a.obs_last_action,
-                              obs_agent_id=a.obs_agent_id, mixer=None, precision=getattr(a, "precision", "fp32"))
+                              obs_agent_id=a.obs_agent_id, mixer=None, precision=precision or getattr(a, "precision", "fp32"))
 
-    def _step_batch(self, ep_batch, t, keep, dims):
-        """pmb_batch with just the fields a rollout step reads.  When the runner keeps its
+    def _step_batch(self, ep_batch, t, keep, dims, entry=_lib.ENTRY_SELECT_ACTIONS):
+        """pmb_batch with just the fields a rollout step reads (entry None: converted to the reference types).  When the runner keeps its
         batch on the host (reference behaviour, basic_controller.py:32,105,113) only the
         timesteps the step needs are copied, re-based so that the kernel's index t maps onto
         them.  bf16 obs and uint8 / bool avail stay as they are where the rollout kernels read them natively for ``dims``."""
         dev = self._device()
         fields = {}
-        if ep_batch["obs"].is_cuda:
+        if ep_batch["obs"].is_cuda and entry is None:
+            # converted fields (compact obs / avail): views of steps t-1 and t only, so that a conversion touches two
+            # timesteps, not the episode (the autograd path keeps them until the backward)
+            lo = max(t - 1, 0)
+            for k in ("obs", "actions", "avail_actions", "filled"):
+                fields[k] = ep_batch[k][:, lo:t + 1]
+            t_local, T_local = t - lo, t + 1 - lo
+        elif ep_batch["obs"].is_cuda:
             for k in ("obs", "actions", "avail_actions", "filled"):
                 fields[k] = ep_batch[k]
             t_local, T_local = t, ep_batch["obs"].shape[1]
@@ -79,7 +94,7 @@ class BasicMAC:
             self._dummies = (zero, zero.to(th.uint8))
         zero, zero_u8 = self._dummies
         fields.update(state=zero, reward=zero, terminated=zero_u8)
-        b = _lib.make_batch(fields, need_state=False, keep=keep, dims=dims, entry=_lib.ENTRY_SELECT_ACTIONS)
+        b = _lib.make_batch(fields, need_state=False, keep=keep, dims=dims, entry=entry)
         return b, t_local, T_local
 
     def _run_step(self, ep_batch, t, epsilon=None, u=None, expo=None, seed=0, offset=0, want_actions=False, want_q=True):
@@ -123,7 +138,8 @@ class BasicMAC:
         sel = self.action_selector
         full = isinstance(bs, slice) and bs == slice(None)
         if self.agent_output_type == "pi_logits":
-            probs = self.forward(ep_batch, t_ep, test_mode=test_mode)
+            with th.no_grad():
+                probs = self.forward(ep_batch, t_ep, test_mode=test_mode)
             avail = ep_batch["avail_actions"][:, t_ep]
             return sel.select_action(probs[bs].to(self._device()), avail[bs].to(self._device()), t_env, test_mode=test_mode)
         if full and sel.rng != "torch":
@@ -136,7 +152,35 @@ class BasicMAC:
         avail = ep_batch["avail_actions"][:, t_ep]
         return sel.select_action(q[bs], avail[bs].to(q.device), t_env, test_mode=test_mode)
 
+    def _autograd_step(self, ep_batch, t):
+        """One autograd node for the agent step at t (AgentStep); the new hidden state keeps the graph."""
+        _lib.require_cuda(self.agent.fc1.weight, "agent parameters")
+        if self.hidden_states is None:
+            raise RuntimeError("call init_hidden(batch_size) before forward/select_actions")
+        keep = []
+        dims = self._dims(ep_batch, precision="fp32")
+        batch, t_local, T_local = self._step_batch(ep_batch, t, keep, dims, entry=None)
+        dims.T = T_local
+        R, H = dims.B * dims.N, dims.H
+        h_in = self.hidden_states.reshape(-1, H)
+        if h_in.shape[0] != R:
+            h_in = h_in.expand(R, H)
+        h_in = h_in.to(device=self._device(), dtype=th.float32).contiguous()
+        q, self.hidden_states = AgentStep.apply(self.agent, dims, (batch, t_local, keep), h_in, *self.agent.parameters())
+        return q
+
     def forward(self, ep_batch, t, test_mode=False):
+        if _lib.autograd_mode(self.args):
+            q = self._autograd_step(ep_batch, t)
+            if self.agent_output_type == "pi_logits":
+                # what pmb_policy_head computes (basic_controller.py:55-71), differentiable
+                avail = ep_batch["avail_actions"][:, t].to(q.device).reshape(q.shape)
+                off = avail == 0
+                q = th.softmax(q.masked_fill(off, -1e10), dim=-1)
+                if not test_mode:
+                    eps = float(self.action_selector.epsilon)
+                    q = ((1.0 - eps) * q + eps / (~off).sum(-1, keepdim=True).float()).masked_fill(off, 0.0)
+            return q.view(ep_batch.batch_size, self.n_agents, -1).to(ep_batch.device)
         q, _ = self._run_step(ep_batch, t)
         if self.agent_output_type == "pi_logits":
             # basic_controller.py:55-71: masked softmax, epsilon floor over the available actions, unavailable -> 0

@@ -40,6 +40,11 @@ int launch_td_loss(const pmb_dims* d, const pmb_batch* b, const float* q_tot, co
 int launch_stats_reset(double* stats, cudaStream_t s);
 int launch_dp_pack(const double* stats, float* tail, cudaStream_t s);
 int launch_dp_unpack(const float* tail, double* stats, cudaStream_t s);
+// agent_step.cu
+int64_t agent_step_bwd_scratch(const pmb_dims* d, int64_t R);
+int agent_step_bwd(const pmb_dims* d, const pmb_batch* b, int t, const float* inputs, int64_t R, const float* flat_agent,
+                   const float* x, const float* h_stash, const float* gates, const float* dq, const float* dh,
+                   float* dh_prev, float* flat_grad_agent, void* scratch, int64_t scratch_bytes, cudaStream_t s);
 // coma.cu
 int coma_launch_inputs(const pmb_dims* d, const pmb_batch* b, int t0, int nt, float* out, cudaStream_t s);
 int coma_launch_gather_taken(const pmb_dims* d, const pmb_batch* b, int t0, int nt, const float* q, float* taken, cudaStream_t s);
@@ -650,6 +655,32 @@ int pmb_agent_unroll_bwd(const pmb_dims* d, const pmb_batch* b, const float* fla
     if ((rc = check_dtypes(d, b, -1, "pmb_agent_unroll_bwd"))) return rc;
     return agent_bwd(d, b, flat_agent, x_on, h_stash, gates, d_chosen, dpre1, flat_grad_agent, scratch, scratch_bytes,
                      (cudaStream_t)stream);
+}
+
+int64_t pmb_agent_step_bwd_workspace_bytes(const pmb_dims* d, int64_t rows) {
+    if (validate_dims(d) || rows <= 0) return -1;
+    return agent_step_bwd_scratch(d, rows);
+}
+
+int pmb_agent_step_bwd(const pmb_dims* d, const pmb_batch* b, int32_t t, const float* inputs, int64_t rows,
+                       const float* flat_agent, const float* x, const float* h_stash, const float* gates, const float* dq,
+                       const float* dh, float* dh_prev, float* flat_grad_agent, void* scratch, int64_t scratch_bytes,
+                       pmb_stream stream) {
+    int rc = validate_dims(d);
+    if (rc) return rc;
+    PMB_REQUIRE(rows > 0 && flat_agent && x && h_stash && gates && flat_grad_agent && scratch, "agent_step_bwd: NULL pointer");
+    PMB_REQUIRE((b == nullptr) != (inputs == nullptr), "agent_step_bwd: pass exactly one of the batch and a dense input");
+    if (b) {
+        PMB_REQUIRE(b->obs && b->ep_index == nullptr, "agent_step_bwd: batch.obs missing or batch.ep_index set");
+        PMB_REQUIRE(rows == (int64_t)d->B * d->N, "agent_step_bwd: rows %lld != B * N", (long long)rows);
+        PMB_REQUIRE(t >= 0 && t < d->T, "agent_step_bwd: t = %d outside [0, %d)", t, d->T);
+        PMB_REQUIRE(!d->obs_last_action || (b->actions && b->filled), "agent_step_bwd: obs_last_action needs actions and filled");
+        if ((rc = check_dtypes(d, b, -1, "pmb_agent_step_bwd"))) return rc;
+    } else {
+        PMB_REQUIRE(!d->obs_last_action && !d->obs_agent_id, "agent_step_bwd: a dense input has no one-hot blocks (D_in = O)");
+    }
+    return agent_step_bwd(d, b, t, inputs, rows, flat_agent, x, h_stash, gates, dq, dh, dh_prev, flat_grad_agent, scratch,
+                          scratch_bytes, (cudaStream_t)stream);
 }
 
 int pmb_clip_rmsprop_update(int64_t n, float* flat_p, float* flat_g, float* flat_sq, float* flat_target,

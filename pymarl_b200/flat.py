@@ -64,11 +64,9 @@ def ensure_block(module, kind, dims):
     addr = block_ptr(module, kind, layout)
     if addr is not None:
         return addr
-    first = _FIRST_ID[kind]
     p0 = _named(module)[_KEYS[kind][0]]
     _lib.require_cuda(p0, "%s parameters" % kind)
-    n = sum(layout.numel[first + i] for i in range(len(_KEYS[kind])))
-    flat = th.empty(n, dtype=th.float32, device=p0.device)
+    flat = th.empty(block_numel(layout, kind), dtype=th.float32, device=p0.device)
     bind(flat, layout, module, kind, base=0)
     return flat.data_ptr()
 
@@ -106,3 +104,20 @@ def is_bound_in_order(module, keys, flat):
             return False
         off += p.numel()
     return True
+
+
+def grad_views(block, layout, module, kind):
+    """Per-parameter views (in named_parameters() order) of a flat gradient block of `kind` that starts at the block's
+    own offset: what a module Function's backward returns for the parameters."""
+    first, keys = _FIRST_ID[kind], _KEYS[kind]
+    block0 = layout.offset[first]
+    view = {}
+    for i, k in enumerate(keys):
+        off, n = layout.offset[first + i] - block0, layout.numel[first + i]
+        view[k] = block[off:off + n]
+    return [view[k].view(p.shape) for k, p in module.named_parameters()]
+
+
+def block_numel(layout, kind):
+    first = _FIRST_ID[kind]
+    return sum(layout.numel[first + i] for i in range(len(_KEYS[kind])))
