@@ -432,6 +432,27 @@ int pmb_coma_train_step(const pmb_dims* d, const pmb_batch* b, const pmb_coma_hp
  * workspace >= pmb_coma_workspace_bytes(d). */
 int pmb_coma_critic_fwd(const pmb_dims* d, const pmb_batch* b, const float* critic_p, int32_t t0, int32_t nt, float* q_out,
                         void* workspace, int64_t workspace_bytes, pmb_stream stream);
+/* ---- COMACritic.forward as one autograd node, for a user's actor-critic learner calling loss.backward() on the
+ * critic's q (coma_learner.py:118-146) ------------------------------------------------------------------------------
+ * pmb_coma_critic_step_fwd: pmb_coma_critic_fwd's launches, giving the same q_out bits, with the two hidden activations
+ * x1 = relu(fc1(input)) and x2 = relu(fc2(x1)) written to x1_out / x2_out, [B * nt * N][E] each.  Row order: the nt
+ * timesteps go in chunks of c = clamp((64 << 20) / (B N D), 1, T) timesteps (the last chunk may be shorter); chunk
+ * after chunk, the rows of a chunk of cn timesteps are (b, tt, n), b-major.  With nt <= c that is [B][nt][N].
+ * workspace >= pmb_coma_workspace_bytes(d).  Per chunk: 4 launches (input generation, three GEMMs) and one copy.
+ * pmb_coma_critic_step_bwd: from dq [B][nt][N][A] = dL/dq (dense fp32) and the x1 / x2 of the forward over the same
+ * (d, batch, t0, nt), OVERWRITES critic_g, a pmb_coma_critic_numel(d)-float block in the flat critic layout, with the
+ * gradients of all six critic tensors.  fc1.weight gets every column of D: the state columns from dx1 summed over the
+ * N agents of an (episode, step), the obs columns dense, the two one-hot action blocks and the agent-id block by index
+ * from actions / filled as the forward generates them; the input matrix is not built.  No gradient reaches the batch.
+ * fp32 kernels on every precision tier.  2 launches (3 when the rows are split into slices), no float atomics:
+ * identical calls give identical bits.  scratch >= pmb_coma_critic_step_bwd_workspace_bytes(d, nt). */
+int pmb_coma_critic_step_fwd(const pmb_dims* d, const pmb_batch* b, const float* critic_p, int32_t t0, int32_t nt,
+                             float* q_out, float* x1_out, float* x2_out, void* workspace, int64_t workspace_bytes,
+                             pmb_stream stream);
+int64_t pmb_coma_critic_step_bwd_workspace_bytes(const pmb_dims* d, int32_t nt);
+int pmb_coma_critic_step_bwd(const pmb_dims* d, const pmb_batch* b, const float* critic_p, int32_t t0, int32_t nt,
+                             const float* dq, const float* x1, const float* x2, float* critic_g, void* scratch,
+                             int64_t scratch_bytes, pmb_stream stream);
 /* BasicMAC.forward's policy head for agent_output_type == "pi_logits" (controllers/basic_controller.py:51-73,
  * mask_before_softmax): probs [rows][A] from logits / avail [rows][A]; test_mode: plain masked softmax. */
 int pmb_policy_head(int64_t rows, int32_t A, float epsilon, int32_t test_mode, const float* logits, const int32_t* avail,

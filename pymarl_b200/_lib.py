@@ -173,6 +173,11 @@ _SIGS = {
     "pmb_coma_train_step": (C.c_int, [C.POINTER(Dims), C.POINTER(Batch), C.POINTER(ComaHParams), _P, _P, _P, _P, _P, _P, _P, _P,
                                       C.c_int64, _P, _P]),
     "pmb_coma_critic_fwd": (C.c_int, [C.POINTER(Dims), C.POINTER(Batch), _P, C.c_int32, C.c_int32, _P, _P, C.c_int64, _P]),
+    "pmb_coma_critic_step_fwd": (C.c_int, [C.POINTER(Dims), C.POINTER(Batch), _P, C.c_int32, C.c_int32, _P, _P, _P, _P,
+                                           C.c_int64, _P]),
+    "pmb_coma_critic_step_bwd_workspace_bytes": (C.c_int64, [C.POINTER(Dims), C.c_int32]),
+    "pmb_coma_critic_step_bwd": (C.c_int, [C.POINTER(Dims), C.POINTER(Batch), _P, C.c_int32, C.c_int32, _P, _P, _P, _P, _P,
+                                           C.c_int64, _P]),
     "pmb_policy_head": (C.c_int, [C.c_int64, C.c_int32, C.c_float, C.c_int32, _P, _P, _P, _P]),
     "pmb_multinomial": (C.c_int, [C.c_int64, C.c_int32, _P, _P, _P, C.c_int32, C.c_uint64, C.c_uint64, _P, _P]),
     "pmb_qlearner_train_step": (C.c_int, [C.POINTER(Dims), C.POINTER(Batch), C.POINTER(HParams), _P, _P, _P, _P, _P,

@@ -45,6 +45,11 @@ int64_t agent_step_bwd_scratch(const pmb_dims* d, int64_t R);
 int agent_step_bwd(const pmb_dims* d, const pmb_batch* b, int t, const float* inputs, int64_t R, const float* flat_agent,
                    const float* x, const float* h_stash, const float* gates, const float* dq, const float* dh,
                    float* dh_prev, float* flat_grad_agent, void* scratch, int64_t scratch_bytes, cudaStream_t s);
+// critic_step.cu
+int64_t critic_step_bwd_scratch(const pmb_dims* d, int nt);
+int critic_step_bwd(const pmb_dims* d, const pmb_batch* b, int t0, int nt, int chunk_nt, const CriticParams& cp,
+                    const float* x1, const float* x2, const float* dq, const CriticGrads& g, void* scratch,
+                    int64_t scratch_bytes, cudaStream_t s);
 // coma.cu
 int coma_launch_inputs(const pmb_dims* d, const pmb_batch* b, int t0, int nt, float* out, cudaStream_t s);
 int coma_launch_gather_taken(const pmb_dims* d, const pmb_batch* b, int t0, int nt, const float* q, float* taken, cudaStream_t s);
@@ -1084,13 +1089,6 @@ ComaPlan coma_plan(const pmb_dims* d) {
     p.total = off + p.scratch_bytes;
     return p;
 }
-struct CriticParams { const float *w1, *b1, *w2, *b2, *w3, *b3; };
-struct CriticGrads { float *w1, *b1, *w2, *b2, *w3, *b3; };
-template <class P, class F>
-P critic_views(F* flat, int64_t D, int64_t Hc, int64_t A) {
-    F* w1 = flat; F* b1 = w1 + Hc * D; F* w2 = b1 + Hc; F* b2 = w2 + Hc * Hc; F* w3 = b2 + Hc; F* b3 = w3 + A * Hc;
-    return P{w1, b1, w2, b2, w3, b3};
-}
 int critic_fwd(const CriticParams& c, const float* inp, int64_t rows, int64_t D, int Hc, int A, float* x1, float* x2, float* q,
                cudaStream_t s) {
     int rc;
@@ -1102,6 +1100,37 @@ int validate_coma(const pmb_dims* d) {
     int rc = validate_dims(d);
     if (rc) return rc;
     PMB_REQUIRE(d->T >= 2 && d->S > 0 && d->E > 0 && d->E <= 1024 && d->A <= 64, "coma: need T >= 2, a state, critic width 1..1024, n_actions <= 64");
+    return PMB_OK;
+}
+// COMACritic.forward over batch timesteps t0 .. t0 + nt - 1 in chunks of coma_plan's chunk_nt; x1_out / x2_out (both or
+// neither): the hidden activations, chunk after chunk, rows (b, tt, n) inside a chunk
+int critic_fwd_range(const pmb_dims* d, const pmb_batch* b, const float* critic_p, int t0, int nt, float* q_out,
+                     float* x1_out, float* x2_out, void* workspace, int64_t workspace_bytes, pmb_stream stream, const char* who) {
+    int rc = validate_coma(d);
+    if (rc) return rc;
+    PMB_REQUIRE(b && critic_p && q_out && workspace && b->obs && b->state && b->actions && b->filled && !b->ep_index,
+                "%s: NULL pointer", who);
+    if ((rc = check_dtypes(d, b, -1, who))) return rc;
+    PMB_REQUIRE(t0 >= 0 && nt > 0 && t0 + nt <= d->T, "%s: bad time range", who);
+    cudaStream_t s = (cudaStream_t)stream;
+    ComaPlan P = coma_plan(d);
+    if (workspace_bytes < P.total) { set_error("coma workspace too small"); return PMB_ERR_WORKSPACE; }
+    char* base = static_cast<char*>(workspace);
+    auto f = [&](int i) { return reinterpret_cast<float*>(base + P.off[i]); };
+    CriticParams cp = critic_views<CriticParams, const float>(critic_p, P.D, P.Hc, d->A);
+    // q_out [B][nt][N][A]; chunks of timesteps keep the materialised input matrix bounded (rows are (b, tt, n) per chunk,
+    // so a chunk's rows are scattered into q_out per episode)
+    for (int c0 = 0; c0 < nt; c0 += (int)P.chunk_nt) {
+        const int cn = nt - c0 < P.chunk_nt ? nt - c0 : (int)P.chunk_nt;
+        const int64_t r0 = P.R * c0;
+        float* x1 = x1_out ? x1_out + r0 * P.Hc : f(1);
+        float* x2 = x2_out ? x2_out + r0 * P.Hc : f(2);
+        if ((rc = coma_launch_inputs(d, b, t0 + c0, cn, f(0), s))) return rc;
+        if ((rc = critic_fwd(cp, f(0), P.R * cn, P.D, (int)P.Hc, d->A, x1, x2, f(3), s))) return rc;
+        PMB_CUDA(cudaMemcpy2DAsync(q_out + (int64_t)c0 * d->N * d->A, sizeof(float) * nt * d->N * d->A, f(3),
+                                   sizeof(float) * cn * d->N * d->A, sizeof(float) * cn * d->N * d->A, (size_t)d->B,
+                                   cudaMemcpyDeviceToDevice, s));
+    }
     return PMB_OK;
 }
 }  // namespace
@@ -1202,29 +1231,36 @@ int pmb_coma_train_step(const pmb_dims* d, const pmb_batch* b, const pmb_coma_hp
 
 int pmb_coma_critic_fwd(const pmb_dims* d, const pmb_batch* b, const float* critic_p, int32_t t0, int32_t nt, float* q_out,
                         void* workspace, int64_t workspace_bytes, pmb_stream stream) {
+    return critic_fwd_range(d, b, critic_p, t0, nt, q_out, nullptr, nullptr, workspace, workspace_bytes, stream,
+                            "pmb_coma_critic_fwd");
+}
+
+int pmb_coma_critic_step_fwd(const pmb_dims* d, const pmb_batch* b, const float* critic_p, int32_t t0, int32_t nt,
+                             float* q_out, float* x1_out, float* x2_out, void* workspace, int64_t workspace_bytes,
+                             pmb_stream stream) {
+    PMB_REQUIRE(x1_out && x2_out, "coma_critic_step_fwd: NULL activation buffer");
+    return critic_fwd_range(d, b, critic_p, t0, nt, q_out, x1_out, x2_out, workspace, workspace_bytes, stream,
+                            "pmb_coma_critic_step_fwd");
+}
+
+int64_t pmb_coma_critic_step_bwd_workspace_bytes(const pmb_dims* d, int32_t nt) {
+    if (validate_coma(d) || nt <= 0 || nt > d->T) return -1;
+    return critic_step_bwd_scratch(d, nt);
+}
+
+int pmb_coma_critic_step_bwd(const pmb_dims* d, const pmb_batch* b, const float* critic_p, int32_t t0, int32_t nt,
+                             const float* dq, const float* x1, const float* x2, float* critic_g, void* scratch,
+                             int64_t scratch_bytes, pmb_stream stream) {
     int rc = validate_coma(d);
     if (rc) return rc;
-    PMB_REQUIRE(b && critic_p && q_out && workspace && b->obs && b->state && b->actions && b->filled && !b->ep_index,
-                "coma_critic_fwd: NULL pointer");
-    if ((rc = check_dtypes(d, b, -1, "pmb_coma_critic_fwd"))) return rc;
-    PMB_REQUIRE(t0 >= 0 && nt > 0 && t0 + nt <= d->T, "coma_critic_fwd: bad time range");
-    cudaStream_t s = (cudaStream_t)stream;
+    PMB_REQUIRE(b && critic_p && dq && x1 && x2 && critic_g && scratch && b->obs && b->state && b->actions && b->filled &&
+                    !b->ep_index, "coma_critic_step_bwd: NULL pointer (or batch.ep_index given)");
+    if ((rc = check_dtypes(d, b, -1, "pmb_coma_critic_step_bwd"))) return rc;
+    PMB_REQUIRE(t0 >= 0 && nt > 0 && t0 + nt <= d->T, "coma_critic_step_bwd: bad time range");
     ComaPlan P = coma_plan(d);
-    if (workspace_bytes < P.total) { set_error("coma workspace too small"); return PMB_ERR_WORKSPACE; }
-    char* base = static_cast<char*>(workspace);
-    auto f = [&](int i) { return reinterpret_cast<float*>(base + P.off[i]); };
     CriticParams cp = critic_views<CriticParams, const float>(critic_p, P.D, P.Hc, d->A);
-    // q_out [B][nt][N][A]; chunks of timesteps keep the materialised input matrix bounded (rows are (b, tt, n) per chunk,
-    // so a chunk's rows are scattered into q_out per episode)
-    for (int c0 = 0; c0 < nt; c0 += (int)P.chunk_nt) {
-        const int cn = nt - c0 < P.chunk_nt ? nt - c0 : (int)P.chunk_nt;
-        if ((rc = coma_launch_inputs(d, b, t0 + c0, cn, f(0), s))) return rc;
-        if ((rc = critic_fwd(cp, f(0), P.R * cn, P.D, (int)P.Hc, d->A, f(1), f(2), f(3), s))) return rc;
-        PMB_CUDA(cudaMemcpy2DAsync(q_out + (int64_t)c0 * d->N * d->A, sizeof(float) * nt * d->N * d->A, f(3),
-                                   sizeof(float) * cn * d->N * d->A, sizeof(float) * cn * d->N * d->A, (size_t)d->B,
-                                   cudaMemcpyDeviceToDevice, s));
-    }
-    return PMB_OK;
+    CriticGrads cg = critic_views<CriticGrads, float>(critic_g, P.D, P.Hc, d->A);
+    return critic_step_bwd(d, b, t0, nt, (int)P.chunk_nt, cp, x1, x2, dq, cg, scratch, scratch_bytes, (cudaStream_t)stream);
 }
 
 int pmb_policy_head(int64_t rows, int32_t A, float epsilon, int32_t test_mode, const float* logits, const int32_t* avail,

@@ -134,6 +134,16 @@ inline MixerParams mixer_params(const pmb_dims* d, const float* flat_mixer) {
                        flat_mixer + (L.offset[PMB_P_V2_W] - base), flat_mixer + (L.offset[PMB_P_V2_B] - base)};
 }
 
+// COMA critic, flat layout in state_dict order: fc1.weight [Hc][D] | fc1.bias | fc2.weight [Hc][Hc] | fc2.bias |
+// fc3.weight [A][Hc] | fc3.bias
+struct CriticParams { const float *w1, *b1, *w2, *b2, *w3, *b3; };
+struct CriticGrads { float *w1, *b1, *w2, *b2, *w3, *b3; };
+template <class P, class F>
+P critic_views(F* flat, int64_t D, int64_t Hc, int64_t A) {
+    F* w1 = flat; F* b1 = w1 + Hc * D; F* w2 = b1 + Hc; F* b2 = w2 + Hc * Hc; F* w3 = b2 + Hc; F* b3 = w3 + A * Hc;
+    return P{w1, b1, w2, b2, w3, b3};
+}
+
 // ---- kernels implemented in other translation units (host launchers) ---------------------
 // gemm_simt.cu
 //   C[m, n] (+ epilogue) = sum_k A[rowmap(m) + k] * W[n*ldw + k]
