@@ -263,7 +263,9 @@ int pmb_clip_rmsprop_update(int64_t n, float* flat_p, float* flat_g, float* flat
 
 /* ---- K8: data-parallel exchange (SURVEY.md section 8e; no counterpart in the reference, which is single-process) ----
  * Episodes shard over ranks; every rank runs pmb_qlearner_train_step with skip_update = 1, then
- *   pmb_dp_pack(n, flat_g, stats)    : appends the five loss sums as (hi, lo) float pairs behind the n gradients
+ *   pmb_dp_pack(n, flat_g, stats)    : appends the five loss sums as (hi, lo) float pairs behind the n gradients (hi + lo
+ *                                      = the double to 2^-48; mask_sum, a count, split at a multiple of 2^12 so that fp32
+ *                                      sums of up to 8 ranks keep it exact below 2^36) and zeroes the other 6 tail floats
  *   ONE all-reduce(sum, fp32) over flat_g[0 .. n + PMB_DP_TAIL_FLOATS)   (NCCL, issued by the host plumbing)
  *   pmb_dp_unpack(n, flat_g, stats)  : restores the (now global) sums
  *   pmb_clip_rmsprop_update(...)     : identical update on every rank (replicated parameters / optimizer state)

@@ -373,7 +373,7 @@ def gather_episode_steps(src, ep_ids, steps, out, filled=None):
         v, o = src[k], out[k]
         if not v.is_contiguous() or tuple(v.shape[:2]) != (n_src, T_src):
             raise PmbError("gather_episode_steps needs contiguous [n_src, T, ...] buffer fields (%r is not)" % k)
-        if tuple(o.shape) != (n, steps) + tuple(v.shape[2:]) or o.dtype != v.dtype or not o[0].is_contiguous():
+        if tuple(o.shape) != (n, steps) + tuple(v.shape[2:]) or o.dtype != v.dtype or (n > 0 and not o[0].is_contiguous()):
             raise PmbError("gather_episode_steps: out[%r] must be episode_rows(%d, %r)" % (k, n, (steps,) + tuple(v.shape[2:])))
     if filled is not None and (not filled.is_contiguous() or filled.dtype != th.int64 or tuple(filled.shape[:2]) != (n_src, T_src)):
         raise PmbError("gather_episode_steps: filled must be the buffer's contiguous int64 [n_src, T] field")

@@ -94,6 +94,17 @@ __device__ __forceinline__ double warp_sum(double v) {
     return v;
 }
 
+// ---- data-parallel exchange: loss sum i as a (hi, lo) float pair (pmb_dp_pack, dp_peer.cu) ----
+// hi + lo reproduces the double to 2^-48.  mask_sum, an integer count, is split at a multiple of 2^12 instead: hi =
+// floor(v / 2^12) * 2^12, lo = v - hi < 2^12.  Then every partial fp32 sum over up to 8 ranks of the hi parts (multiples of
+// 2^12) and of the lo parts (integers < 2^15) is exact, so the exchanged count stays exact up to 2^36 in all; with the
+// plain split an odd global count above 2^24 would round.
+__device__ __forceinline__ void dp_pack_sum(int i, double v, float* pair) {
+    const double hi = i == PMB_S_MASK_SUM ? floor(v * (1.0 / 4096.0)) * 4096.0 : (double)(float)v;
+    pair[0] = (float)hi;
+    pair[1] = (float)(v - hi);
+}
+
 __device__ __forceinline__ float sigmoidf_acc(float x) { return 1.0f / (1.0f + expf(-x)); }
 
 // flat parameter views -----------------------------------------------------------------------

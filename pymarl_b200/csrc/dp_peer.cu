@@ -53,12 +53,8 @@ dp_fused_kernel(PeerArgs A, long long step, unsigned long long epoch, float* __r
 
     // ---- P0: publish, then wait for everybody's gradients ----
     if (blockIdx.x == 0) {
-        if (threadIdx.x < 5) {                                  // loss sums as (hi, lo) float pairs behind the gradient
-            const double v = stats[threadIdx.x];
-            const float hi = (float)v;
-            mine[A.n + 2 * threadIdx.x] = hi;
-            mine[A.n + 2 * threadIdx.x + 1] = (float)(v - (double)hi);
-        }
+        if (threadIdx.x < 5)                                    // loss sums as (hi, lo) float pairs behind the gradient
+            dp_pack_sum(threadIdx.x, stats[threadIdx.x], mine + A.n + 2 * threadIdx.x);
         __syncthreads();
         __threadfence_system();
         if (threadIdx.x < world) {
@@ -91,7 +87,8 @@ dp_fused_kernel(PeerArgs A, long long step, unsigned long long epoch, float* __r
         }
         if (threadIdx.x < 5) {
             double hi = 0.0, lo = 0.0;
-            float fh = 0.f, fl = 0.f;                           // summed in fp32 in rank order, like the NCCL path
+            float fh = 0.f, fl = 0.f;                           // summed in fp32 in rank order, like the NCCL path;
+                                                                // mask_sum's pairs add exactly (dp_pack_sum)
             for (int r = 0; r < world; ++r) { fh += __ldcv(A.buf[r] + A.n + 2 * threadIdx.x); fl += __ldcv(A.buf[r] + A.n + 2 * threadIdx.x + 1); }
             hi = (double)fh; lo = (double)fl;
             stats[threadIdx.x] = hi + lo;

@@ -85,15 +85,13 @@ __global__ void stats_reset_kernel(double* stats) {
 }
 
 // Data-parallel exchange: the five double loss sums ride in the tail of the fp32 gradient buffer as (hi, lo) float pairs,
-// so ONE all-reduce(sum, fp32) over [grads | 10 floats] carries everything a step exchanges.  hi + lo reproduces the
-// double to 2^-48; the fp32 sums over <= 8 ranks keep ~1e-7 relative (mask_sum, an integer < 2^24, stays exact).
+// so ONE all-reduce(sum, fp32) over [grads | 10 floats] carries everything a step exchanges (dp_pack_sum, common.cuh).
+// hi + lo reproduces the double to 2^-48; the fp32 sums over W <= 8 ranks add at most (W - 1) 2^-24 of the sum of the
+// magnitudes, and mask_sum stays exact up to a global count of 2^36.
 __global__ void dp_pack_stats_kernel(const double* __restrict__ stats, float* __restrict__ tail) {
     const int i = threadIdx.x;
     if (i < 5) {
-        const double v = stats[i];
-        const float hi = (float)v;
-        tail[2 * i] = hi;
-        tail[2 * i + 1] = (float)(v - (double)hi);
+        dp_pack_sum(i, stats[i], tail + 2 * i);
     } else if (i < PMB_DP_TAIL_FLOATS / 2) {
         tail[2 * i] = 0.f;
         tail[2 * i + 1] = 0.f;

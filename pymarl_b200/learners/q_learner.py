@@ -171,9 +171,12 @@ class QLearner:
         if self._workspace is None or self._workspace.numel() < need or self._workspace.device != dev:
             self._workspace = None
             self._workspace = th.empty(need, dtype=th.uint8, device=dev)
+        self._ensure_stats(dev)
+        return need
+
+    def _ensure_stats(self, dev):
         if self._stats is None or self._stats.device != dev:
             self._stats = th.zeros(_lib.STATS_LEN, dtype=th.float64, device=dev)
-        return need
 
     def workspace_views(self, dims):
         """Named tensors over the step's workspace (tests / debugging)."""
@@ -404,7 +407,9 @@ class QLearner:
         dims.B = B
         pb = _lib.make_batch(fields, need_state=(a.mixer == "qmix"), keep=keep, ep_index=ep_index, dims=dims,
                              entry=_lib.ENTRY_TRAIN_STEP)
+        # a rank without episodes (batch_size < world) builds no workspace, but its stats take part in the exchange
         need = self._ensure_workspace(dims, dev) if B > 0 else 0
+        self._ensure_stats(dev)
         if dp and (self._dp_scratch is None or self._dp_scratch.device != dev):
             self._dp_scratch = th.empty(4096, dtype=th.float32, device=dev)
 
